@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- captions/s of the Caption-HN hot path on B200 (BASELINE.json metric), one JSON line on stdout.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W]                      # our CUDA path (default N=1)
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR] # our CUDA path (default N=1)
   python bench.py --impl reference [--gpus N] [--steps K] [--warmup W]     # the reference's CPU path (oracle port)
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N # N > 1 (one rank per GPU, NCCL)
 
@@ -27,6 +27,9 @@ sys.path.insert(0, ROOT)
 
 CFG = dict(B=512, T=20, E=200, H=150, V=9684, L=1, D=2048)
 CPU_SAMPLE_B = 512  # same batch as the GPU arm: the per-step hypernet cost amortises over the batch, so a smaller sample would understate the CPU
+DUMP_LOGIT_ROWS = 256          # (caption, position) rows of the [B*T, V] logits that --dump-outputs writes
+DUMP_GRAD_ENTRIES = 1 << 19    # entries written per parameter gradient (all of them when it has fewer)
+DUMP_MAX_BYTES = 64 << 20
 
 
 def parse():
@@ -38,7 +41,16 @@ def parse():
     ap.add_argument("--batch", type=int, default=CFG["B"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (loss, logits, parameter gradients) "
+                         "as DIR/<name>.npy, float32; large arrays as a fixed seeded sample, %d MB in all at most"
+                         % (DUMP_MAX_BYTES >> 20))
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -134,7 +146,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warmup = max(1, min(args.steps, 5)), max(1, min(args.warmup, 1))
+    steps, warmup = args.steps, args.warmup
     r = cpu_reference_arm(steps, warmup)
     line = {
         "impl": "reference", "metric": "hypernet-GRU train captions/s", "value": r["value"], "unit": "captions/s",
@@ -203,11 +215,11 @@ def run_ours(args):
         style = model.captioner.embed.weight[4:5]          # 'factual' row, hypernet_attention.py:139-142 idiom
         captioner = model.forward(style)
         feats = model.image_encoder(pooled)
-        loss, _logits = captioner.forward_loss(feats, caps, h0=h0, ignore_index=None)   # decoder + CE (hypernet.py:139-145)
+        loss, logits = captioner.forward_loss(feats, caps, h0=h0, ignore_index=None)   # decoder + CE (hypernet.py:139-145)
         (loss * inv_world if world > 1 else loss).backward()
         if world > 1:
             parallel.allreduce_shared_grads(shared)
-        return loss
+        return loss, logits
 
     # End to end through the module API, the way a training loop with a pinned-memory loader runs it: every step's
     # inputs are copied host->device inside the timed region (on a copy stream, one step ahead, into one of two device
@@ -251,7 +263,7 @@ def run_ours(args):
             e2e_state["primed"] = True
         _issue_copy(i + 1)                                    # next step's inputs fly while this step computes
         cur.wait_event(ev_copied[i % 2])
-        loss = run_step(*dbuf[i % 2])
+        loss, _ = run_step(*dbuf[i % 2])
         ev_free[i % 2].record(cur)
         loss_ring[i % 2].copy_(loss.detach().reshape(1), non_blocking=True)
         ev_loss[i % 2].record(cur)
@@ -287,11 +299,18 @@ def run_ours(args):
     for _ in range(max(3, args.warmup)):
         run_step(pooled_d, caps_d, h0_d)
     l0 = _cabi.launches()
-    ms = timed(lambda: run_step(pooled_d, caps_d, h0_d), args.steps)
+    last = [None]
+
+    def headline_step():
+        last[0] = run_step(pooled_d, caps_d, h0_d)
+    ms = timed(headline_step, args.steps)
     launches = _cabi.launches() - l0
     if gstep is not None:                                     # replayed launches are not seen by the library's counter
         launches = gstep.launches_per_step * args.steps
     value = B * world * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last[0], model)
+    last = None
 
     for _ in range(2):
         step_e2e()
@@ -535,6 +554,35 @@ def run_ours(args):
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(dirname, loss, logits, model):
+    """What one headline step returns to its caller, as float32 .npy files under `dirname`: loss.npy, logits_rows.npy
+    (DUMP_LOGIT_ROWS rows of the [B*T, V] logits) and grad.<parameter>.npy for every parameter gradient (flattened;
+    DUMP_GRAD_ENTRIES entries of the larger ones).  The rows and entries are drawn from generators seeded by the array's
+    name, so every run with the same arguments writes the same positions and two builds compare entry for entry."""
+    import zlib
+    import numpy as np
+
+    def pick(name, x, k):
+        """k rows of x (all of them when it has no more)."""
+        if x.shape[0] <= k:
+            return x
+        g = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+        return x[torch.randint(x.shape[0], (k,), generator=g).sort().values.to(x.device)]
+
+    out = {"loss": loss.detach().reshape(1)}
+    lg = logits.detach()
+    out["logits_rows"] = pick("logits_rows", lg.reshape(-1, lg.shape[-1]), DUMP_LOGIT_ROWS)
+    for name, p in model.named_parameters():
+        if p.grad is not None:
+            out["grad." + name] = pick(name, p.grad.detach().reshape(-1), DUMP_GRAD_ENTRIES)
+    total = sum(v.numel() * 4 for v in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs would write {total} bytes, more than {DUMP_MAX_BYTES}")
+    os.makedirs(dirname, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), v.float().cpu().numpy())
 
 
 def roofline_block(alg_bytes, ms, peak, what):

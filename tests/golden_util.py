@@ -1,4 +1,5 @@
 """Loading of the committed golden vectors (tests/golden/*.npz, made by oracle/make_golden.py)."""
+import hashlib
 import os
 
 import numpy as np
@@ -8,11 +9,25 @@ GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def load_case(name):
+    """The arrays of one case.  Reduced parts (oracle/make_golden.py) come back as follows: `features` is redrawn from
+    its seed and checked against its SHA-256; a matrix stored as `<k>/rows` + `<k>/values` is rebuilt with zeros in the
+    rows the case never reads; a [.., V] output listed under `vocab_axis/<k>` holds the entries `vocab_sample` only --
+    compare it with golden_rel_err / golden_grad_close."""
     z = np.load(os.path.join(GOLDEN, name + ".npz"), allow_pickle=False)
     out = {}
     for k in z.files:
         v = z[k]
         out[k] = v if v.dtype.kind in "US" else torch.from_numpy(v)
+    if "features/seed" in out:
+        g = torch.Generator().manual_seed(int(out.pop("features/seed")))
+        f = torch.randn(out.pop("features/shape").tolist(), generator=g)
+        assert hashlib.sha256(f.numpy().tobytes()).hexdigest() == str(out.pop("features/sha256")), \
+            "torch.randn no longer reproduces the golden features from their seed"
+        out["features"] = f
+    for k in [k[:-len("/rows")] for k in out if k.endswith("/rows")]:
+        full = torch.zeros(out.pop(k + "/shape").tolist(), dtype=out[k + "/values"].dtype)
+        full[out.pop(k + "/rows")] = out.pop(k + "/values")
+        out[k] = full
     return out
 
 
@@ -20,20 +35,40 @@ def params_of(case):
     return {k[3:]: v.clone() for k, v in case.items() if k.startswith("sd/")}
 
 
-def rel_err(a, b):
-    """max|a-b| / max|b|  (the tolerance form of SURVEY.md 8(d))."""
+def rel_err(a, b, scale=None):
+    """max|a-b| / max|b|  (the tolerance form of SURVEY.md 8(d)); `scale` replaces max|b|."""
     a, b = a.detach().double().cpu(), b.detach().double().cpu()
     d = (a - b).abs().max().item()
-    s = b.abs().max().item()
+    s = b.abs().max().item() if scale is None else float(scale)
     return d / s if s > 0 else d
 
 
-def grad_close(a, b, rtol, atol=1e-7):
-    """Gradient comparison: relative to max|ref|, with an absolute floor for gradients that are analytically zero
-    (e.g. d/d v_a.bias -- softmax is shift invariant -- which come out as 1e-9 rounding noise)."""
+def grad_close(a, b, rtol, atol=1e-7, scale=None):
+    """Gradient comparison: relative to max|ref| (or `scale`), with an absolute floor for gradients that are
+    analytically zero (e.g. d/d v_a.bias -- softmax is shift invariant -- which come out as 1e-9 rounding noise)."""
     a, b = a.detach().double().cpu(), b.detach().double().cpu()
     d = (a - b).abs().max().item()
-    return d <= atol or d <= rtol * b.abs().max().item()
+    return d <= atol or d <= rtol * (b.abs().max().item() if scale is None else float(scale))
+
+
+def _stored_part(case, key, x):
+    """x reduced the way the case stores `key`, and the scale max|ref| of the full reference array (None: x is whole)."""
+    if "vocab_axis/" + key not in case:
+        return x, None
+    idx = case["vocab_sample"].to(x.device)
+    return x.index_select(int(case["vocab_axis/" + key]), idx), case["absmax/" + key]
+
+
+def golden_rel_err(case, key, x):
+    """rel_err(x, case[key]) for a full-size x, also where the case keeps a vocabulary sample of `key`."""
+    part, scale = _stored_part(case, key, x)
+    return rel_err(part, case[key], scale)
+
+
+def golden_grad_close(case, key, x, rtol, atol=1e-7):
+    """grad_close(x, case[key], rtol, atol) for a full-size x, also where the case keeps a vocabulary sample of `key`."""
+    part, scale = _stored_part(case, key, x)
+    return grad_close(part, case[key], rtol, atol, scale)
 
 
 def same_greedy_paths(a, b, tol=1e-4, min_frac=0.5):

@@ -106,6 +106,30 @@ def test_reference_arm_line_has_the_contract_keys(monkeypatch, capsys):
     assert line["config"] == bench.workload_config(args, args.gpus)
 
 
+def test_dump_outputs_writes_float32_samples_at_fixed_positions(tmp_path):
+    """bench.py --dump-outputs: loss, logits rows and every parameter gradient as float32 .npy; arrays larger than the
+    per-array budget are sampled at positions that depend on the array's name only, so two runs write the same entries."""
+    import numpy as np
+    import torch
+    bench = _bench()
+    torch.manual_seed(0)
+    model = torch.nn.Linear(300, 2000)                       # weight: 600 000 entries, more than DUMP_GRAD_ENTRIES
+    (model(torch.randn(4, 300)) * torch.randn(4, 2000)).sum().backward()
+    loss, logits = torch.tensor(2.5), torch.randn(8, 5, 97)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), loss, logits, model)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["grad.bias.npy", "grad.weight.npy", "logits_rows.npy", "loss.npy"]
+    got = {n: np.load(tmp_path / "a" / n) for n in names}
+    assert all(v.dtype == np.float32 for v in got.values())
+    assert all(np.array_equal(v, np.load(tmp_path / "b" / n)) for n, v in got.items())
+    assert got["loss.npy"].tolist() == [2.5]
+    assert np.array_equal(got["logits_rows.npy"], logits.reshape(40, 97).numpy())         # 40 rows: all of them
+    assert np.array_equal(got["grad.bias.npy"], model.bias.grad.numpy())
+    w = got["grad.weight.npy"]
+    assert w.shape == (bench.DUMP_GRAD_ENTRIES,) and np.isin(w, model.weight.grad.numpy()).all()
+
+
 def test_reference_arm_uses_our_arms_config_at_n_gpus_and_only_rank0_prints(monkeypatch, capsys):
     bench = _bench()
     monkeypatch.setattr(bench, "cpu_reference_arm", _fake_arm)

@@ -6,7 +6,7 @@ import torch
 
 pytestmark = pytest.mark.gpu
 
-from golden_util import load_case, params_of, rel_err, grad_close
+from golden_util import load_case, params_of, rel_err, grad_close, golden_rel_err, golden_grad_close
 from oracle import caption_hn_oracle as O
 
 TOL_LOGITS = 1e-4   # BASELINE.json north_star: fp32 mode within 1e-4 relative on logits and loss
@@ -60,14 +60,14 @@ def test_pooled_golden(name, L, kind, mode):
     feats = m.image_encoder(c["pooled"].cuda())
     h0 = c["h0"].cuda() if kind == "gru" else None        # DecoderRNN starts from zeros (later.py:256-259)
     logits = captioner(feats, c["captions"].cuda(), True, h0=h0)
-    assert rel_err(logits, c["tf/logits"]) < TOL_LOGITS
+    assert golden_rel_err(c, "tf/logits", logits) < TOL_LOGITS
     loss = C.cross_entropy(logits, c["captions"].cuda(), None)
     assert abs(loss.item() - c["tf/loss"].item()) < TOL_LOGITS * abs(c["tf/loss"].item())
     loss.backward()
     named = dict(m.named_parameters())
     for k in ("image_encoder.fc.weight", "image_encoder.fc.bias", "captioner.embed.weight",
               "captioner.fc_out.weight", "captioner.fc_out.bias"):
-        assert grad_close(named[k].grad, c["tf/grad/" + k], TOL_GRAD), k
+        assert golden_grad_close(c, "tf/grad/" + k, named[k].grad, TOL_GRAD), k
     if mode == "literal":
         for ci, cell in enumerate(cells_mod):
             for k in ("weight_ih", "weight_hh", "bias_ih", "bias_hh"):
@@ -96,8 +96,8 @@ def test_pooled_infer_golden_token_exact(name, L, kind, table, monkeypatch):
         captioner = m.forward(c["style"].cuda())
         probs = captioner.infer(m.image_encoder(c["pooled"].cuda()), max_len=c["infer/probs"].shape[1],
                                 h0=c["h0"].cuda() if kind == "gru" else None)
-    assert torch.equal(probs.argmax(-1).cpu(), c["infer/probs"].argmax(-1))
-    assert rel_err(probs, c["infer/probs"]) < TOL_LOGITS
+    assert torch.equal(probs.argmax(-1).cpu(), c["infer/tokens"])
+    assert golden_rel_err(c, "infer/probs", probs) < TOL_LOGITS
 
 
 def test_pooled_rng_consumption_matches_reference():
@@ -108,7 +108,7 @@ def test_pooled_rng_consumption_matches_reference():
     feats = m.image_encoder(c["pooled"].cuda())
     torch.manual_seed(1)
     logits = captioner(feats, c["captions"].cuda(), True)
-    assert rel_err(logits, c["tf/logits"]) < TOL_LOGITS
+    assert golden_rel_err(c, "tf/logits", logits) < TOL_LOGITS
 
 
 @pytest.mark.parametrize("B,T,E,H,V,L", [(37, 9, 24, 30, 311, 1), (64, 20, 200, 150, 2000, 1), (21, 6, 24, 30, 211, 2),

@@ -4,7 +4,7 @@ import pytest
 import torch
 
 from oracle import caption_hn_oracle as O
-from golden_util import load_case, params_of, rel_err, grad_close
+from golden_util import load_case, params_of, rel_err, grad_close, golden_rel_err, golden_grad_close
 
 TOL = 2e-6  # same torch CPU kernels in the same order; observed <= 1e-6
 
@@ -75,7 +75,7 @@ def test_pooled_variant_matches_reference(name, L, kind):
     for ci, cell in enumerate(cells):
         for k, w in zip(("weight_ih", "weight_hh", "bias_ih", "bias_hh"), cell):
             assert rel_err(w, c[f"gen/{ci}/{k}"]) < TOL, (ci, k)
-    assert rel_err(logits, c["tf/logits"]) < TOL
+    assert golden_rel_err(c, "tf/logits", logits) < TOL
     loss = O.caption_loss(logits, c["captions"], None)
     assert abs(loss.item() - c["tf/loss"].item()) < 1e-6 * abs(c["tf/loss"].item())
     loss.backward()
@@ -83,12 +83,12 @@ def test_pooled_variant_matches_reference(name, L, kind):
         for k, w in zip(("weight_ih", "weight_hh", "bias_ih", "bias_hh"), cell):
             assert grad_close(w.grad, c[f"tf/grad/gen/{ci}/{k}"], 1e-5), (ci, k)
     for k in ("image_encoder.fc.weight", "captioner.embed.weight", "captioner.fc_out.weight", "captioner.fc_out.bias"):
-        assert grad_close(p[k].grad, c["tf/grad/" + k], 1e-5), k
+        assert golden_grad_close(c, "tf/grad/" + k, p[k].grad, 1e-5), k
     with torch.no_grad():
         probs, _, _ = O.path_pooled(p, c["style"], c["pooled"], None, c["h0"], L=L, infer_len=c["infer/probs"].shape[1],
                                     cell=kind)
-    assert torch.equal(probs.argmax(-1), c["infer/probs"].argmax(-1))
-    assert rel_err(probs, c["infer/probs"]) < TOL
+    assert torch.equal(probs.argmax(-1), c["infer/tokens"])
+    assert golden_rel_err(c, "infer/probs", probs) < TOL
 
 
 @pytest.mark.parametrize("name,L,kind", POOLED_CASES)
