@@ -70,22 +70,25 @@ __global__ void __launch_bounds__(BS_THREADS) beam_step_kernel(const BeamArgs a)
         if (tid == 0) {
             float t = 0.f;
             for (int w = 0; w < BS_THREADS / 32; ++w) t += s_rv[w];
-            s_lse[r] = mx + logf(t);
+            const float lse = mx + logf(t);
+            s_lse[r] = isfinite(lse) ? lse : NAN;      // a NaN / +inf logit or an all -inf row: every score NaN, no candidate
             s_ts[r] = a.scores[r0 + r];
         }
         __syncthreads();
     }
-    // ---- top-n of the nrows * V candidates: n passes, pass j takes the best candidate that comes after pick j-1 ----
+    // ---- top-n of the nrows * V candidates: n passes, pass j takes the best candidate that comes after pick j-1.  A NaN
+    //      score is never `after` anything: such candidates are not eligible ----
     float last_s = INFINITY;
     int last_i = -1;
     const int ncand = nrows * V;
+    int found = n;
     for (int j = 0; j < n; ++j) {
         float bs = -INFINITY;
         int bi = 0x7fffffff;
         for (int c = tid; c < ncand; c += BS_THREADS) {
             const int r = c / V, v = c - r * V;
             const float s = s_ts[r] + (a.logits[(r0 + r) * V + v] - s_lse[r]);
-            const bool after = s < last_s || (s == last_s && c > last_i);
+            const bool after = s < last_s || (s == last_s && c > last_i);      // false for NaN
             if (after && better(s, c, bs, bi)) { bs = s; bi = c; }
         }
 #pragma unroll
@@ -107,6 +110,13 @@ __global__ void __launch_bounds__(BS_THREADS) beam_step_kernel(const BeamArgs a)
         __syncthreads();
         last_s = s_pick_s[j];
         last_i = s_pick_i[j];
+        if (last_i == 0x7fffffff) { found = j; break; }   // (block-uniform) no eligible candidate left
+    }
+    if (found < n) {
+        // the image ends without a caption, and nothing is read through the missing pick
+        if (tid == 0) { a.live[b] = 0; a.failed[b] = 1; }
+        for (int j = tid; j < k; j += BS_THREADS) a.words[r0 + j] = -1;
+        return;
     }
     // ---- bookkeeping (one thread): completed beams out, survivors compacted ----
     const int len = a.step;                       // tokens in every live history (leading 0 + step-1 words)
@@ -169,12 +179,14 @@ extern "C" {
 
 // One beam-search bookkeeping step for B images x k beams (see file header).  step is 1-based; last != 0 marks the final
 // permitted step (reference: step > max_steps): images that still have open beams get failed[b] = 1.
-// seq_in / seq_out: token histories [B*k, L] (ping-pong between steps), L >= max steps + 2.
+// seq_in / seq_out: token histories [B*k, L] (ping-pong between steps), L >= max steps + 2.  k <= V: step 1 ranks V
+// candidates.  Rows whose log-sum-exp is not finite offer no candidates; an image left with fewer than its live count of
+// candidates ends with failed[b] = 1, live[b] = 0.
 int caphn_beam_step(const float* logits, const float* h_out, float* h_next, float* scores, int* live, int* prev_tok,
                     long long* words, const int* seq_in, int* seq_out, float* comp_score, int* comp_seq, int* comp_len,
                     int* ncomp, int* failed, int B, int k, int V, int H, int L, int step, int end_tok, int last,
                     void* stream) {
-    if (B <= 0 || k <= 0 || k > BS_MAXK || V <= 0 || H <= 0 || L < 2 || step < 1) return CAPHN_EINVAL;
+    if (B <= 0 || k <= 0 || k > BS_MAXK || V <= 0 || k > V || H <= 0 || L < 2 || step < 1) return CAPHN_EINVAL;
     BeamArgs a{logits, h_out, h_next, scores, live, prev_tok, words, seq_in, seq_out, comp_score, comp_seq, comp_len,
                ncomp, failed, B, k, V, H, L, step, end_tok, last};
     beam_step_kernel<<<B, BS_THREADS, 0, (cudaStream_t)stream>>>(a);

@@ -360,7 +360,8 @@ __global__ void __launch_bounds__(CE_THREADS) ce_fwd_split_kernel(const float* _
     }
 }
 
-// Row softmax (optional, Y may be null) and first-max argmax (matches torch.argmax / topk(1) tie-breaking: lowest index).
+// Row softmax (optional, Y may be null) and first-max argmax (matches torch.argmax / topk(1) tie-breaking: lowest index;
+// NaN counts as -inf, DESIGN.md §6).
 __global__ void __launch_bounds__(CE_THREADS) softmax_argmax_kernel(const float* __restrict__ X, long ld, int V,
                                                                     float* __restrict__ Y, long ldy,
                                                                     long long* __restrict__ amax) {
@@ -371,7 +372,7 @@ __global__ void __launch_bounds__(CE_THREADS) softmax_argmax_kernel(const float*
     float mx = -INFINITY;
     int mi = 0x7fffffff;
     for (int i = threadIdx.x; i < V; i += CE_THREADS) {
-        const float v = x[i];
+        const float v = isnan(x[i]) ? -INFINITY : x[i];     // else [NaN, -inf, ..] would tie to index 1, not 0
         if (v > mx || (v == mx && i < mi)) { mx = v; mi = i; }
     }
 #pragma unroll
@@ -493,6 +494,7 @@ __global__ void gather_rows_kernel(const float* __restrict__ table, const long l
 // Greedy feedback after caphn_gemm_tc_amax: finish the row arg-max from the epilogue's partials (ties: lowest column, like
 // torch.argmax / topk(1)), write the token, and gather the row of `table` it selects (the embedding, or the pre-multiplied
 // input projection Emb W_ih^T + b_ih) -- one launch between the vocabulary projection of step t and the recurrence of t+1.
+// A row whose partials are all empty (its logits all NaN / -inf) gets token 0, never the empty slot's column.
 __global__ void __launch_bounds__(128) argmax_finish_gather_kernel(const float* __restrict__ pval, const int* __restrict__ pidx,
                                                                     int ld, int nparts, const float* __restrict__ table,
                                                                     int E, long long* __restrict__ tok,
@@ -513,6 +515,7 @@ __global__ void __launch_bounds__(128) argmax_finish_gather_kernel(const float* 
             const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
             if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
         }
+        if (bi == 0x7fffffff) bi = 0;
         if (threadIdx.x == 0) { s_tok = bi; if (tok) tok[i] = bi; }
     }
     __syncthreads();

@@ -105,6 +105,7 @@ __global__ void __launch_bounds__(GD_MAXW * 32) gru_decode_step_kernel(const Gru
                 const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
                 if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
             }
+            if (bi == 0x7fffffff) bi = 0;                  // all partials empty (logits all NaN / -inf): token 0
             if (lane == 0 && b < B) {
                 s_tok[2 * warp + rr] = bi;
                 if (a.tok && blockIdx.x == 0) a.tok[b] = bi;

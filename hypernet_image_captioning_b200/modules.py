@@ -351,7 +351,7 @@ class DecoderGRU(nn.Module):
         hop = ops.SplitOperand(hhi, hlo, B, H, Kp)
         hbuf = [torch.empty(B, H, device=x.device, dtype=torch.float32) for _ in range(2)]
         GIb = torch.empty(B, 3 * H, device=x.device, dtype=torch.float32)
-        fused_step = ops.gru_decode_step_ok(H)      # else: arg-max finish + gather, GRU step, operand split as three launches
+        fused_step = ops.gru_decode_step_ok(H, self.vocab_size)      # else: arg-max finish + gather, GRU step, operand split as three launches
         nparts = 0
         import contextlib
         cur = torch.cuda.current_stream()

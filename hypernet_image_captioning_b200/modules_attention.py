@@ -523,8 +523,10 @@ class AttentionGru(nn.Module):
             raise ValueError("beam_search_batched expects features [B, P, D]")
         B, P, D = feats.shape
         k = int(beam_size)
-        W_ih, W_hh, b_ih, b_hh = [w.detach().contiguous() for w in self._gru_weights()]
         E, H, V = self.embedding_dim, self.hidden_dim, self.vocab_size
+        if k > V:
+            raise ValueError(f"beam_size {k} exceeds the vocabulary size {V}")
+        W_ih, W_hh, b_ih, b_hh = [w.detach().contiguous() for w in self._gru_weights()]
         dev = feats.device
         a = self.attention
         emb_w = self.embed.weight.detach()

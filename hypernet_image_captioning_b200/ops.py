@@ -833,9 +833,11 @@ def argmax_finish_gather(pval, pidx, nparts, table=None, tok=None, out=None):
                _p(tok), _p(out), out.stride(0) if out is not None else 0, _stream())
 
 
-def gru_decode_step_ok(H):
-    """The fused decode-step kernel keeps 96 rows of W_hh and up to 32 states in shared memory as float2: H even, <= ~390."""
-    return H % 2 == 0 and (96 * (H + 2) + 32 * H) * 4 <= 200 * 1024
+def gru_decode_step_ok(H, V):
+    """The fused decode-step kernel keeps 96 rows of W_hh and up to 32 states in shared memory as float2: H even, <= ~390;
+    and each lane holds 8 arg-max partial slots: at most 256 = 2 ceil(V / BN) per row, bounded here with the narrowest N
+    tile the GEMM picks for V > 256 (BN = 128), i.e. V <= 16384."""
+    return H % 2 == 0 and (96 * (H + 2) + 32 * H) * 4 <= 200 * 1024 and 2 * ((V + 127) // 128) <= 256
 
 
 def gru_decode_step(GI, pval, pidx, nparts, table, W_hh, b_hh, hprev, hnew, hi=None, lo=None, tok=None):

@@ -189,7 +189,8 @@ int caphn_ce_bwd(const float* X, long ld, const long long* tgt, long M, int V, i
 int caphn_ce_bwd_split(const float* X, long ld, const long long* tgt, long M, int V, int has_ignore, long long ignore,
                        const float* lse, const float* gscale, const float* lossbuf, void* hi, void* lo, long Vp,
                        void* hiT, void* loT, long Mp, float* dbias, void* stream);
-/* Y (optional) = row softmax of X[M,V]; amax (optional, int64) = row argmax, lowest index on ties. */
+/* Y (optional) = row softmax of X[M,V]; amax (optional, int64) = row argmax, lowest index on ties, NaN counted as -inf
+ * (an all-NaN / all -inf row gives 0). */
 int caphn_softmax_argmax(const float* X, long ld, long M, int V, float* Y, long ldy, long long* amax, void* stream);
 /* out[i,:] = table[idx[i],:]  (idx int64; negative idx -> zero row). */
 int caphn_gather_rows(const float* table, const long long* idx, long n, int E, float* out, long ldo, void* stream);
@@ -307,7 +308,9 @@ int caphn_attstep_bwd_grouped(const float* dHbm, const float* dattn, const float
  * beams (rows b*k.., live beams first) one launch does what the reference does on the host between two decoder steps --
  * log-softmax + running scores, top-k_live over (live rows x V) (step 1: row 0 only), completed beams moved to the image's
  * complete list, survivors compacted with their history / score / hidden state, next input words (-1 = zero embedding).
- * step is 1-based; last != 0: images with beams still open are flagged in failed[] (the reference returns no caption). */
+ * step is 1-based; last != 0: images with beams still open are flagged in failed[] (the reference returns no caption).
+ * k <= V (else CAPHN_EINVAL).  A row whose log-sum-exp is not finite (a NaN / +inf logit) offers no candidates; an image
+ * left with fewer eligible candidates than live beams ends at once with failed[b] = 1, live[b] = 0. */
 int caphn_beam_step(const float* logits, const float* h_out, float* h_next, float* scores, int* live, int* prev_tok,
                     long long* words, const int* seq_in, int* seq_out, float* comp_score, int* comp_seq, int* comp_len,
                     int* ncomp, int* failed, int B, int k, int V, int H, int L, int step, int end_tok, int last,
@@ -323,8 +326,9 @@ int caphn_adam_step_bf16(void* p, const void* g, float* master, float* m, float*
 /* Greedy decode (models/decoderlstm.py:89-96: top_idx = topk(log_softmax(output / 0.5), 1) == arg-max of the logits):
  * caphn_gemm_tc_amax = caphn_gemm_tc_ex whose epilogue also reduces every row of every output tile to (max, column)
  * partials [M, amax_ld] (*nparts slots are written; amax_ld >= 2*ceil(N/128) suffices); caphn_argmax_finish_gather
- * finishes the arg-max (lowest column on ties), writes the token and gathers the row of `table` it selects (embedding, or
- * the pre-multiplied input projection) -- replacing a full pass over the logits + a separate gather per decode step. */
+ * finishes the arg-max (lowest column on ties; NaN never wins; 0 for a row with no candidate), writes the token and gathers
+ * the row of `table` it selects (embedding, or the pre-multiplied input projection) -- replacing a full pass over the
+ * logits + a separate gather per decode step. */
 int caphn_gemm_tc_amax(const void* Ahi, const void* Alo, long a_ld, int a_mn, const void* Bhi, const void* Blo, long b_ld,
                        int b_mn, long K, float* C, long ldc, const float* bias, int M, int N, float* amax_val,
                        int* amax_idx, int amax_ld, int* nparts, void* stream);
@@ -376,7 +380,8 @@ int caphn_gemm_tc_prof(const void* Ahi, const void* Alo, long a_ld, int a_mn, co
  * launch: finishes the arg-max of the previous vocabulary projection from the partials of caphn_gemm_tc_amax (GI == NULL; the
  * token goes to tok if non-NULL), takes the input projection from row tok of table [V, 3H] (= Emb W_ih^T + b_ih) -- or uses
  * GI [B, 3H] directly (step 0) --, applies the GRU cell with W_hh [3H, H] / b_hh and writes hnew [B, H] plus, if hi != NULL, its
- * bf16 hi / lo operand rows [B, Kp] for the next vocabulary projection.  hnew must not alias hprev. */
+ * bf16 hi / lo operand rows [B, Kp] for the next vocabulary projection.  hnew must not alias hprev.  nparts <= 256
+ * (else CAPHN_EINVAL); a row with no candidate in its partials gets token 0. */
 int caphn_gru_decode_step(const float* GI, const float* pval, const int* pidx, int ldp, int nparts, const float* table,
                           const float* Whh, const float* bhh, const float* hprev, float* hnew, void* hi, void* lo, long Kp,
                           long long* tok, int B, int H, void* stream);

@@ -181,6 +181,22 @@ def test_softmax_argmax_vector_and_generic_paths(V):
     assert rel_err(out[:, 1, :], ref) < 2e-6 and float(out[:, 0].abs().max()) == 0.0 and float(out[:, 2].abs().max()) == 0.0
     _, am2 = ops.softmax_argmax(x, want_probs=False)
     assert torch.equal(am2, am)
+    # non-finite rows: the selection contract (NaN counts as -inf, lowest index on ties; all NaN / all -inf -> 0)
+    from test_gpu_decode_select import greedy_token
+    nan, inf = float("nan"), float("inf")
+    y = x.clone()
+    y[0] = nan
+    y[1] = -inf; y[1, 0] = nan                       # [NaN, -inf, -inf, ...]
+    y[2] = -inf
+    y[3, V // 3] = inf; y[3, V - 1] = inf            # tied +inf
+    y[4, ::3] = nan; y[4, V - 1] = 20.0              # NaN everywhere but a finite maximum
+    y[5] = -inf; y[5, 1 % V] = nan; y[5, V - 1] = nan
+    y[6, 0] = nan
+    _, am3 = ops.softmax_argmax(y, want_probs=True)
+    _, am4 = ops.softmax_argmax(y, want_probs=False)
+    want = greedy_token(y.cpu())
+    assert torch.equal(am3.cpu(), want) and torch.equal(am4.cpu(), want)
+    assert am3[:3].tolist() == [0, 0, 0] and am3[3].item() == V // 3 and am3[4].item() == V - 1
 
 
 @pytest.mark.parametrize("B,T,H", [(3, 5, 6), (9, 4, 150), (21, 3, 33), (16, 6, 200), (5, 2, 301)])
@@ -298,10 +314,13 @@ def test_gemm_tc_a_stationary_schedule_is_bit_identical(M, N, K, monkeypatch):
     assert torch.equal(outs["0"], outs["1"]) and torch.equal(outs["0"], outs["2"])
 
 
-@pytest.mark.parametrize("B,H,V", [(512, 150, 9684), (37, 34, 301), (16, 200, 1000), (5, 6, 40), (300, 256, 500)])
+@pytest.mark.parametrize("B,H,V", [(512, 150, 9684), (37, 34, 301), (16, 200, 1000), (5, 6, 40), (300, 256, 500),
+                                   (64, 32, 16384)])
 def test_fused_decode_step_matches_the_three_launch_chain(B, H, V):
     """caphn_gru_decode_step (arg-max finish + projection-table gather + GRU cell + bf16 operand rows in one launch) ==
-    argmax_finish_gather -> gru_seq_fwd(T = 1) -> split_bf16, the chain it replaces in DecoderGRU.infer (later.py:459-490)."""
+    argmax_finish_gather -> gru_seq_fwd(T = 1) -> split_bf16, the chain it replaces in DecoderGRU.infer (later.py:459-490).
+    V = 40: one partial slot; V = 16384: all 256 slots the kernel holds, the winner in the last lane's last register.
+    Both also take rows of empty (-inf, no column) and NaN partials, whose token is 0."""
     import torch
     from hypernet_image_captioning_b200 import ops
     g = torch.Generator().manual_seed(3)
@@ -336,6 +355,20 @@ def test_fused_decode_step_matches_the_three_launch_chain(B, H, V):
     ops.gru_decode_step(GI, None, None, 0, None, W_hh, b_hh, h, hn0)
     assert (hn0 - h_ref).abs().max().item() < 2e-6
     del sp
+    # every slot in use, the winner in the last one; empty and NaN rows
+    from test_gpu_decode_select import NONE, finish_partials
+    pv[1::4, nslot - 1] = 50.0
+    pv[2::5], pi[2::5] = float("-inf"), NONE
+    pv[3::7] = float("nan")
+    tok_ref2 = torch.empty(B, device="cuda", dtype=torch.int64)
+    ops.argmax_finish_gather(pv, pi, nslot, table, tok_ref2, GI)
+    want = finish_partials(pv, pi, nslot)
+    assert torch.equal(tok_ref2.cpu(), want)
+    assert bool((want[2::5] == 0).all()) and bool((want[3::7] == 0).all())
+    h_ref2 = ops.gru_seq_fwd(GI, WhhT, b_hh, h, 1, save=False, want_bm=False)[0][1]
+    ops.gru_decode_step(None, pv, pi, nslot, table, W_hh, b_hh, h, hn, hi, lo, tok)
+    assert torch.equal(tok, tok_ref2)
+    assert (hn - h_ref2).abs().max().item() < 2e-6
 
 
 @pytest.mark.parametrize("B,T,H", [(3, 5, 6), (9, 4, 150), (21, 3, 33), (16, 6, 160), (512, 20, 150), (6, 2, 100)])
