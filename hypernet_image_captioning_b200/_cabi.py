@@ -92,6 +92,7 @@ SIGNATURES = {
     "caphn_gemm_tc_scaled": [P, P, L, I, P, P, L, I, L, P, L, P, I, I, I, P, P, P],
     "caphn_gemm_tc_prof": [P, P, L, I, P, P, L, I, L, P, L, P, I, I, I, P, P],
     "caphn_gru_decode_step": [P, P, P, I, I, P, P, P, P, P, P, P, L, P, I, I, P],
+    "caphn_gru_decode_step_tok": [P, I, P, P, P, P, P, P, P, L, I, I, P],
     "caphn_gru_resident_plan": [I, P],
     "caphn_gru_resident_fwd": [P, P, P, P, P, P, I, I, I, P],
     "caphn_gru_resident_bwd": [P, P, P, P, P, P, P, I, I, I, P],

@@ -3,7 +3,9 @@
 // left (caphn_gemm_tc_amax), takes the next input's projection  P[tok] = Emb[tok] W_ih^T + b_ih  from the projection table,
 // runs the GRU cell against the generated W_hh and writes the new state both as fp32 and as the bf16 hi/lo operand rows of the
 // next vocabulary projection.  Replaces argmax_finish_gather + gru_seq_fwd(T = 1) + split_bf16 -- three dependent launches
-// (5 + 16 + 3 us at B = 512, H = 150) on the 20-step dependency chain of DecoderGRU.infer.
+// (5 + 16 + 3 us at B = 512, H = 150) on the 20-step dependency chain of DecoderGRU.infer.  The token-fed variant
+// (caphn_gru_decode_step_tok) takes the token from an array instead: DecoderGRU.beam_search_batched feeds it the words the
+// beam bookkeeping kernel chose.
 //
 // Grid: (ceil(H / 32) unit blocks, row blocks), sized to at most one CTA per SM (one wave, no SM with two CTAs' worth of
 // shared-memory reads): a CTA of W warps owns 2 W batch rows x 32 hidden units.  The 3 x 32 rows of W_hh it needs sit in shared
@@ -23,6 +25,12 @@ __device__ __forceinline__ void gd_cp_async8(void* dst, const void* src) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((uint32_t)__cvta_generic_to_shared(dst)), "l"(src) : "memory");
 }
 
+// Where a step's input projection comes from (template parameter of the kernel).  GD_SRC_GREEDY: GI if given, else row tok
+// of the table with tok finished from the arg-max partials -- one instantiation, so greedy decode runs the same machine code
+// for both.  GD_SRC_TOK: row tokin[b] of the table (an entry outside [0, V): row 0).  tokin / V are kernel parameters of
+// their own, not GruDecArgs fields, so the greedy instantiation's parameter block and machine code stay as they were.
+enum GruDecSrc { GD_SRC_GREEDY = 0, GD_SRC_TOK = 1 };
+
 struct GruDecArgs {
     const float* GI;        // [B, 3H] input projection incl. b_ih (step 0), or NULL: gather table[tok] with tok from the partials
     const float* pval; const int* pidx; int ldp, nparts;   // arg-max partials of the previous step [B, ldp]
@@ -36,7 +44,8 @@ struct GruDecArgs {
     int B, H, ldw, nw;      // ldw: shared row stride of the weight slice; nw: warps per CTA (rows per CTA = 2 nw)
 };
 
-__global__ void __launch_bounds__(GD_MAXW * 32) gru_decode_step_kernel(const GruDecArgs a) {
+template <int SRC>
+__global__ void __launch_bounds__(GD_MAXW * 32) gru_decode_step_kernel(const GruDecArgs a, const int* tokin, int V) {
     extern __shared__ float2 gd_smem2[];
     float* gd_smem = reinterpret_cast<float*>(gd_smem2);
     const int H = a.H, B = a.B, H3 = 3 * a.H, ldw = a.ldw, nw = a.nw, H2 = a.H >> 1;
@@ -68,10 +77,12 @@ __global__ void __launch_bounds__(GD_MAXW * 32) gru_decode_step_kernel(const Gru
     float pvr[2][PMAX];
     int pir[2][PMAX];
     float hreg[2][KMAX];
+    int tin[2] = {0, 0};
 #pragma unroll
     for (int rr = 0; rr < 2; ++rr) {
         const int b = b0 + 2 * warp + rr;
-        if (!a.GI) {
+        if (SRC == GD_SRC_TOK && b < B) tin[rr] = tokin[b];
+        if (SRC == GD_SRC_GREEDY && !a.GI) {
 #pragma unroll
             for (int it = 0; it < PMAX; ++it) {
                 const int q = lane + 32 * it;
@@ -87,7 +98,7 @@ __global__ void __launch_bounds__(GD_MAXW * 32) gru_decode_step_kernel(const Gru
         }
     }
     // (3) finish the arg-max of the previous step for this warp's rows (lowest column on ties)
-    if (!a.GI) {
+    if (SRC == GD_SRC_GREEDY && !a.GI) {
 #pragma unroll
         for (int rr = 0; rr < 2; ++rr) {
             const int b = b0 + 2 * warp + rr;
@@ -123,7 +134,8 @@ __global__ void __launch_bounds__(GD_MAXW * 32) gru_decode_step_kernel(const Gru
         for (int rr = 0; rr < 2; ++rr) {
             const int r = 2 * warp + rr, b = b0 + r;
             if (b < B) {
-                const float* gi = a.GI ? a.GI + (long)b * H3 : a.table + (long)s_tok[r] * H3;
+                const float* gi = SRC == GD_SRC_TOK ? a.table + (long)((unsigned)tin[rr] < (unsigned)V ? tin[rr] : 0) * H3
+                                : a.GI ? a.GI + (long)b * H3 : a.table + (long)s_tok[r] * H3;
                 gir[rr] = gi[j]; giz[rr] = gi[H + j]; gin[rr] = gi[2 * H + j];
             }
         }
@@ -181,6 +193,31 @@ __global__ void __launch_bounds__(GD_MAXW * 32) gru_decode_step_kernel(const Gru
 
 using namespace caphn;
 
+// Sizes the grid and launches the instantiation for SRC; the caller has checked the source-specific arguments.
+template <int SRC>
+static int gd_launch(const GruDecArgs& args, const int* tokin, int V, void* stream) {
+    GruDecArgs a = args;
+    const int B = a.B, H = a.H;
+    if (B <= 0 || H <= 0 || (H & 1) || !a.Whh || !a.bhh || !a.hprev || !a.hnew || a.hnew == a.hprev) return CAPHN_EINVAL;
+    if (((uintptr_t)a.Whh & 7)) return CAPHN_EINVAL;
+    if (a.hi && a.Kp < H) return CAPHN_EINVAL;
+    // row blocks: as many as keep the grid within one CTA per SM, at most 32 rows (16 warps) per CTA
+    const int ub = ceil_div(H, GD_UNITS);
+    int rb = kNumSMs / ub;
+    if (rb < 1) rb = 1;
+    int nw = ceil_div(ceil_div(B, rb), 2);
+    if (nw > GD_MAXW) nw = GD_MAXW;
+    if (nw < 1) nw = 1;
+    a.ldw = ((H >> 1) & 1) ? H : H + 2;                    // (ldw / 2) odd
+    a.nw = nw;
+    const size_t smem = ((size_t)3 * GD_UNITS * a.ldw + (size_t)2 * nw * H) * sizeof(float);
+    if (smem > 200 * 1024 || H > 416) return CAPHN_EINVAL;
+    CAPHN_CHECK(cudaFuncSetAttribute(gru_decode_step_kernel<SRC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    dim3 grid((unsigned)ub, (unsigned)ceil_div(B, 2 * nw));
+    gru_decode_step_kernel<SRC><<<grid, nw * 32, smem, (cudaStream_t)stream>>>(a, tokin, V);
+    CAPHN_RETURN_LAST();
+}
+
 extern "C" {
 
 // One greedy-decode step of DecoderGRU.infer (single layer).  GI != NULL: the input projection [B, 3H] (incl. b_ih) is given
@@ -191,26 +228,21 @@ extern "C" {
 int caphn_gru_decode_step(const float* GI, const float* pval, const int* pidx, int ldp, int nparts, const float* table,
                           const float* Whh, const float* bhh, const float* hprev, float* hnew, void* hi, void* lo, long Kp,
                           long long* tok, int B, int H, void* stream) {
-    if (B <= 0 || H <= 0 || (H & 1) || !Whh || !bhh || !hprev || !hnew || hnew == hprev) return CAPHN_EINVAL;
-    if (((uintptr_t)Whh & 7)) return CAPHN_EINVAL;
     if (!GI && (!pval || !pidx || !table || nparts <= 0 || nparts > ldp)) return CAPHN_EINVAL;
-    if (hi && Kp < H) return CAPHN_EINVAL;
-    // row blocks: as many as keep the grid within one CTA per SM, at most 32 rows (16 warps) per CTA
-    const int ub = ceil_div(H, GD_UNITS);
-    int rb = kNumSMs / ub;
-    if (rb < 1) rb = 1;
-    int nw = ceil_div(ceil_div(B, rb), 2);
-    if (nw > GD_MAXW) nw = GD_MAXW;
-    if (nw < 1) nw = 1;
-    const int ldw = ((H >> 1) & 1) ? H : H + 2;            // (ldw / 2) odd
-    GruDecArgs a{GI, pval, pidx, ldp, nparts, table, Whh, bhh, hprev, hnew, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo, Kp, tok,
-                 B, H, ldw, nw};
-    const size_t smem = ((size_t)3 * GD_UNITS * ldw + (size_t)2 * nw * H) * sizeof(float);
-    if (smem > 200 * 1024 || H > 416 || nparts > 256) return CAPHN_EINVAL;
-    CAPHN_CHECK(cudaFuncSetAttribute(gru_decode_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    dim3 grid((unsigned)ub, (unsigned)ceil_div(B, 2 * nw));
-    gru_decode_step_kernel<<<grid, nw * 32, smem, (cudaStream_t)stream>>>(a);
-    CAPHN_RETURN_LAST();
+    if (nparts > 256) return CAPHN_EINVAL;
+    const GruDecArgs a{GI, pval, pidx, ldp, nparts, table, Whh, bhh, hprev, hnew, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo, Kp,
+                       tok, B, H, 0, 0};
+    return gd_launch<GD_SRC_GREEDY>(a, nullptr, 0, stream);
+}
+
+// The same step with the input token given: row b's input projection is table[tok[b]] (an entry outside [0, V) reads row 0).
+// Beam search feeds the tokens its bookkeeping kernel chose (caphn_beam_step's prev_tok).  No partials, so no limit on V.
+int caphn_gru_decode_step_tok(const int* tok, int V, const float* table, const float* Whh, const float* bhh,
+                              const float* hprev, float* hnew, void* hi, void* lo, long Kp, int B, int H, void* stream) {
+    if (!tok || !table || V <= 0) return CAPHN_EINVAL;
+    const GruDecArgs a{nullptr, nullptr, nullptr, 0, 0, table, Whh, bhh, hprev, hnew, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo,
+                       Kp, nullptr, B, H, 0, 0};
+    return gd_launch<GD_SRC_TOK>(a, tok, V, stream);
 }
 
 }  // extern "C"

@@ -387,6 +387,96 @@ class DecoderGRU(nn.Module):
             ops.softmax_argmax(flat, want_probs=True, probs_out=flat, want_argmax=False)
         return outputs
 
+    @torch.no_grad()
+    def beam_search_batched(self, features, beam_size=3, end_sentence=2, max_steps=50, h0=None, sync_every=8):
+        """Beam search over the decoder step of ``infer`` for a whole batch, device-resident: ``features`` [B, E] (what
+        ``infer`` takes, ``image_encoder(pooled)``) -> list of B results, each the best complete token sequence (leading 0,
+        trailing ``end_sentence``) or ``None`` where a beam is still open after ``max_steps`` + 1 steps.  Same result format
+        and bookkeeping as ``AttentionGru.beam_search_batched`` (hypernet_attention.py:268-312: step 1 ranks row 0 only,
+        summed log-probabilities without length normalisation, finished beams leave, ties to the lower flat index).
+
+        Step 1 feeds ``features`` with ``h0`` (``None``: ``torch.rand(B, H)`` as ``infer`` draws it), each image's row
+        repeated for its k beams; later steps feed Emb[w] for the word w each beam chose -- the true word, without the
+        attention search's zero-embedding quirk (hypernet_attention.py:265-266), so ``beam_size=1`` gives ``infer``'s
+        greedy tokens.  First cell only, as in ``infer``.  Per step: one fused decode-step launch (projection-table row
+        -> GRU cell -> bf16 operand rows), the vocabulary GEMM and the bookkeeping kernel (csrc/beam.cu); the host reads
+        the results once at the end and peeks at an 'all images finished' flag every ``sync_every`` steps."""
+        streams.wait_pending()
+        W_ih, W_hh, b_ih, b_hh = [t.detach().contiguous() for t in self._cells()[0]]
+        if features.dim() != 2 or features.shape[1] != W_ih.shape[1]:
+            raise ValueError(f"beam_search_batched expects features [B, {W_ih.shape[1]}], got {list(features.shape)}")
+        H, V, k = self.hidden_size, self.vocab_size, int(beam_size)
+        if not 1 <= k <= 8:
+            raise ValueError(f"beam_size {k} outside [1, 8]")
+        if k > V:
+            raise ValueError(f"beam_size {k} exceeds the vocabulary size {V}")
+        feats = features.contiguous().float()
+        if h0 is None:
+            h0 = self._h0(feats)
+        B, dev = feats.shape[0], feats.device
+        R, L = B * k, int(max_steps) + 3
+        rep = lambda x: x.unsqueeze(1).expand(B, k, *x.shape[1:]).reshape(R, *x.shape[1:]).contiguous()
+        emb, fc_w, fc_b = self.embed.weight.detach(), self.fc_out.weight.detach(), self.fc_out.bias.detach()
+        xproj, vocab = ops.LinearPlan(W_ih, b_ih), ops.LinearPlan(fc_w, fc_b)
+        table = ops.linear(emb, W_ih, b_ih)                           # [V, 3H]: the input projection of every word
+        GI0 = rep(xproj(feats))                                       # rows b*k + j: beam j of image b
+        h = rep(h0.contiguous().float())
+        fused = ops.gru_decode_step_tok_ok(H)                         # else: table gather + GRU step as two launches
+        tc = ops._tc_ok(R, V, H)
+        hop = hhi = hlo = None                                        # hop: the new state's operand rows for the GEMM
+        if fused:
+            hout = torch.empty(R, H, device=dev, dtype=torch.float32)
+            if tc:
+                Kp = ops.round64(H)
+                hhi = torch.empty(R, Kp, device=dev, dtype=torch.bfloat16)
+                hlo = torch.empty(R, Kp, device=dev, dtype=torch.bfloat16) if ops.TC_SPLIT else None
+                hop = ops.SplitOperand(hhi, hlo, R, H, Kp)
+        else:
+            WhhT = ops.transpose_pad(W_hh, ops.round4(3 * H))
+        i32 = lambda *s: torch.zeros(*s, device=dev, dtype=torch.int32)
+        h_next = torch.zeros(R, H, device=dev, dtype=torch.float32)     # rows of finished beams stay finite
+        scores = torch.zeros(R, device=dev, dtype=torch.float32)
+        live = torch.full((B,), k, device=dev, dtype=torch.int32)
+        prev_tok, ncomp, failed = i32(R), i32(B), i32(B)
+        words = torch.empty(R, device=dev, dtype=torch.int64)          # (the attention search's input; unused here)
+        seq = [i32(R, L), i32(R, L)]                                  # histories start with the token 0
+        comp_score = torch.zeros(R, device=dev, dtype=torch.float32)
+        comp_seq, comp_len = i32(R, L), i32(R)
+        logits = torch.empty(R, V, device=dev, dtype=torch.float32)
+        n_steps = int(max_steps) + 1
+        for step in range(1, n_steps + 1):
+            if fused:
+                if step == 1:
+                    ops.gru_decode_step(GI0, None, None, 0, None, W_hh, b_hh, h, hout, hhi, hlo)
+                else:
+                    ops.gru_decode_step_tok(prev_tok, table, W_hh, b_hh, h, hout, hhi, hlo)
+            else:
+                GI = GI0 if step == 1 else ops.gather_rows(table, prev_tok.long())
+                hout = ops.gru_seq_fwd(GI, WhhT, b_hh, h, 1, save=False, want_bm=False)[0][1]
+            if hop is not None:
+                ops.gemm_tc(hop, vocab.operand(), bias=fc_b, out=logits)
+            else:
+                vocab(hout, out=logits)
+            ops._cabi.call("caphn_beam_step", logits.data_ptr(), hout.data_ptr(), h_next.data_ptr(), scores.data_ptr(),
+                           live.data_ptr(), prev_tok.data_ptr(), words.data_ptr(), seq[(step - 1) & 1].data_ptr(),
+                           seq[step & 1].data_ptr(), comp_score.data_ptr(), comp_seq.data_ptr(), comp_len.data_ptr(),
+                           ncomp.data_ptr(), failed.data_ptr(), B, k, V, H, L, step, int(end_sentence),
+                           int(step == n_steps), ops._stream())
+            h = h_next                                                # the decode step never writes the state it reads
+            if sync_every and step % sync_every == 0 and step < n_steps and int(live.max()) == 0:
+                break
+        nc, fl = ncomp.cpu().tolist(), failed.cpu().tolist()           # the one read-back of the search
+        cs, cq, cl = comp_score.cpu().view(B, k), comp_seq.cpu().view(B, k, L), comp_len.cpu().view(B, k)
+        out = []
+        for b in range(B):
+            if fl[b] or nc[b] == 0:
+                out.append(None)
+                continue
+            sc = cs[b, :nc[b]].tolist()
+            j = sc.index(max(sc))                                     # first maximum, as list.index does (:319-321)
+            out.append(cq[b, j, :int(cl[b, j])].tolist())
+        return out
+
 
 class DecoderRNN(DecoderGRU):
     """Drop-in for later.py:227 DecoderRNN: the LSTM captioner the pooled hypernet builds when ``type != 'gru'``
@@ -405,6 +495,10 @@ class DecoderRNN(DecoderGRU):
 
     def _h0(self, features):
         return torch.zeros(features.size(0), self.hidden_size, device=features.device, dtype=features.dtype)
+
+    def beam_search_batched(self, *args, **kwargs):
+        raise NotImplementedError("beam search is implemented for the GRU captioner (DecoderGRU) only: the LSTM cell state "
+                                  "would have to follow the beams, and there is no LSTM decode-step kernel")
 
     def forward_loss(self, features, captions, h0=None, ignore_index=None):
         if h0 is None:

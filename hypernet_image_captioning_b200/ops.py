@@ -855,6 +855,25 @@ def gru_decode_step(GI, pval, pidx, nparts, table, W_hh, b_hh, hprev, hnew, hi=N
     return hnew
 
 
+def gru_decode_step_tok_ok(H):
+    """The token-fed decode step reads no arg-max partials: only the shared-memory bound of gru_decode_step_ok (H even,
+    <= 398) applies, for any V."""
+    return H % 2 == 0 and (96 * (H + 2) + 32 * H) * 4 <= 200 * 1024
+
+
+def gru_decode_step_tok(tok, table, W_hh, b_hh, hprev, hnew, hi=None, lo=None):
+    """gru_decode_step with the input token given (csrc/gru_decode.cu, caphn_gru_decode_step_tok): row b's input projection
+    is table[tok[b]] (int32 tokens; one outside [0, V) reads row 0), then the GRU cell and the operand rows as there."""
+    _chk(tok, torch.int32)
+    B, H = hprev.shape
+    assert W_hh.is_contiguous() and hprev.is_contiguous() and hnew.is_contiguous() and hnew.data_ptr() != hprev.data_ptr()
+    assert table.is_contiguous() and table.shape[1] == 3 * H and tok.is_contiguous() and tok.numel() == B
+    _cabi.call("caphn_gru_decode_step_tok", tok.data_ptr(), table.shape[0], table.data_ptr(), W_hh.data_ptr(),
+               b_hh.data_ptr(), hprev.data_ptr(), hnew.data_ptr(), _p(hi), _p(lo), hi.stride(0) if hi is not None else 0, B,
+               H, _stream())
+    return hnew
+
+
 def attstep_h_operand(lw, B, H, Fd, t_done):
     """The hidden state h_{t_done} as the bf16 hi/lo operand rows the step-split gates kernel has just written into its
     workspace for the next step's U kernel (attgru_step.cu: hsp buffers) -- the A operand of the vocabulary projection,

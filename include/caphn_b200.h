@@ -386,6 +386,12 @@ int caphn_gru_decode_step(const float* GI, const float* pval, const int* pidx, i
                           const float* Whh, const float* bhh, const float* hprev, float* hnew, void* hi, void* lo, long Kp,
                           long long* tok, int B, int H, void* stream);
 
+/* caphn_gru_decode_step with the input token given (beam search: the prev_tok of caphn_beam_step): row b's input projection
+ * is row tok[b] of table [V, 3H]; an entry outside [0, V) reads row 0.  No arg-max partials are read, so V is not bounded;
+ * the H limits of caphn_gru_decode_step apply.  hnew must not alias hprev. */
+int caphn_gru_decode_step_tok(const int* tok, int V, const float* table, const float* Whh, const float* bhh,
+                              const float* hprev, float* hnew, void* hi, void* lo, long Kp, int B, int H, void* stream);
+
 /* Weights-resident GRU recurrence without a cluster (csrc/gru_resident.cu): one CTA per 4 batch rows keeps the whole generated
  * W_hh as thread-private weight vectors (shared memory + registers), so every step is CTA-local.  Same contract as
  * caphn_gru_cluster_fwd / _bwd (nn.GRUCell per step + BPTT, later.py:411,418); *ok of the plan call says whether H fits. */
