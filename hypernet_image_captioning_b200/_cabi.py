@@ -51,8 +51,6 @@ SIGNATURES = {
     "caphn_lstm_seq_bwd": [P, P, P, I, P, P, P, I, I, I, I, P],
     "caphn_attgru_seq_fwd": [P] * 14 + [L] + [P] * 5 + [I] * 9 + [P],
     "caphn_attgru_seq_bwd": [P] * 23 + [I] * 7 + [P],
-    "caphn_attgru_cluster_plan": [I, I, I, P],
-    "caphn_attgru_cluster_fwd": [P] * 14 + [L] + [P] * 5 + [I] * 8 + [P],
     "caphn_attstep_pack_size": [I, I, I, I, P, P],
     "caphn_attstep_pack": [P, P, P, I, I, I, P, P],
     "caphn_attstep_fwd": [P] * 13 + [L] + [P] * 5 + [I] * 8 + [P],
@@ -64,8 +62,6 @@ SIGNATURES = {
     "caphn_split_bf16_gather": [P, L, P, L, I, P, P, L, P],
     "caphn_split_bf16_batched": [P, L, L, I, I, I, P, P, L, P],
     "caphn_group_colsum": [P, L, P, I, I, I, I, P, L, P],
-    "caphn_gemm_tc_lse": [P, P, L, I, P, P, L, I, L, P, L, P, I, I, P, P, I, P, P],
-    "caphn_ce_fwd_partials": [P, P, I, I, P, L, P, L, I, LL, P, P, P, P],
     "caphn_gemm_tc_amax": [P, P, L, I, P, P, L, I, L, P, L, P, I, I, P, P, I, P, P],
     "caphn_argmax_finish_gather": [P, P, I, I, L, P, I, P, P, L, P],
     "caphn_beam_step": [P] * 14 + [I] * 8 + [P],
@@ -90,7 +86,6 @@ SIGNATURES = {
     "caphn_bleu_counts": [P, P, I, P, P, I, I, I, P, P],
     "caphn_ce_fwd_split": [P, L, P, L, I, I, LL, P, P, P, P, P, L, P],
     "caphn_gemm_tc_scaled": [P, P, L, I, P, P, L, I, L, P, L, P, I, I, I, P, P, P],
-    "caphn_gemm_tc_prof": [P, P, L, I, P, P, L, I, L, P, L, P, I, I, I, P, P],
     "caphn_gru_decode_step": [P, P, P, I, I, P, P, P, P, P, P, P, L, P, I, I, P],
     "caphn_gru_decode_step_tok": [P, I, P, P, P, P, P, P, P, L, I, I, P],
     "caphn_gru_resident_plan": [I, P],

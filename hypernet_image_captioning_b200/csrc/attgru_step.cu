@@ -564,7 +564,7 @@ static int attstep_fwd_impl(const float* Kp, const float* f, const float* GIw, c
     // double-buffered CTA per SM
     int agrid = B < 2 * kNumSMs ? B : 2 * kNumSMs, nbuf = 1;
     int rpc = (B + agrid - 1) / agrid;
-    if (2 * (as_smem(P, H, F, rpc, 1) + 1024) > 227 * 1024 || getenv("CAPHN_ATT_DOUBLE_BUFFER")) {
+    if (2 * (as_smem(P, H, F, rpc, 1) + 1024) > 227 * 1024) {
         agrid = as_grid(B, P, H, F); rpc = (B + agrid - 1) / agrid; nbuf = 2;
     }
     const bool small_tiles = tiles && tile_rows <= YS_NB_SMALL;
@@ -579,25 +579,24 @@ static int attstep_fwd_impl(const float* Kp, const float* f, const float* GIw, c
         attstep_split_kernel<<<ceil_div(B * (KP / 2), 256), 256, 0, st>>>(Hall + t0 * BH, B, H, KP, hbuf(t0), hbuf(t0 + 1));
         CAPHN_LAUNCH_CHECK();
     }
-    static const bool pdl = []() { const char* e = getenv("CAPHN_PDL"); return !(e && e[0] == '0'); }();
     for (int t = t0; t < t1; ++t) {
         float* ut = Upre ? Upre + t * BH : ubuf;
         AttStepU u{(const uint4*)pack, bu, hbuf(t), ut, B, H, NUT, NKT, KP};
         CAPHN_CHECK(launch_pdl(attstep_u_kernel, dim3(ceil_div(NUT, US_WARPS), ceil_div(B, US_NB)), dim3(US_THREADS), usmem,
-                               st, pdl && !(t == t0 && resume), u));
+                               st, !(t == t0 && resume), u));
         ++caphn_launch_counter;
         AttStepA x{Kp, f, va, bv, ut, attn, ctx + (long)t * B * ldctx, ldctx, csp, B, T, t, P, H, F, KP, rpc, nbuf};
-        CAPHN_CHECK(launch_pdl(attstep_attn_kernel, dim3(agrid), dim3(AS_THREADS), asmem, st, pdl, x));
+        CAPHN_CHECK(launch_pdl(attstep_attn_kernel, dim3(agrid), dim3(AS_THREADS), asmem, st, true, x));
         ++caphn_launch_counter;
         AttStepY y{csp, hbuf(t), hbuf(t + 1), Hall + t * BH, GIw + (long)t * B * 3 * H, (const uint4*)pack, bhh,
                    Hall + (t + 1) * BH, Hbm, R ? R + t * BH : nullptr, Z ? Z + t * BH : nullptr,
                    Nn ? Nn + t * BH : nullptr, GHN ? GHN + t * BH : nullptr, B, T, t, H, NUT, NKT, KP,
                    (const int4*)tiles, pack_elems(H, F)};
         if (small_tiles) {
-            CAPHN_CHECK(launch_pdl(attstep_gates_kernel<YS_NB_SMALL>, dim3(NUT, ntiles), dim3(YS_THREADS), ysmem, st, pdl, y));
+            CAPHN_CHECK(launch_pdl(attstep_gates_kernel<YS_NB_SMALL>, dim3(NUT, ntiles), dim3(YS_THREADS), ysmem, st, true, y));
         } else {
             CAPHN_CHECK(launch_pdl(attstep_gates_kernel<YS_NB>, dim3(NUT, tiles ? ntiles : ceil_div(B, YS_NB)),
-                                   dim3(YS_THREADS), ysmem, st, pdl, y));
+                                   dim3(YS_THREADS), ysmem, st, true, y));
         }
         ++caphn_launch_counter;
     }

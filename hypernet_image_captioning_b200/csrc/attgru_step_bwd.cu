@@ -651,7 +651,7 @@ static int attstep_bwd_impl(const float* dHbm, const float* dattn, const float* 
     const uint4* p2 = p1 + (long)NFT * NKT3 * 64;
     int agrid = B < 2 * kNumSMs ? B : 2 * kNumSMs, nbuf = 1;
     int rpc = (B + agrid - 1) / agrid;
-    if (2 * (ba_smem(P, H, F, rpc, 1) + 1024) > 227 * 1024 || getenv("CAPHN_ATT_DOUBLE_BUFFER")) {
+    if (2 * (ba_smem(P, H, F, rpc, 1) + 1024) > 227 * 1024) {
         agrid = ba_grid(B, P, H, F); rpc = (B + agrid - 1) / agrid; nbuf = 2;
     }
     const size_t s1 = g1_smem(KP), s2 = g2_smem(KP3), sa = ba_smem(P, H, F, rpc, nbuf), sd = bd_smem(P, H, T);
@@ -664,35 +664,34 @@ static int attstep_bwd_impl(const float* dHbm, const float* dattn, const float* 
     CAPHN_CHECK(cudaFuncSetAttribute(attbwd_gemm_kernel<G2_NB_SMALL, G2_PF_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s2s));
     CAPHN_CHECK(cudaFuncSetAttribute(attbwd_attn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sa));
     CAPHN_CHECK(cudaFuncSetAttribute(attbwd_dk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sd));
-    static const bool pdl = []() { const char* e = getenv("CAPHN_PDL"); return !(e && e[0] == '0'); }();
     const int NG1 = ceil_div(NFT, G2_WARPS), NG2 = ceil_div(NUT, G2_WARPS);
     for (int t = T - 1; t >= 0; --t) {
         BwdG1 g1{p0, dusp, dhp, keep, dHbm, R + t * BH, Z + t * BH, Nn + t * BH, GHN + t * BH, Hall + t * BH,
                  dGI + (long)t * B * 3 * H, dGH + (long)t * B * 3 * H, gisp, ghsp, nullptr, B, T, t, H, NUT, NKT, KP, KP3,
                  t == T - 1 ? 0 : 1};
         CAPHN_CHECK(launch_pdl(attbwd_gate_kernel, dim3(NUT, ceil_div(B, G1_NB)), dim3(G1_THREADS), s1, st,
-                               pdl && t != T - 1, g1));
+                               t != T - 1, g1));
         ++caphn_launch_counter;
         BwdG2 g2{p1, p2, gisp, ghsp, dCTX + (long)t * B * F, dhp, B, H, F, NUT, NFT, NKT3, KP3, NG1, (const int4*)tiles,
                  pb / 16};
         if (small_tiles) {
-            CAPHN_CHECK(launch_pdl(attbwd_gemm_kernel<G2_NB_SMALL, G2_PF_SMALL>, dim3(NG1 + NG2, ntiles), dim3(G2_THREADS), s2s, st, pdl, g2));
+            CAPHN_CHECK(launch_pdl(attbwd_gemm_kernel<G2_NB_SMALL, G2_PF_SMALL>, dim3(NG1 + NG2, ntiles), dim3(G2_THREADS), s2s, st, true, g2));
         } else {
             CAPHN_CHECK(launch_pdl(attbwd_gemm_kernel<G2_NB, G2_PF_BIG>, dim3(NG1 + NG2, tiles ? ntiles : ceil_div(B, G2_NB)),
-                                   dim3(G2_THREADS), s2, st, pdl, g2));
+                                   dim3(G2_THREADS), s2, st, true, g2));
         }
         ++caphn_launch_counter;
         BwdA ba{Kp, f, va, dCTX + (long)t * B * F, attn, dattn, Upre + t * BH, dS, dU + t * BH, dusp, dbv,
                 B, T, t, P, H, F, KP, rpc, nbuf};
-        CAPHN_CHECK(launch_pdl(attbwd_attn_kernel, dim3(agrid), dim3(BA_THREADS), sa, st, pdl, ba));
+        CAPHN_CHECK(launch_pdl(attbwd_attn_kernel, dim3(agrid), dim3(BA_THREADS), sa, st, true, ba));
         ++caphn_launch_counter;
     }
     BwdG1 g1{p0, dusp, dhp, keep, dHbm, R, Z, Nn, GHN, Hall, dGI, dGH, gisp, ghsp, dh0, B, T, 0, H, NUT, NKT, KP, KP3, 2};
-    CAPHN_CHECK(launch_pdl(attbwd_gate_kernel, dim3(NUT, ceil_div(B, G1_NB)), dim3(G1_THREADS), s1, st, pdl, g1));
+    CAPHN_CHECK(launch_pdl(attbwd_gate_kernel, dim3(NUT, ceil_div(B, G1_NB)), dim3(G1_THREADS), s1, st, true, g1));
     ++caphn_launch_counter;
     BwdD bd{Kp, va, Upre, dS, dK, dva, B, T, P, H};
     const int dgrid = B < kNumSMs ? B : kNumSMs;
-    CAPHN_CHECK(launch_pdl(attbwd_dk_kernel, dim3(dgrid), dim3(BD_THREADS), sd, st, pdl, bd));
+    CAPHN_CHECK(launch_pdl(attbwd_dk_kernel, dim3(dgrid), dim3(BD_THREADS), sd, st, true, bd));
     ++caphn_launch_counter;
     return (int)cudaGetLastError();
 }

@@ -76,35 +76,6 @@ __global__ void __launch_bounds__(CE_THREADS) ce_fwd_kernel(const float* __restr
     }
 }
 
-// Cross-entropy forward from the log-sum-exp partials the logits GEMM's epilogue produced (caphn_gemm_tc_lse): one warp per
-// row merges the nparts (m, s) pairs -> lse, reads the ONE logit it needs (the target's) and writes row_loss / row_valid.
-__global__ void __launch_bounds__(128) ce_from_partials_kernel(const float* __restrict__ pm, const float* __restrict__ ps,
-                                                                int ldp, int nparts, const float* __restrict__ X, long ld,
-                                                                const long long* __restrict__ tgt, long M, int has_ignore,
-                                                                long long ignore, float* __restrict__ lse,
-                                                                float* __restrict__ row_loss, float* __restrict__ row_valid) {
-    const long m = (long)blockIdx.x * 4 + (threadIdx.x >> 5);
-    const int lane = threadIdx.x & 31;
-    if (m >= M) return;
-    float mx = -INFINITY;
-    for (int q = lane; q < nparts; q += 32) mx = fmaxf(mx, pm[m * ldp + q]);
-    mx = warp_max(mx);
-    float s = 0.f;
-    for (int q = lane; q < nparts; q += 32) {
-        const float pmq = pm[m * ldp + q];
-        if (pmq > -INFINITY) s += ps[m * ldp + q] * expf(pmq - mx);
-    }
-    s = warp_sum(s);
-    if (lane == 0) {
-        const float l = mx + logf(s);
-        lse[m] = l;
-        const long long t = tgt[m];
-        const bool valid = !(has_ignore && t == ignore);
-        row_valid[m] = valid ? 1.f : 0.f;
-        row_loss[m] = valid ? (l - X[m * ld + t]) : 0.f;
-    }
-}
-
 // out[0] = sum(row_loss) / sum(row_valid)   out[1] = sum(row_valid)        (single CTA; deterministic)
 __global__ void __launch_bounds__(1024) ce_finish_kernel(const float* __restrict__ row_loss,
                                                          const float* __restrict__ row_valid, long M,
@@ -652,19 +623,6 @@ int caphn_ce_fwd_split(const float* X, long ld, const long long* tgt, long M, in
     CAPHN_CHECK(cudaFuncSetAttribute(ce_fwd_split_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     ce_fwd_split_kernel<<<(unsigned)M, CE_THREADS, smem, st>>>(X, ld, tgt, V, has_ignore, ignore, lse, scratch, scratch + M,
                                                                (__nv_bfloat16*)hi, (__nv_bfloat16*)lo, Vp);
-    CAPHN_LAUNCH_CHECK();
-    ce_finish_kernel<<<1, 1024, 0, st>>>(scratch, scratch + M, M, lossbuf);
-    CAPHN_RETURN_LAST();
-}
-
-// caphn_ce_fwd from the (max, sum-exp) partials of caphn_gemm_tc_lse instead of a pass over X: same outputs.
-int caphn_ce_fwd_partials(const float* pm, const float* ps, int ldp, int nparts, const float* X, long ld,
-                          const long long* tgt, long M, int has_ignore, long long ignore, float* lse, float* scratch,
-                          float* lossbuf, void* stream) {
-    if (M <= 0 || nparts <= 0 || nparts > ldp) return CAPHN_EINVAL;
-    cudaStream_t st = (cudaStream_t)stream;
-    ce_from_partials_kernel<<<(unsigned)((M + 3) / 4), 128, 0, st>>>(pm, ps, ldp, nparts, X, ld, tgt, M, has_ignore, ignore,
-                                                                      lse, scratch, scratch + M);
     CAPHN_LAUNCH_CHECK();
     ce_finish_kernel<<<1, 1024, 0, st>>>(scratch, scratch + M, M, lossbuf);
     CAPHN_RETURN_LAST();

@@ -73,13 +73,6 @@ __device__ __forceinline__ bool elect_one() {
         : "=r"(pred));
     return pred != 0;
 }
-// L2 prefetch of one TMA box (no shared memory involved): turns the DRAM latency of a streamed operand into L2 latency for the
-// load that follows a few k-blocks later
-__device__ __forceinline__ void tma_prefetch_2d(const CUtensorMap* tmap, int x, int y) {
-    asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];"
-                 ::"l"(reinterpret_cast<uint64_t>(tmap)), "r"(x), "r"(y)
-                 : "memory");
-}
 __device__ __forceinline__ void tcgen05_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tcgen05_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 
@@ -137,7 +130,6 @@ __device__ __forceinline__ void tma_store_2d(const CUtensorMap* tmap, const void
 }
 __device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void tma_store_wait_read1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
 __device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 __device__ __forceinline__ void red_add_v2(float* p, float a, float b) {
     asm volatile("red.global.add.v2.f32 [%0], {%1, %2};" ::"l"(p), "f"(a), "f"(b) : "memory");
@@ -188,10 +180,6 @@ struct TcParams {
     // reduces the columns it reads of every row to (max, column) and writes them to amax_val / amax_idx [M, amax_ld],
     // slot 2 * n-tile + warp half; a tiny kernel finishes the reduction (and gathers the next input row).  null: off.
     float* amax_val; int* amax_idx; int amax_ld;
-    // stat_mode 1: arg-max partials (above).  2: log-sum-exp partials for the fused cross-entropy -- amax_val = running row
-    // max m, amax_idx = the bits of s = sum exp(x - m) over the columns this warp read (SURVEY K7+K8: the loss statistics
-    // come out of the logits GEMM instead of a second pass over the 0.4 GB of logits).
-    int stat_mode;
     int M, N, num_kb, relu;
     int BN;          // N tile (multiple of 16, <= 256)
     int splitk;      // K split factor; > 1 => epilogue adds atomically into a zero-initialised C
@@ -210,17 +198,6 @@ struct TcParams {
     // of a product that was bound by it (1.17 GB for 0.4 GB of output at M=10240, N=9684, K=150).
     int astat;
     int a_slab_bytes;
-    // staging buffers per epilogue warp (TMA-store epilogue): 2 = the warp fills one 4 KB tile while the bulk store of the
-    // previous one is still reading the other (the wait for that read was the largest epilogue stall in the ncu source view)
-    int stg_bufs;
-    // k-blocks by which an L2 prefetch of the A operand runs ahead of its load (0 = off; long-K products whose A streams
-    // from DRAM through a 2-3 stage ring)
-    int pf_dist;
-    // diagnostics (caphn_gemm_tc_prof; NULL otherwise): 16 cycle counters per CTA -- [0] producer waiting for a free stage,
-    // [1] producer waiting for the A slab to be free, [2] MMA thread waiting for operands, [3] MMA thread waiting for a free
-    // accumulator, [4] MMA thread total, [5] epilogue warp 4 waiting for an accumulator, [6] waiting for bulk-store reads,
-    // [7] epilogue warp 4 total, [8] producer total, [9] units of this CTA
-    long long* prof;
 };
 
 __device__ __forceinline__ UnitInfo decode_unit(const TcParams& p, int unit, int tiles_m, int BN) {
@@ -261,7 +238,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     uint8_t* tiles = smem;
     float* stg = reinterpret_cast<float*>(smem + (size_t)p.a_slab_bytes + (size_t)p.stages * p.stage_bytes);
-    uint64_t* full = reinterpret_cast<uint64_t*>(stg + p.stg_bufs * STG_FLOATS_V2);
+    uint64_t* full = reinterpret_cast<uint64_t*>(stg + (p.splitk > 1 ? 0 : STG_FLOATS_V2));   // split-K: no staging
     uint64_t* empty = full + MAX_STAGES;
     uint64_t* tfull = empty + MAX_STAGES;
     uint64_t* tempty = tfull + 2;
@@ -316,14 +293,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
         uint32_t phase = 0;
         int cur_a0 = -1;
         uint32_t a_it = 0;
-        long long w_empty = 0, w_aempty = 0;
-        const long long t_start = clock64();
         for (int ui = 0, unit = u_first; ui < u_count; ++ui, unit += u_step) {
             const UnitInfo u = decode_unit(p, unit, tiles_m, BN);
             if (p.astat && u.a0 != cur_a0) {       // new m-tile: (re)load the A slab once the MMAs reading the old one are done
-                const long long tw = clock64();
                 mbar_wait(aempty, (a_it & 1) ^ 1);
-                w_aempty += clock64() - tw;
                 if (elect_one()) {
                     mbar_expect_tx(afull, (uint32_t)p.a_slab_bytes);
                     for (int i = 0; i < u.nkb; ++i) {
@@ -337,23 +310,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
             }
             for (int i = 0; i < u.nkb; ++i) {
                 const int ka = u.ka0 + i * BK, kbk = u.kb0 + i * BK;
-                const long long tw = clock64();
                 mbar_wait(empty + stage, phase ^ 1);
-                w_empty += clock64() - tw;
                 uint8_t* st = tiles + (size_t)stage * p.stage_bytes;
                 if (elect_one()) {
-                    if (p.pf_dist > 0 && i + p.pf_dist < u.nkb) {      // A tiles of a later k-block -> L2
-                        const int kp = ka + p.pf_dist * BK;
-                        if (!p.a_mn) {
-                            tma_prefetch_2d(&tmAh, kp, u.a0);
-                            if (SPLIT) tma_prefetch_2d(&tmAl, kp, u.a0);
-                        } else {
-                            for (int h = 0; h < BM / 64; ++h) {
-                                tma_prefetch_2d(&tmAh, u.a0 + h * 64, kp);
-                                if (SPLIT) tma_prefetch_2d(&tmAl, u.a0 + h * 64, kp);
-                            }
-                        }
-                    }
                     mbar_expect_tx(full + stage, (uint32_t)p.stage_bytes);
                     // K-major operand: one box [64 k x rows].  MN-major operand: boxes of [64 mn x 64 k] (8 KiB each).
                     if (p.astat) {
@@ -381,10 +340,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
                 if (++stage == p.stages) { stage = 0; phase ^= 1; }
             }
         }
-        if (p.prof && lane == 0) {
-            long long* pr = p.prof + (long)blockIdx.x * 16;
-            pr[0] = w_empty; pr[1] = w_aempty; pr[8] = clock64() - t_start; pr[9] = u_count;
-        }
     } else if (warp == 1) {
         // MMA issuer: converged warp, one elected lane issues the tcgen05.mma / tcgen05.commit instructions
         const uint32_t idesc = make_idesc(BM, BN, p.a_mn != 0, p.b_mn != 0);
@@ -397,18 +352,12 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
         int cur_a0 = -1;
         uint32_t a_it = 0;
         const uint32_t slab_base = smem_u32(slab);
-        long long w_full = 0, w_tempty = 0;
-        const long long t_start = clock64();
         for (int ui = 0, unit = u_first; ui < u_count; ++ui, unit += u_step, ++it) {
             const UnitInfo u = decode_unit(p, unit, tiles_m, BN);
             const int kb0 = 0, kb1 = u.nkb;
             const int as = it & 1;
             const uint32_t aph = (it >> 1) & 1;
-            {
-                const long long tw = clock64();
-                mbar_wait(tempty + as, aph ^ 1);
-                w_tempty += clock64() - tw;
-            }
+            mbar_wait(tempty + as, aph ^ 1);
             tcgen05_fence_after();
             if (p.astat && u.a0 != cur_a0) {
                 mbar_wait(afull, a_it & 1);
@@ -418,11 +367,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
             }
             const uint32_t tmem_d = tmem_base + (uint32_t)(as * BN);
             for (int kb = kb0; kb < kb1; ++kb) {
-                {
-                    const long long tw = clock64();
-                    mbar_wait(full + stage, phase);
-                    w_full += clock64() - tw;
-                }
+                mbar_wait(full + stage, phase);
                 tcgen05_fence_after();
                 const uint32_t sbase = smem_u32(tiles + (size_t)stage * p.stage_bytes);
                 const uint32_t abase = p.astat ? slab_base + (uint32_t)(kb * ablk) : sbase;
@@ -463,33 +408,21 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
             }
             __syncwarp();
         }
-        if (p.prof && lane == 0) {
-            long long* pr = p.prof + (long)blockIdx.x * 16;
-            pr[2] = w_full; pr[3] = w_tempty; pr[4] = clock64() - t_start;
-        }
     } else if (warp >= 4) {
         const int ew = warp - 4;
         const int q = warp & 3;                   // TMEM lane quadrant this warp may access (warp id % 4)
         const int half = ew >> 2;                 // two warps per quadrant split the 32-column chunks
-        float* const st0 = stg + ew * (p.stg_bufs * 32 * STG_STRIDE);
-        float* st = st0;
-        int sti = 0;                              // TMA-store items issued by this warp (selects the staging buffer)
+        float* const st = stg + ew * (32 * STG_STRIDE);
         const int nchunks = (BN + 31) / 32;
         const bool atomic = p.splitk > 1;
         const bool vec = !atomic && ((p.ldc & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.C) & 15) == 0);
         int it = 0;
         const float alpha = p.scale_num ? p.scale_num[0] / fmaxf(p.scale_den ? p.scale_den[0] : 1.f, 1.f) : 1.f;
-        long long w_tfull = 0, w_store = 0;
-        const long long t_start = clock64();
         for (int ui = 0, unit = u_first; ui < u_count; ++ui, unit += u_step, ++it) {
             const UnitInfo u = decode_unit(p, unit, tiles_m, BN);
             const int as = it & 1;
             const uint32_t aph = (it >> 1) & 1;
-            {
-                const long long tw = clock64();
-                mbar_wait(tfull + as, aph);
-                w_tfull += clock64() - tw;
-            }
+            mbar_wait(tfull + as, aph);
             tcgen05_fence_after();
             const int row0 = u.a0 + q * 32;           // (non-grouped TMA-store path only: global row of this warp's first row)
             const int rl0 = q * 32;                   // first tile-local row of this warp
@@ -499,9 +432,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
             const int* rmap = p.rowmap ? p.rowmap + u.map0 : nullptr;
             int last_c = half;
             while (last_c + 2 < nchunks) last_c += 2;
-            float am_best = -INFINITY;            // arg-max partial (mode 1) / running max (mode 2) of row (rl0 + lane) over this warp's chunks
+            float am_best = -INFINITY;            // arg-max partial of row (rl0 + lane) over this warp's chunks
             int am_idx = 0x7fffffff;
-            float lse_s = 0.f;                    // mode 2: sum exp(x - am_best)
             if (half >= nchunks) {                 // nothing to read for this warp: release the stage immediately
                 tcgen05_fence_before();
                 if (lane == 0) mbar_arrive(tempty + as);
@@ -565,47 +497,23 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
                     }
                     continue;
                 }
-                if (p.amax_val && p.stat_mode == 1) {         // lane = row: 32 consecutive columns of it are in r[]
+                if (p.amax_val) {                             // lane = row: 32 consecutive columns of it are in r[]
                     const float bl = (add_bias && lane < cvalid) ? biasp[cl0 + lane] : 0.f;
 #pragma unroll
-                    for (int j = 0; j < 32; ++j) {
-                        const float v = __uint_as_float(r[j]) + __shfl_sync(0xffffffffu, bl, j);
-                        r[j] = __float_as_uint(v);            // the bias is in: the store paths below must not add it again
-                        if (j < cvalid && v > am_best) { am_best = v; am_idx = colbase + j; }   // ascending columns: first max wins
+                    for (int j = 0; j < 32; ++j)              // the bias is in: the store paths below must not add it again
+                        r[j] = __float_as_uint(__uint_as_float(r[j]) + __shfl_sync(0xffffffffu, bl, j));
+                    // a separate scan: fused into the loop above, the kernel compiled to 18-24 more registers
+#pragma unroll
+                    for (int j = 0; j < 32; ++j) {            // ascending columns: first max wins
+                        const float v = __uint_as_float(r[j]);
+                        if (j < cvalid && v > am_best) { am_best = v; am_idx = colbase + j; }
                     }
                     bias_done = true;
-                } else if (p.amax_val) {                      // stat_mode 2: running (max, sum exp) of the row
-                    const float bl = (add_bias && lane < cvalid) ? biasp[cl0 + lane] : 0.f;
-                    float cm = -INFINITY;
-#pragma unroll
-                    for (int j = 0; j < 32; ++j) {
-                        const float v = __uint_as_float(r[j]) + __shfl_sync(0xffffffffu, bl, j);
-                        r[j] = __float_as_uint(v);            // the bias is in: the store paths below must not add it again
-                        if (j < cvalid) cm = fmaxf(cm, v);
-                    }
-                    bias_done = true;
-                    if (cm > -INFINITY) {
-                        const float nm = fmaxf(am_best, cm);
-                        float acc = 0.f;
-#pragma unroll
-                        for (int j = 0; j < 32; ++j)
-                            if (j < cvalid) acc += __expf(__uint_as_float(r[j]) - nm);
-                        lse_s = lse_s * __expf(am_best - nm) + acc;       // exp(-inf) = 0 on the first chunk
-                        am_best = nm;
-                    }
                 }
                 if constexpr (TMA_STORE) {
                     // chunks that lie fully inside the N tile (TMA clips at the matrix edge, not at the tile edge)
                     if (!atomic && BN - c * 32 >= 32) {
-                        const long long tw = clock64();
-                        if (p.stg_bufs == 2) {
-                            st = st0 + (sti & 1) * (32 * STG_STRIDE);
-                            if (lane == 0) tma_store_wait_read1();     // the store before the previous one has read `st`
-                        } else {
-                            if (lane == 0) tma_store_wait_read();      // the previous store has finished reading `st`
-                        }
-                        w_store += clock64() - tw;
-                        ++sti;
+                        if (lane == 0) tma_store_wait_read();          // the previous store has finished reading `st`
                         __syncwarp();
                         const float bl = (add_bias && !bias_done && lane < cvalid) ? biasp[cl0 + lane] : 0.f;
 #pragma unroll
@@ -629,7 +537,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
                     }
                     if (lane == 0) tma_store_wait_read();              // legacy path below reuses the staging tile
                     __syncwarp();
-                    st = st0;
                 }
 #pragma unroll
                 for (int j4 = 0; j4 < 8; ++j4)   // row = lane; float4 slot j4 lives at (j4 ^ (row & 7)): conflict-free
@@ -691,15 +598,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
             if (p.amax_val && rl0 + lane < u.m_valid) {
                 const long o = (long)(u.a0 + rl0 + lane) * p.amax_ld + 2 * (u.b0 / BN) + half;
                 p.amax_val[o] = am_best;
-                p.amax_idx[o] = p.stat_mode == 2 ? __float_as_int(lse_s) : am_idx;
+                p.amax_idx[o] = am_idx;
             }
         }
         if constexpr (TMA_STORE) {
             if (lane == 0) tma_store_wait_all();       // shared memory must outlive the bulk stores that read it
-        }
-        if (p.prof && ew == 0 && lane == 0) {
-            long long* pr = p.prof + (long)blockIdx.x * 16;
-            pr[5] = w_tfull; pr[6] = w_store; pr[7] = clock64() - t_start;
         }
     }
     tcgen05_fence_before();
@@ -842,8 +745,8 @@ int caphn_split_bf16_t(const float* src, long lds, int R, int C, void* hi, void*
 // Alo == Blo == NULL selects plain bf16.  splitk: 0 = automatic, 1 = none, > 1 = split K, partial tiles added atomically.
 static int gemm_tc_impl(const void* Ahi, const void* Alo, long a_ld, int a_mn, const void* Bhi, const void* Blo, long b_ld,
                         int b_mn, long K, float* C, long ldc, const float* bias, int M, int N, int relu, int splitk,
-                        float* amax_val, int* amax_idx, int amax_ld, void* stream, int* bn_used = nullptr, int stat_mode = 1,
-                        const float* scale_num = nullptr, const float* scale_den = nullptr, long long* prof = nullptr) {
+                        float* amax_val, int* amax_idx, int amax_ld, void* stream, int* bn_used = nullptr,
+                        const float* scale_num = nullptr, const float* scale_den = nullptr) {
     if (M <= 0 || N <= 0 || K <= 0 || ((Alo == nullptr) != (Blo == nullptr))) return CAPHN_EINVAL;
     if (scale_den && !scale_num) return CAPHN_EINVAL;
     if (amax_val && (!amax_idx || splitk > 1 || relu)) return CAPHN_EINVAL;
@@ -857,7 +760,10 @@ static int gemm_tc_impl(const void* Ahi, const void* Alo, long a_ld, int a_mn, c
     p.C = C; p.ldc = ldc; p.bias = bias; p.M = M; p.N = N; p.relu = relu; p.a_mn = a_mn ? 1 : 0; p.b_mn = b_mn ? 1 : 0;
     p.num_kb = (int)((K + tc::BK - 1) / tc::BK);
     p.K = (int)K;
-    p.scale_num = scale_num; p.scale_den = scale_den; p.prof = prof;
+    p.scale_num = scale_num; p.scale_den = scale_den;
+    // A-stationary schedule (see TcParams::astat), used where the shape allows it; CAPHN_TC_ASTAT=0 switches it off
+    const char* ae = getenv("CAPHN_TC_ASTAT");
+    const bool astat_on = !(ae && atoi(ae) == 0);
     // N tile: one tile when N <= 256 (rounded up to 16, or to 64 for an MN-major B whose boxes are 64 wide), else 128
     if (N <= 256) {
         p.BN = b_mn ? ((N + 63) / 64) * 64 : ((N + 15) / 16) * 16;
@@ -868,8 +774,7 @@ static int gemm_tc_impl(const void* Ahi, const void* Alo, long a_ld, int a_mn, c
         // With many waves the quantisation loss is small and BN = 128 keeps 3 operand stages in flight: left alone.
         const int step = b_mn ? 64 : 16;
         const long tm = ceil_div(M, tc::BM);
-        static const bool auto_bn = [] { const char* e = getenv("CAPHN_TC_BN_AUTO"); return !(e && e[0] == '0'); }();
-        const bool few_waves = auto_bn && tm * ceil_div(N, 128) <= 8L * kNumSMs;
+        const bool few_waves = tm * ceil_div(N, 128) <= 8L * kNumSMs;
         long best_cost = -1;
         p.BN = 128;
         for (int bn = 128; few_waves && bn <= 256; bn += step) {
@@ -877,13 +782,11 @@ static int gemm_tc_impl(const void* Ahi, const void* Alo, long a_ld, int a_mn, c
             const long cost = ((t + kNumSMs - 1) / kNumSMs) * (bn + 32);
             if (best_cost < 0 || cost < best_cost) { best_cost = cost; p.BN = bn; }
         }
-        if (!few_waves && auto_bn) {
+        if (!few_waves) {
             // many waves: the kernel is bound by the MMA's operand fetch from shared memory (a cta_group::1 MMA reads
             // 4 KB of A + 32 BN bytes of B per 64 BN / 128 cycles of math), so either A stays resident and BN = 128 keeps three
             // B stages (A-stationary schedule, short K), or the tile is as wide as it gets: BN = 256 moves 25 % fewer operand
             // bytes per flop (K = 200: 159 -> 144 us at M = 10240, N = 9684, with two 96 KB stages).
-            const char* ae0 = getenv("CAPHN_TC_ASTAT");
-            const bool astat_on = !(ae0 && atoi(ae0) == 0);
             const size_t slab0 = (size_t)p.num_kb * (split ? 2 : 1) * tc::TILE_BYTES;
             const size_t fixed0 = (size_t)tc::STG_FLOATS_V2 * 4 + (2 * tc::MAX_STAGES + 6) * 8 + 16 + 1024;
             const size_t bst0 = (size_t)(split ? 2 : 1) * 128 * tc::BK * 2;
@@ -916,7 +819,6 @@ static int gemm_tc_impl(const void* Ahi, const void* Alo, long a_ld, int a_mn, c
     p.splitk = (p.num_kb + p.kb_per - 1) / p.kb_per;
     p.b_bytes = p.BN * tc::BK * 2;
     p.stage_bytes = (split ? 2 : 1) * (tc::TILE_BYTES + p.b_bytes);
-    if (amax_val) { p.amax_val = amax_val; p.stat_mode = stat_mode; }
     bool tma_store = false;
     {   // TMA-store epilogue: full 32-column chunks leave through cp.async.bulk.tensor stores.  Bit-identical to the default
         // epilogue and 2-9 % faster on the logits products (profiles/r02_gemm_tma_store.txt); N % 4 == 0 only (a clipped
@@ -925,55 +827,32 @@ static int gemm_tc_impl(const void* Ahi, const void* Alo, long a_ld, int a_mn, c
         const char* e = getenv("CAPHN_TC_TMA_STORE");
         tma_store = !(e && e[0] == '0') && p.splitk == 1 && (ldc % 4 == 0) && (N % 4 == 0) && ((uintptr_t)C % 16 == 0);
     }
-    const char* ae = getenv("CAPHN_TC_ASTAT");
-    const int astat_mode = ae ? atoi(ae) : 1;
-    const char* se = getenv("CAPHN_TC_STG2");
-    const int stg2_mode = se ? atoi(se) : 0;
     const size_t slab = (size_t)p.num_kb * (split ? 2 : 1) * tc::TILE_BYTES;
     const size_t bstage = (size_t)(split ? 2 : 1) * p.b_bytes;
-    // A-stationary schedule (see TcParams::astat): K-major operands, no split-K, >= 4 tiles per CTA, >= 4 n-tiles, the A slab
-    // and enough B stages fit in shared memory.  CAPHN_TC_ASTAT=0 switches it off, =2 accepts 2 B stages instead of 3.
-    const bool astat_shape = astat_mode > 0 && !a_mn && !b_mn && p.splitk == 1 && ceil_div(N, p.BN) >= 4 &&
-                             tiles >= 4 * kNumSMs;
-    size_t fixed = 0;
-    int stages = 0;
-    // plan(bufs): shared-memory plan with `bufs` staging tiles per epilogue warp; false when fewer than 2 stages fit
-    auto plan = [&](int bufs) -> bool {     // bufs == 0: split-K, the epilogue adds from registers (no staging tile)
-        fixed = (size_t)bufs * tc::STG_FLOATS_V2 * 4 + (2 * tc::MAX_STAGES + 6) * 8 + 16 + 1024;
-        p.stg_bufs = bufs;
-        p.astat = 0; p.a_slab_bytes = 0;
-        p.stage_bytes = (split ? 2 : 1) * (tc::TILE_BYTES + p.b_bytes);
-        const int min_st = astat_mode >= 2 ? 2 : 3;
-        if (astat_shape && slab + fixed + (size_t)min_st * bstage <= tc::SMEM_BUDGET) {
-            p.astat = 1;
-            p.a_slab_bytes = (int)slab;
-            p.stage_bytes = (int)bstage;
-            stages = (int)((tc::SMEM_BUDGET - fixed - slab) / bstage);
-        } else {
-            if (fixed + 2 * (size_t)p.stage_bytes > tc::SMEM_BUDGET) return false;
-            stages = (int)((tc::SMEM_BUDGET - fixed) / p.stage_bytes);
-        }
-        if (stages > tc::MAX_STAGES) stages = tc::MAX_STAGES;
-        return stages >= 2;
-    };
-    // two staging tiles per epilogue warp (CAPHN_TC_STG2=1) only with the TMA-store epilogue and when the stages still fit
-    if (p.splitk > 1) {
-        if (!plan(0)) return CAPHN_EINVAL;
-    } else if (!(tma_store && stg2_mode > 0 && plan(2)) && !plan(1)) {
-        return CAPHN_EINVAL;
+    // A-stationary schedule: K-major operands, no split-K, >= 4 tiles per CTA, >= 4 n-tiles, the A slab and three B stages
+    // fit in shared memory.
+    const bool astat_shape = astat_on && !a_mn && !b_mn && p.splitk == 1 && ceil_div(N, p.BN) >= 4 && tiles >= 4 * kNumSMs;
+    // one staging tile per epilogue warp; none under split-K, where the epilogue adds from registers
+    const size_t fixed = (size_t)(p.splitk > 1 ? 0 : tc::STG_FLOATS_V2 * 4) + (2 * tc::MAX_STAGES + 6) * 8 + 16 + 1024;
+    int stages;
+    if (astat_shape && slab + fixed + 3 * bstage <= tc::SMEM_BUDGET) {
+        p.astat = 1;
+        p.a_slab_bytes = (int)slab;
+        p.stage_bytes = (int)bstage;
+        stages = (int)((tc::SMEM_BUDGET - fixed - slab) / bstage);
+    } else {
+        if (fixed + 2 * (size_t)p.stage_bytes > tc::SMEM_BUDGET) return CAPHN_EINVAL;
+        stages = (int)((tc::SMEM_BUDGET - fixed) / p.stage_bytes);
     }
+    if (stages > tc::MAX_STAGES) stages = tc::MAX_STAGES;
+    if (stages < 2) return CAPHN_EINVAL;
     p.stages = stages;
-    {   // L2 prefetch distance for the A operand of long-K products (CAPHN_TC_PREFETCH=<k-blocks>, 0 = off)
-        const char* pe = getenv("CAPHN_TC_PREFETCH");
-        const int pf = pe ? atoi(pe) : 0;
-        p.pf_dist = (!p.astat && p.kb_per >= 16 && pf > 0) ? pf : 0;
-    }
     p.tmem_cols = (2 * p.BN <= 256) ? 256u : 512u;
     const size_t smem = (size_t)p.a_slab_bytes + (size_t)stages * p.stage_bytes + fixed;
     if (bn_used) *bn_used = p.BN;
     if (amax_val) {
         if (amax_ld < 2 * ceil_div(N, p.BN)) return CAPHN_EINVAL;
-        p.amax_val = amax_val; p.amax_idx = amax_idx; p.amax_ld = amax_ld; p.stat_mode = stat_mode;
+        p.amax_val = amax_val; p.amax_idx = amax_idx; p.amax_ld = amax_ld;
     }
     if (p.splitk > 1) {
         if (ldc == N) {
@@ -1041,7 +920,7 @@ int caphn_gemm_tc_grouped(const void* Ahi, const void* Alo, long a_inner, long a
     tc::TcParams p{};
     p.C = C; p.ldc = ldc; p.bias = bias; p.units = (const tc::GUnit*)units; p.rowmap = rowmap; p.num_units = num_units;
     p.M = 0; p.N = 0; p.relu = 0; p.a_mn = a_mn ? 1 : 0; p.b_mn = b_mn ? 1 : 0; p.num_kb = 0; p.BN = BN;
-    p.splitk = 1; p.kb_per = 0; p.stg_bufs = 1;
+    p.splitk = 1; p.kb_per = 0;
     p.b_bytes = p.BN * tc::BK * 2;
     p.stage_bytes = (split ? 2 : 1) * (tc::TILE_BYTES + p.b_bytes);
     const size_t fixed = (size_t)tc::STG_FLOATS_V2 * 4 + (2 * tc::MAX_STAGES + 6) * 8 + 16 + 1024;
@@ -1084,17 +963,7 @@ int caphn_gemm_tc_scaled(const void* Ahi, const void* Alo, long a_ld, int a_mn, 
                          const float* scale_num, const float* scale_den, void* stream) {
     if (!scale_num) return CAPHN_EINVAL;
     return gemm_tc_impl(Ahi, Alo, a_ld, a_mn, Bhi, Blo, b_ld, b_mn, K, C, ldc, bias, M, N, 0, splitk, nullptr, nullptr, 0,
-                        stream, nullptr, 1, scale_num, scale_den);
-}
-
-// Diagnostics: caphn_gemm_tc_ex that also fills prof [148, 16] (int64 cycle counters per CTA, see TcParams::prof): where
-// the producer, the MMA thread and one epilogue warp spend their time waiting.  tools/bench_vocab.py prints them.
-int caphn_gemm_tc_prof(const void* Ahi, const void* Alo, long a_ld, int a_mn, const void* Bhi, const void* Blo, long b_ld,
-                       int b_mn, long K, float* C, long ldc, const float* bias, int M, int N, int splitk, long long* prof,
-                       void* stream) {
-    if (!prof) return CAPHN_EINVAL;
-    return gemm_tc_impl(Ahi, Alo, a_ld, a_mn, Bhi, Blo, b_ld, b_mn, K, C, ldc, bias, M, N, 0, splitk, nullptr, nullptr, 0,
-                        stream, nullptr, 1, nullptr, nullptr, prof);
+                        stream, nullptr, scale_num, scale_den);
 }
 
 // caphn_gemm_tc_ex + row arg-max partials in the epilogue (greedy decode: logits_t = h_t W^T + b, next word = arg-max):
@@ -1108,21 +977,6 @@ int caphn_gemm_tc_amax(const void* Ahi, const void* Alo, long a_ld, int a_mn, co
     int bn = 0;
     const int rc = gemm_tc_impl(Ahi, Alo, a_ld, a_mn, Bhi, Blo, b_ld, b_mn, K, C, ldc, bias, M, N, 0, 1, amax_val, amax_idx,
                                 amax_ld, stream, &bn);
-    if (nparts && bn > 0) *nparts = 2 * ceil_div(N, bn);
-    return rc;
-}
-
-// caphn_gemm_tc_ex + row log-sum-exp partials in the epilogue (training: logits = H W^T + b feed F.cross_entropy,
-// cc_train_hypernet.py:152-153 / hypernet.py:139-145): pm / ps [M, ld] receive, per row and per (n-tile, warp half), the
-// running max m and s = sum exp(x - m) of the columns that warp read (slots without columns: m = -inf, s = 0).
-// *nparts = slots written per row.  Finish with caphn_ce_fwd_partials.
-int caphn_gemm_tc_lse(const void* Ahi, const void* Alo, long a_ld, int a_mn, const void* Bhi, const void* Blo, long b_ld,
-                      int b_mn, long K, float* C, long ldc, const float* bias, int M, int N, float* pm, float* ps, int ld,
-                      int* nparts, void* stream) {
-    if (!pm || !ps) return CAPHN_EINVAL;
-    int bn = 0;
-    const int rc = gemm_tc_impl(Ahi, Alo, a_ld, a_mn, Bhi, Blo, b_ld, b_mn, K, C, ldc, bias, M, N, 0, 1, pm, (int*)ps, ld,
-                                stream, &bn, 2);
     if (nparts && bn > 0) *nparts = 2 * ceil_div(N, bn);
     return rc;
 }

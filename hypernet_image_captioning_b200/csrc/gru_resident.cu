@@ -513,9 +513,8 @@ static int gr_dispatch(bool bwd, GruResArgs& a, cudaStream_t st) {
     int KR = 0, ldw = 0;
     size_t smem = 0;
     if (bwd) {
-        static const bool colblk = [] { const char* e = getenv("CAPHN_GRU_BWD_COLBLK"); return !(e && e[0] == '0'); }();
         int C = 0, KS = 0;
-        if (colblk && gr_plan_bwdc(a.H, &C, &KS, &ldw, &smem)) {
+        if (gr_plan_bwdc(a.H, &C, &KS, &ldw, &smem)) {
             a.KS = KS; a.ldw = ldw;
             switch (C) {
                 case 1: return gr_launch_bwdc<1>(a, smem, st);

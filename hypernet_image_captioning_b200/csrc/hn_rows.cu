@@ -451,36 +451,13 @@ static int rows_linear_bwd_t(const T* W, const float* A, long lda, const float* 
             switch (gc) {
                 case 4: rc = launch_rows_bwd<T, 4, 1, 4>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
                 case 2: rc = launch_rows_bwd<T, 2, 2, 2>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
-                default: {
-                    // tuning knob (tools/bench_rows.py): vectors per lane x rows in flight of the single-group kernel
-                    const char* e = getenv("CAPHN_ROWS_BWD_VARIANT");
-                    switch (e ? atoi(e) : 0) {
-                        case 1: rc = launch_rows_bwd<T, 1, 4, 4>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
-                        case 2: rc = launch_rows_bwd<T, 1, 2, 4>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
-                        case 3: rc = launch_rows_bwd<T, 1, 8, 1>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
-                        case 4: rc = launch_rows_bwd<T, 1, 8, 2>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
-                        case 5: rc = launch_rows_bwd<T, 1, 2, 8>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
-                        default: rc = launch_rows_bwd<T, 1, 4, 2>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
-                    }
-                    break;
-                }
+                default: rc = launch_rows_bwd<T, 1, 4, 2>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
             }
         } else {
             switch (gc) {
                 case 4: rc = launch_rows_bwd<T, 4, 1, 2>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
                 case 2: rc = launch_rows_bwd<T, 2, 1, 4>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
-                default: {
-                    const char* e = getenv("CAPHN_ROWS_BWD_VARIANT");
-                    switch (e ? atoi(e) : 0) {
-                        case 1: rc = launch_rows_bwd<T, 1, 4, 2>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
-                        case 2: rc = launch_rows_bwd<T, 1, 4, 4>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
-                        case 3: rc = launch_rows_bwd<T, 1, 2, 8>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
-                        case 4: rc = launch_rows_bwd<T, 1, 1, 8>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
-                        case 5: rc = launch_rows_bwd<T, 1, 1, 4>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
-                        default: rc = launch_rows_bwd<T, 1, 2, 4>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
-                    }
-                    break;
-                }
+                default: rc = launch_rows_bwd<T, 1, 2, 4>(W, Ag, lda, dPg, N, dW, dAg, ldda, N, (int)K, acc, nda, st); break;
             }
         }
         if (rc) return rc;

@@ -256,18 +256,14 @@ def vocab_bwd_from_dlogits(dl, Hbm2, fc_w, need_w=True, need_b=True):
 # forward (ops.ce_fwd_split: 0.4 GB read + 0.4 GB written at [10240, 9684], instead of ce_fwd's read followed by
 # ce_bwd_split's read + write in the backward); the scalar grad_output / #valid rows is applied by the epilogues of the two
 # backward products, and the bias gradient is one more output column of the dW product (a row of ones appended to H).
-CE_FUSED_FWD = True
-
-
-def ce_fwd_for_loss(logits2d, targets, ignore_index, H, need_grad, stats=None):
+def ce_fwd_for_loss(logits2d, targets, ignore_index, H, need_grad):
     """Forward of the fused loss nodes.  Returns (lossbuf, lse, hi, lo): hi / lo = the unscaled gradient operand when the
     one-pass kernel applies (gradients wanted, both backward products on the tensor cores, row fits in shared memory), else
     None / None and the backward runs ce_bwd_split."""
     M, V = logits2d.shape
-    if (CE_FUSED_FWD and need_grad and stats is None and V <= ops.CE_FWD_SPLIT_MAX_V and ops._tc_ok(M, H, V)
-            and ops._tc_ok(V, H + 1, M)):
+    if need_grad and V <= ops.CE_FWD_SPLIT_MAX_V and ops._tc_ok(M, H, V) and ops._tc_ok(V, H + 1, M):
         return ops.ce_fwd_split(logits2d, targets, ignore_index)
-    lossbuf, lse = ops.ce_fwd_stats(logits2d, targets, ignore_index, stats)
+    lossbuf, lse = ops.ce_fwd(logits2d, targets, ignore_index)
     return lossbuf, lse, None, None
 
 
@@ -279,8 +275,8 @@ class VocabPrep:
     second branch next to the logits product instead of in front of the dW product."""
 
     def __init__(self, M, V, H, need_grad, like):
-        self.on = bool(CE_FUSED_FWD and need_grad and V <= ops.CE_FWD_SPLIT_MAX_V and ops._tc_ok(M, H, V)
-                       and ops._tc_ok(V, H + 1, M) and ops._tc_ok(M, V, H))
+        self.on = bool(need_grad and V <= ops.CE_FWD_SPLIT_MAX_V and ops._tc_ok(M, H, V) and ops._tc_ok(V, H + 1, M)
+                       and ops._tc_ok(M, V, H))
         self.w = self.wt = self.ht = None
         self.br = streams.Branches("vprep", like=like) if self.on else None
 
@@ -345,7 +341,7 @@ def vocab_bwd_fused(logits2d, targets, ignore_index, lse, lossbuf, gscale, Hbm2,
 # ----------------------------------------------------------------------------------------------------------------------
 # Variant A decoder: teacher-forced DecoderGRU.forward  (reference later.py:389-457)
 # ----------------------------------------------------------------------------------------------------------------------
-def _gru_decoder_forward(feats, captions, h0, emb_w, fc_w, fc_b, cells, want_stats=False, prep=None):
+def _gru_decoder_forward(feats, captions, h0, emb_w, fc_w, fc_b, cells, prep=None):
     B, T = captions.shape
     NL = len(cells) // 4
     W_ih, W_hh, b_ih, b_hh = cells[0:4]
@@ -384,11 +380,8 @@ def _gru_decoder_forward(feats, captions, h0, emb_w, fc_w, fc_b, cells, want_sta
         streams.wait_pending()      # (whatever else the forked hypernet computation queued; done long before this point)
     if prep is not None and prep.on:
         logits = prep.logits(Hbm.view(B * T, H), fc_b)
-        return logits.view(B, T, -1), (caps, X, Hall, Hbm, saved, Hmid, emb_w, fc_w), None
-    if want_stats:      # fused loss node: the cross-entropy statistics come out of this GEMM's epilogue
-        logits, stats = ops.linear_lse(Hbm.view(B * T, H), fc_w.contiguous(), fc_b)
-        return logits.view(B, T, -1), (caps, X, Hall, Hbm, saved, Hmid, emb_w, fc_w), stats
-    logits = ops.linear(Hbm.view(B * T, H), fc_w.contiguous(), fc_b)
+    else:
+        logits = ops.linear(Hbm.view(B * T, H), fc_w.contiguous(), fc_b)
     return logits.view(B, T, -1), (caps, X, Hall, Hbm, saved, Hmid, emb_w, fc_w)
 
 
@@ -584,13 +577,11 @@ class DecoderGRULossFn(Function):
     def forward(ctx, ignore_index, feats, captions, h0, emb_w, fc_w, fc_b, *cells):
         Bc, Tc = captions.shape
         prep = VocabPrep(Bc * Tc, fc_w.shape[0], cells[1].shape[1], any(ctx.needs_input_grad), feats)
-        if ops.CE_FUSED_STATS:             # (the epilogue-statistics experiment takes the logits product itself)
-            prep.on = False
-        logits, sv, stats = _gru_decoder_forward(feats, captions, h0, emb_w, fc_w, fc_b, cells, want_stats=True, prep=prep)
+        logits, sv = _gru_decoder_forward(feats, captions, h0, emb_w, fc_w, fc_b, cells, prep=prep)
         B, T, V = logits.shape
         targets = captions.reshape(-1).contiguous()
         lossbuf, lse, dhi, dlo = ce_fwd_for_loss(logits.view(B * T, V), targets, ignore_index, sv[3].shape[-1],
-                                                 any(ctx.needs_input_grad), stats)
+                                                 any(ctx.needs_input_grad))
         prep.finish()
         ctx.save_for_backward(*sv, *cells, logits, targets, lse, lossbuf, dhi, dlo, *prep.saved())
         ctx.NL = len(cells) // 4

@@ -13,8 +13,6 @@ generated weights become leaves and their gradient lands on ``captioner.<cell>.w
 """
 from typing import List
 
-import os
-
 import torch
 from torch import nn
 
@@ -207,12 +205,6 @@ class PooledFeatureEncoder(nn.Module):
         return Fn.linear(pooled, self.fc.weight, self.fc.bias)
 
 
-# Greedy decode returns softmax probabilities (later.py:472): normalise every step's logits in place on a side stream
-# (False: measured 1.898 ms per B=512, T=20 decode), or all of them in one pass after the last step (True: 1.927 ms -- the
-# 0.8 GB pass is then serial).  CAPHN_DECODE_SOFTMAX=step|end.
-DECODE_SOFTMAX_AT_END = os.environ.get("CAPHN_DECODE_SOFTMAX", "step") == "end"
-
-
 class DecoderGRU(nn.Module):
     """Drop-in for later.py:362 DecoderGRU (constructor signature, forward/infer signatures, state_dict keys).
 
@@ -324,7 +316,7 @@ class DecoderGRU(nn.Module):
         # vocabulary GEMM's epilogue as per-tile partials and is finished inside the gather of the next input row, so the
         # softmax that produces the RETURNED probabilities (later.py:472) is off the dependency chain: the logits are written
         # straight into outputs[:, t] and normalised in place on a side stream while the next step runs.
-        fast = table is not None and ops.DECODE_FUSED_ARGMAX and ops._tc_ok(B, self.vocab_size, H)
+        fast = table is not None and ops._tc_ok(B, self.vocab_size, H)
         if not fast:
             for t in range(max_len):
                 if t == 0:
@@ -374,17 +366,9 @@ class DecoderGRU(nn.Module):
                         GI = GIb
                     h = ops.gru_seq_fwd(GI, WhhT, b_hh, h, 1, save=False, want_bm=False)[0][1]
                     nparts = ops.gemm_tc_amax(ops.split_bf16(h), vocab.operand(), fc_b, lg, pv, pi)
-            if not DECODE_SOFTMAX_AT_END:
-                if chain is not None:
-                    cur.wait_stream(chain)                           # (up to this step's GEMM)
-                ops.softmax_argmax(lg, want_probs=True, probs_out=lg, want_argmax=False)     # in place, off the chain
-        if DECODE_SOFTMAX_AT_END:
-            # one pass over all B*T rows once the chain is done: 0.8 GB at HBM speed, and no 512-CTA softmax launch competing
-            # with the latency-bound chain at every step
             if chain is not None:
-                cur.wait_stream(chain)
-            flat = outputs.view(B * max_len, self.vocab_size)
-            ops.softmax_argmax(flat, want_probs=True, probs_out=flat, want_argmax=False)
+                cur.wait_stream(chain)                               # (up to this step's GEMM)
+            ops.softmax_argmax(lg, want_probs=True, probs_out=lg, want_argmax=False)         # in place, off the chain
         return outputs
 
     @torch.no_grad()

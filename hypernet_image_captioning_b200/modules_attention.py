@@ -80,7 +80,7 @@ class FeatureFn(Function):
 
 
 def _attgru_forward(need_grad, f3, K3, h0, captions, use_sampling, emb_w, W_ih, W_hh, b_ih, b_hh, fc_w, fc_b, Ua_w, Ua_b,
-                    va_w, va_b, stats_out=None):
+                    va_w, va_b):
     """The time loop of AttentionGru.forward (models/decoderlstm.py:78-108) + the vocabulary projection, given the
     loop-invariant tensors of FeatureFn.  Returns (logits, attn, tensors to save, dims)."""
     B, P, Fd = f3.shape
@@ -115,17 +115,8 @@ def _attgru_forward(need_grad, f3, K3, h0, captions, use_sampling, emb_w, W_ih, 
         Xw = ops.build_inputs(None, emb_w, caps, 1)                    # [T*B, E]
         XC[:, :E].copy_(Xw)
         GIw = ops.linear(Xw, W_ih_w, b_ih.contiguous())                # [T*B, 3H]
-        if ops.attgru_cluster_ok(H, Fd, P):
-            # weights-resident path: U_a / W_hh / W_ih[:,E:] stay on chip for all T steps (cluster of 8 CTAs)
-            ops.attgru_cluster_fwd(K3, f3, GIw, Ua_w.contiguous(), Ua_b, va, bv, W_ih, W_hh, b_hh, Hall, Hbm, attn, XC,
-                                   E, saved, 0, T)
-        else:
-            ops.attgru_fwd(K3, f3, GIw, lw, Ua_b, va, bv, b_hh, Hall, Hbm, attn, XC, E, saved, 0, T)
-        if stats_out is not None:       # fused loss node: cross-entropy statistics out of the logits GEMM's epilogue
-            _, st = ops.linear_lse(Hbm.view(B * T, H), fc_w, fc_b, out=logits.view(B * T, V))
-            stats_out.append(st)
-        else:
-            ops.linear(Hbm.view(B * T, H), fc_w, fc_b, out=logits.view(B * T, V))
+        ops.attgru_fwd(K3, f3, GIw, lw, Ua_b, va, bv, b_hh, Hall, Hbm, attn, XC, E, saved, 0, T)
+        ops.linear(Hbm.view(B * T, H), fc_w, fc_b, out=logits.view(B * T, V))
     else:
         GIw = torch.empty(T * B, 3 * H, device=dev, dtype=torch.float32)
         xproj, vocab = ops.LinearPlan(W_ih_w, b_ih.contiguous()), ops.LinearPlan(fc_w, fc_b)   # split once, reuse per step
@@ -141,7 +132,7 @@ def _attgru_forward(need_grad, f3, K3, h0, captions, use_sampling, emb_w, W_ih, 
         # per step instead of 7 -- the arg-max of the logits comes out of the vocabulary GEMM's epilogue as per-tile partials
         # and is finished inside the gather of the next step's input row; h_t goes to the GEMM as the bf16 hi/lo rows the
         # gates kernel has already written for the next step (no separate operand split).
-        fast = table is not None and lw.pack is not None and ops._tc_ok(B, V, H) and ops.DECODE_FUSED_ARGMAX
+        fast = table is not None and lw.pack is not None and ops._tc_ok(B, V, H)
         if fast:
             pv = torch.empty(B, 2 * ((V + 127) // 128), device=dev, dtype=torch.float32)
             pi = torch.empty(B, 2 * ((V + 127) // 128), device=dev, dtype=torch.int32)
@@ -244,12 +235,11 @@ class AttentionGruLossFn(Function):
 
     @staticmethod
     def forward(ctx, ignore_index, f3, K3, h0, captions, use_sampling, *params):
-        stats = []
-        logits, attn, sv, dims = _attgru_forward(True, f3, K3, h0, captions, use_sampling, *params, stats_out=stats)
+        logits, attn, sv, dims = _attgru_forward(True, f3, K3, h0, captions, use_sampling, *params)
         B, T, V = logits.shape
         targets = captions.reshape(-1).contiguous()
         lossbuf, lse, dhi, dlo = Fn.ce_fwd_for_loss(logits.view(B * T, V), targets, ignore_index, dims[4],
-                                                    any(ctx.needs_input_grad), stats[0] if stats else None)
+                                                    any(ctx.needs_input_grad))
         ctx.save_for_backward(*sv, logits, targets, lse, lossbuf, dhi, dlo)
         ctx.dims = dims
         ctx.ignore_index = ignore_index

@@ -261,14 +261,11 @@ def lstm_seq_bwd(dHbm, saved, Hall, Whh_p, extra=()):
     return dG, dh0
 
 
-CLUSTER_RECURRENCE = True   # use the weights-resident cluster kernels when W_hh fits (single layer)
 _cluster_plan_cache = {}
 
 
 def gru_cluster_size(H):
     """Cluster size of the weights-resident GRU kernels for hidden size H (0 = not applicable)."""
-    if not CLUSTER_RECURRENCE:
-        return 0
     if H not in _cluster_plan_cache:
         import ctypes
         cs = ctypes.c_int(0)
@@ -277,14 +274,11 @@ def gru_cluster_size(H):
     return _cluster_plan_cache[H]
 
 
-RESIDENT_RECURRENCE = True   # CTA-resident W_hh (smem + registers, no cluster) where it fits; else the cluster kernels
 _resident_plan_cache = {}
 
 
 def gru_resident_ok(H):
     """True when the CTA-resident GRU kernels (csrc/gru_resident.cu) apply to hidden size H."""
-    if not RESIDENT_RECURRENCE:
-        return False
     if H not in _resident_plan_cache:
         import ctypes
         ok = ctypes.c_int(0)
@@ -510,7 +504,6 @@ def relu_mask_(ref, y):
     return y
 
 
-DECODE_FUSED_ARGMAX = True   # greedy decode: arg-max partials in the vocabulary GEMM's epilogue, finished inside the next gather
 ATT_STEP = True   # two batch-wide kernels per step (attention | tensor-core gates) instead of the persistent streaming kernel
 
 
@@ -585,37 +578,6 @@ def attgru_seq_fwd(Kp, f, GIw, lw, bu, va, bv, bhh, Hall, Hbm, attn, XC, E, save
                va.data_ptr(), bv.data_ptr(), lw.WihcT.data_ptr(), lw.WhhT.data_ptr(), bhh.data_ptr(), Hall.data_ptr(),
                _p(Hbm), attn.data_ptr(), ctx_ptr, XC.stride(0), sp[0], sp[1], sp[2], sp[3], sp[4],
                B, T, P, H, Fd, lw.ldh, lw.ld3, t0, t1, _stream())
-
-
-_attcl_cache = {}
-
-
-ATT_CLUSTER = False   # experimental weights-resident attention forward (correct, not yet faster than streaming)
-
-
-def attgru_cluster_ok(H, Fd, P, force=False):
-    if not (ATT_CLUSTER or force):
-        return False
-    key = (H, Fd, P)
-    if key not in _attcl_cache:
-        import ctypes
-        ok = ctypes.c_int(0)
-        _cabi.call("caphn_attgru_cluster_plan", H, Fd, P, ctypes.byref(ok))
-        _attcl_cache[key] = bool(ok.value)
-    return _attcl_cache[key]
-
-
-def attgru_cluster_fwd(Kp, f, GIw, U_a, bu, va, bv, W_ih, W_hh, bhh, Hall, Hbm, attn, XC, E, saved, t0, t1):
-    """Weights-resident attention recurrence (cluster of 8, register-resident MMA fragments); plain row-major weights."""
-    B, P, H = Kp.shape
-    Fd = f.shape[2]
-    T = Hall.shape[0] - 1
-    sp = [saved[i].data_ptr() for i in range(5)] if saved is not None else [None] * 5
-    ctx_ptr = XC.data_ptr() + 4 * E
-    _cabi.call("caphn_attgru_cluster_fwd", Kp.data_ptr(), f.data_ptr(), GIw.data_ptr(), U_a.data_ptr(), bu.data_ptr(),
-               va.data_ptr(), bv.data_ptr(), W_ih.data_ptr(), W_hh.data_ptr(), bhh.data_ptr(), Hall.data_ptr(),
-               _p(Hbm), attn.data_ptr(), ctx_ptr, XC.stride(0), sp[0], sp[1], sp[2], sp[3], sp[4],
-               B, T, P, H, Fd, E, t0, t1, _stream())
 
 
 def attgru_seq_bwd(dHbm, dattn, Kp, f, attn, saved, Hall, U_a, va, W_ih, W_hh, E):
@@ -776,51 +738,6 @@ def gemm_tc_amax(A: SplitOperand, Bm: SplitOperand, bias, out, pval, pidx):
                int(Bm.mn), A.K, out.data_ptr(), out.stride(0), _p(bias), M, N, pval.data_ptr(), pidx.data_ptr(),
                pval.stride(0), ctypes.byref(n), _stream())
     return int(n.value)
-
-
-# Training: log-sum-exp partials out of the logits GEMM's epilogue (caphn_gemm_tc_lse) instead of the ce_fwd pass over the
-# logits.  Correct (tests/test_gpu_ops.py) but OFF: that GEMM is epilogue-bound, and the 32 shuffles + max + exp per 32
-# columns cost more than the 73 us pass they remove -- measured 4.38 -> 4.50 ms (pooled step) and 2.84 -> 2.97 ms
-# (attention step) with it on (profiles/r02_ce_epilogue_fusion_negative.txt).
-CE_FUSED_STATS = False
-
-
-def linear_lse(X, W, bias, out=None):
-    """out = X W^T + bias on the tensor cores + row log-sum-exp partials from the epilogue.  Returns (out, stats) with
-    stats = (pm, ps, nparts), or (out, None) when the product does not take the tensor-core path."""
-    _chk(X), _chk(W)
-    M, K = X.shape
-    N = W.shape[0]
-    if not (CE_FUSED_STATS and _tc_ok(M, N, K)):
-        return linear(X, W, bias, out=out), None
-    import ctypes
-    A, Bm = split_bf16(X), split_bf16(W)
-    if out is None:
-        out = torch.empty(M, N, device=X.device, dtype=torch.float32)
-    ld = 2 * ((N + 127) // 128)
-    pm = torch.empty(M, ld, device=X.device, dtype=torch.float32)
-    ps = torch.empty(M, ld, device=X.device, dtype=torch.float32)
-    n = ctypes.c_int(0)
-    _cabi.call("caphn_gemm_tc_lse", A.hi.data_ptr(), _p(A.lo), A.ld, 0, Bm.hi.data_ptr(), _p(Bm.lo), Bm.ld, 0, A.K,
-               out.data_ptr(), out.stride(0), _p(bias), M, N, pm.data_ptr(), ps.data_ptr(), ld, ctypes.byref(n), _stream())
-    return out, (pm, ps, int(n.value))
-
-
-def ce_fwd_stats(logits2d, targets, ignore_index, stats):
-    """ce_fwd from the epilogue's partials (``stats`` of linear_lse); falls back to the pass over the logits without them."""
-    if stats is None:
-        return ce_fwd(logits2d, targets, ignore_index)
-    pm, ps, nparts = stats
-    M, V = logits2d.shape
-    dev = logits2d.device
-    lse = torch.empty(M, device=dev, dtype=torch.float32)
-    scratch = torch.empty(2 * M, device=dev, dtype=torch.float32)
-    lossbuf = torch.empty(2, device=dev, dtype=torch.float32)
-    has = ignore_index is not None
-    _cabi.call("caphn_ce_fwd_partials", pm.data_ptr(), ps.data_ptr(), pm.stride(0), nparts, logits2d.data_ptr(),
-               logits2d.stride(0), targets.data_ptr(), M, int(has), int(ignore_index) if has else 0, lse.data_ptr(),
-               scratch.data_ptr(), lossbuf.data_ptr(), _stream())
-    return lossbuf, lse
 
 
 def argmax_finish_gather(pval, pidx, nparts, table=None, tok=None, out=None):

@@ -162,16 +162,6 @@ int caphn_attstep_bwd(const float* dHbm, const float* dattn, const float* Kp, co
                       const float* Hall, const float* va, const void* pack, void* work, float* dGI, float* dGH,
                       float* dU, float* dCTX, float* dK, float* dva, float* dbv, float* dh0, int B, int T, int P, int H,
                       int F, void* stream);
-/* Weights-resident forward variant: U_a, W_hh and W_ih[:,E:] stay on chip for all steps, split by hidden unit over a
- * cluster of 8 CTAs (register-resident warp-MMA fragments, bf16x3), attention partitioned by batch row, DSMEM exchanges.
- * Takes the PLAIN row-major weights Ua [H,H], Wih [3H,E+F], Whh [3H,H].  caphn_attgru_cluster_plan: *ok = 1 if the
- * sizes are supported (H, F <= 208, ...); otherwise use caphn_attgru_seq_fwd. */
-int caphn_attgru_cluster_plan(int H, int F, int P, int* ok);
-int caphn_attgru_cluster_fwd(const float* Kp, const float* f, const float* GIw, const float* Ua, const float* bu,
-                             const float* va, const float* bv, const float* Wih, const float* Whh, const float* bhh,
-                             float* Hall, float* Hbm, float* attn, float* ctx, long ldctx, float* Upre, float* R, float* Z,
-                             float* Nn, float* GHN, int B, int T, int P, int H, int F, int E, int t0, int t1,
-                             void* stream);
 /* df[b,p,:] += sum_t attn[b,t,p] * dCTX[t,b,:]  (context-vector backward, deferred out of the BPTT loop). */
 int caphn_attn_df(const float* attn, const float* dCTX, float* df, int B, int T, int P, int F, void* stream);
 
@@ -346,17 +336,6 @@ int caphn_gru_cluster_bwd_grouped(const float* dHbm, const float* saved, const f
                                   float* dGH, float* dh0, int B, int T, int H, const int* tiles, int ntiles, long wstride,
                                   void* stream);
 
-/* Cross-entropy statistics out of the logits GEMM (SURVEY K7+K8): caphn_gemm_tc_lse = caphn_gemm_tc_ex whose epilogue also
- * keeps, per row and per (n-tile, epilogue-warp half), the running max m and s = sum exp(x - m) of the columns it wrote
- * (pm / ps [M, ld], *nparts slots per row); caphn_ce_fwd_partials merges them into lse, reads the one target logit per row
- * and produces the same (lse, lossbuf) as caphn_ce_fwd -- without re-reading the [M, V] logits (0.4 GB at B=512, T=20). */
-int caphn_gemm_tc_lse(const void* Ahi, const void* Alo, long a_ld, int a_mn, const void* Bhi, const void* Blo, long b_ld,
-                      int b_mn, long K, float* C, long ldc, const float* bias, int M, int N, float* pm, float* ps, int ld,
-                      int* nparts, void* stream);
-int caphn_ce_fwd_partials(const float* pm, const float* ps, int ldp, int nparts, const float* X, long ld,
-                          const long long* tgt, long M, int has_ignore, long long ignore, float* lse, float* scratch,
-                          float* lossbuf, void* stream);
-
 /* Cross-entropy forward and gradient operand in ONE pass over the logits (the fused loss nodes; F.cross_entropy +
  * its backward at cc_train_hypernet.py:152-153 / hypernet.py:139-145): caphn_ce_fwd's outputs plus the bf16 hi/lo split of
  * the UNSCALED gradient u = softmax(X) - onehot(tgt) (0 on ignored rows) as a tensor-core operand [M, Vp] (Vp % 64 == 0;
@@ -369,12 +348,6 @@ int caphn_ce_fwd_split(const float* X, long ld, const long long* tgt, long M, in
 int caphn_gemm_tc_scaled(const void* Ahi, const void* Alo, long a_ld, int a_mn, const void* Bhi, const void* Blo, long b_ld,
                          int b_mn, long K, float* C, long ldc, const float* bias, int M, int N, int splitk,
                          const float* scale_num, const float* scale_den, void* stream);
-
-/* Diagnostics: caphn_gemm_tc_ex (no ReLU) that also writes 16 int64 cycle counters per CTA into prof [148, 16] -- the time
- * the TMA producer, the MMA thread and one epilogue warp spend waiting on each of their barriers (gemm_tc.cu TcParams::prof). */
-int caphn_gemm_tc_prof(const void* Ahi, const void* Alo, long a_ld, int a_mn, const void* Bhi, const void* Blo, long b_ld,
-                       int b_mn, long K, float* C, long ldc, const float* bias, int M, int N, int splitk, long long* prof,
-                       void* stream);
 
 /* One greedy-decode step of the pooled captioner (later.py:459-490: argmax feedback -> embedding -> nn.GRUCell) as one
  * launch: finishes the arg-max of the previous vocabulary projection from the partials of caphn_gemm_tc_amax (GI == NULL; the

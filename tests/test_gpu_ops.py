@@ -218,33 +218,6 @@ def test_gru_cluster_matches_streaming_kernel(B, T, H):
     assert rel_err(dGI1, dGI0) < 1e-5 and rel_err(dGH1, dGH0) < 1e-5 and rel_err(dh01, dh00) < 1e-5
 
 
-def test_ce_statistics_from_the_gemm_epilogue_match_the_separate_pass():
-    """caphn_gemm_tc_lse + caphn_ce_fwd_partials (log-sum-exp partials out of the logits GEMM's epilogue; off by default,
-    ops.CE_FUSED_STATS) == gemm_tc + ce_fwd: identical logits, lse / loss within fp32 rounding; ignore_index honoured."""
-    import torch
-    from hypernet_image_captioning_b200 import ops
-    g = torch.Generator().manual_seed(0)
-    M, K, V = 1300, 150, 9684
-    X = (torch.randn(M, K, generator=g) * 0.5).cuda()
-    W = (torch.randn(V, K, generator=g) * 0.2).cuda()
-    b = torch.randn(V, generator=g).cuda()
-    tgt = torch.randint(0, V, (M,), generator=g).cuda()
-    tgt[::7] = 0
-    ref_logits = ops.linear(X, W, b)
-    old = ops.CE_FUSED_STATS
-    ops.CE_FUSED_STATS = True
-    try:
-        logits, stats = ops.linear_lse(X, W, b)
-    finally:
-        ops.CE_FUSED_STATS = old
-    assert stats is not None and torch.equal(logits, ref_logits)
-    for ign in (None, 0):
-        lb_ref, lse_ref = ops.ce_fwd(ref_logits, tgt, ign)
-        lb, lse = ops.ce_fwd_stats(logits, tgt, ign, stats)
-        assert (lse - lse_ref).abs().max().item() < 2e-6 * lse_ref.abs().max().item()
-        assert abs(lb[0].item() - lb_ref[0].item()) < 1e-6 * abs(lb_ref[0].item()) and lb[1].item() == lb_ref[1].item()
-
-
 @pytest.mark.parametrize("M,V,ignore", [(1300, 9684, 0), (1300, 9684, None), (257, 1502, 0), (130, 9685, 0)])
 def test_ce_forward_with_gradient_operand_in_one_pass(M, V, ignore):
     """caphn_ce_fwd_split (loss + UNSCALED gradient operand from one read of the logits) followed by the scaled products
@@ -298,7 +271,7 @@ def test_ce_forward_with_gradient_operand_in_one_pass(M, V, ignore):
 def test_gemm_tc_a_stationary_schedule_is_bit_identical(M, N, K, monkeypatch):
     """The A-stationary schedule of the tensor-core GEMM (A slab resident per m-tile, contiguous tile runs per CTA; the
     vocabulary projection) only reorders tiles: bit-identical to the round-robin schedule, bias / ragged N / ragged K
-    included (CAPHN_TC_ASTAT=0 switches it off, =2 also accepts two B stages, e.g. K = 200)."""
+    included (CAPHN_TC_ASTAT=0 switches it off)."""
     import torch
     from hypernet_image_captioning_b200 import ops
     g = torch.Generator().manual_seed(2)
@@ -306,12 +279,12 @@ def test_gemm_tc_a_stationary_schedule_is_bit_identical(M, N, K, monkeypatch):
     W = (torch.randn(N, K, generator=g) * 0.3).cuda()
     b = torch.randn(N, generator=g).cuda()
     outs = {}
-    for mode in ("0", "1", "2"):
+    for mode in ("0", "1"):
         monkeypatch.setenv("CAPHN_TC_ASTAT", mode)
         outs[mode] = ops.linear(X, W, b).clone()
     ref = X.double() @ W.double().t() + b.double()
     assert (outs["0"].double() - ref).abs().max().item() < 2e-5 * ref.abs().max().item()
-    assert torch.equal(outs["0"], outs["1"]) and torch.equal(outs["0"], outs["2"])
+    assert torch.equal(outs["0"], outs["1"])
 
 
 @pytest.mark.parametrize("B,H,V", [(512, 150, 9684), (37, 34, 301), (16, 200, 1000), (5, 6, 40), (300, 256, 500),

@@ -1,4 +1,4 @@
-"""Micro-benchmark: attention recurrence forward -- persistent L2-streaming kernel, resident cluster kernel, step-split path."""
+"""Micro-benchmark: attention recurrence forward and backward -- persistent L2-streaming kernel vs step-split path."""
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from hypernet_image_captioning_b200 import ops
@@ -16,24 +16,22 @@ XC, saved = torch.zeros(T * B, E + Fo, device=dev), torch.empty(5, T, B, H, devi
 lw = ops.AttGruWeights(W_ih, W_hh, Ua, E, P, step=False)
 lws = ops.AttGruWeights(W_ih, W_hh, Ua, E, P, step=True)
 
-def run(cluster):
-    if cluster == 2:
+def run(step):
+    if step:
         ops.attgru_fwd(Kp, f, GIw, lws, bu, va, bv, bhh, Hall, Hbm, attn, XC, E, saved, 0, T)
-    elif cluster:
-        ops.attgru_cluster_fwd(Kp, f, GIw, Ua, bu, va, bv, W_ih, W_hh, bhh, Hall, Hbm, attn, XC, E, saved, 0, T)
     else:
         ops.attgru_seq_fwd(Kp, f, GIw, lw, bu, va, bv, bhh, Hall, Hbm, attn, XC, E, saved, 0, T)
 
-for cl in (0, 1, 2):
+for step in (False, True):
     for _ in range(2):
-        run(cl)
+        run(step)
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(5):
-        run(cl)
+        run(step)
     e1.record(); torch.cuda.synchronize()
-    print(("streaming         ", "cluster (resident)", "step-split        ")[cl], f"{e0.elapsed_time(e1) / 5 * 1e3:9.1f} us  ({e0.elapsed_time(e1) / 5 / T * 1e3:.1f} us/step)")
+    print("step-split        " if step else "streaming         ", f"{e0.elapsed_time(e1) / 5 * 1e3:9.1f} us  ({e0.elapsed_time(e1) / 5 / T * 1e3:.1f} us/step)")
 
 # ---- backward: persistent streaming kernel vs step-split ----
 ops.attgru_fwd(Kp, f, GIw, lws, bu, va, bv, bhh, Hall, Hbm, attn, XC, E, saved, 0, T)

@@ -71,10 +71,3 @@ print(f"{sys.argv[1] if len(sys.argv) > 1 else ''} attention greedy decode: {ms:
 ma.async_hypernet = True          # hypernet weight streaming next to the feature branch (streams.py)
 ms = timed(dec_att)
 print(f"{sys.argv[1] if len(sys.argv) > 1 else ''} attention greedy decode, async hypernet: {ms:.3f} ms ({B / ms * 1e3:.0f} captions/s)")
-ma.async_hypernet = False
-from hypernet_image_captioning_b200 import ops as _ops  # noqa: E402
-_ops.DECODE_FUSED_ARGMAX = False
-from hypernet_image_captioning_b200 import graphs as _graphs  # noqa: E402
-_graphs.clear()
-ms = timed(dec_att)
-print(f"{sys.argv[1] if len(sys.argv) > 1 else ''} attention greedy decode, separate argmax/split launches (round-1 loop): {ms:.3f} ms")

@@ -18,11 +18,7 @@ for (N, K) in ((90000, 11250), (67500, 8437), (240000, 480)):
         A = torch.randn(1, K, device="cuda"); dY = torch.randn(1, N, device="cuda")
         bytes_w = N * K * W.element_size()
         f = t(lambda: ops.rows_linear_fwd(W, None, A, 0))
-        line = f"N={N} K={K} {str(dt):16s} fwd {f*1e3:8.1f} us {bytes_w/f/1e6:7.0f} GB/s | bwd (GB/s) by variant:"
-        for var in range(6):
-            os.environ["CAPHN_ROWS_BWD_VARIANT"] = str(var)
-            b = t(lambda: ops.rows_linear_bwd(W, A, None, dY, 0))
-            line += f"  v{var} {2*bytes_w/b/1e6:6.0f}"
-        os.environ.pop("CAPHN_ROWS_BWD_VARIANT", None)
-        print(line, flush=True)
+        b = t(lambda: ops.rows_linear_bwd(W, A, None, dY, 0))
+        print(f"N={N} K={K} {str(dt):16s} fwd {f*1e3:8.1f} us {bytes_w/f/1e6:7.0f} GB/s | bwd {b*1e3:8.1f} us "
+              f"{2*bytes_w/b/1e6:7.0f} GB/s", flush=True)
         del W

@@ -46,20 +46,16 @@ for H in (150, 200):
     xs, ws = ops.split_bf16(X), ops.split_bf16(W)
     out = torch.empty(M, V, device="cuda")
     res = {}
-    for stg2 in ("0", "1"):
-        for mode in ("0", "1", "2"):
-            os.environ["CAPHN_TC_ASTAT"] = mode
-            os.environ["CAPHN_TC_STG2"] = stg2
-            us = timed(lambda: ops.gemm_tc(xs, ws, bias=b, out=out))
-            res[mode + stg2] = out.clone()
-            print(f"H={H} logits GEMM astat={mode} stg2={stg2}: {us:7.1f} us ({4.0 * M * V / us / 1e3:5.0f} GB/s of output)",
-                  flush=True)
+    for mode in ("0", "1"):
+        os.environ["CAPHN_TC_ASTAT"] = mode
+        us = timed(lambda: ops.gemm_tc(xs, ws, bias=b, out=out))
+        res[mode] = out.clone()
+        print(f"H={H} logits GEMM astat={mode}: {us:7.1f} us ({4.0 * M * V / us / 1e3:5.0f} GB/s of output)", flush=True)
     os.environ.pop("CAPHN_TC_ASTAT", None)
-    os.environ.pop("CAPHN_TC_STG2", None)
-    print(f"    bit-identical: {all(torch.equal(res['00'], v) for v in res.values())}")
+    print(f"    bit-identical: {torch.equal(res['0'], res['1'])}")
     t_set = timed(lambda: out.zero_())
     print(f"    (memset of the same [M, V] fp32 buffer: {t_set:6.1f} us = {4.0 * M * V / t_set / 1e3:5.0f} GB/s)")
-    logits = res["00"]
+    logits = res["0"]
     gs = torch.ones(1, device="cuda")
     t_fwd = timed(lambda: ops.ce_fwd(logits, tgt, 0))
     lb, lse = ops.ce_fwd(logits, tgt, 0)
@@ -77,49 +73,6 @@ for H in (150, 200):
     wt = ops.split_bf16_t(W)
     ht = ops.split_bf16_t(X, ones_row=True)
     wbuf = torch.empty(V, ops.round4(H + 1), device="cuda")[:, :H + 1]
-    for pf in ("0", "2", "4", "8"):
-        os.environ["CAPHN_TC_PREFETCH"] = pf
-        print(f"H={H} L2 prefetch distance {pf}: dH {timed(lambda: ops.gemm_tc(d, wt, scale=(gs, lb1[1:]))):6.1f} us, "
-              f"[dW | db] {timed(lambda: ops.gemm_tc(dT, ht, scale=(gs, lb1[1:]), out=wbuf)):6.1f} us", flush=True)
-    os.environ.pop("CAPHN_TC_PREFETCH", None)
     print(f"H={H} dH product alone {timed(lambda: ops.gemm_tc(d, wt, scale=(gs, lb1[1:]))):6.1f} us, "
           f"[dW | db] product alone {timed(lambda: ops.gemm_tc(dT, ht, scale=(gs, lb1[1:]), out=wbuf)):6.1f} us", flush=True)
 
-
-def prof(A, Bm, name, bias=None):
-    """Where the GEMM's roles wait (cycle counters of caphn_gemm_tc_prof, averaged over the CTAs)."""
-    from hypernet_image_captioning_b200 import _cabi
-    M, N = A.rows, Bm.rows
-    out = torch.empty(M, N, device="cuda")
-    pr = torch.zeros(148, 16, device="cuda", dtype=torch.int64)
-    p = lambda t: None if t is None else t.data_ptr()
-    for _ in range(3):
-        _cabi.call("caphn_gemm_tc_prof", A.hi.data_ptr(), p(A.lo), A.ld, int(A.mn), Bm.hi.data_ptr(), p(Bm.lo), Bm.ld,
-                   int(Bm.mn), A.K, out.data_ptr(), out.stride(0), p(bias), M, N, 0, pr.data_ptr(),
-                   torch.cuda.current_stream().cuda_stream)
-    torch.cuda.synchronize()
-    a = pr.double().mean(0).tolist()
-    mx = pr.double().max(0).values.tolist()
-    us = lambda c: c / 1.9e3
-    print(f"  {name}: units/CTA {a[9]:.1f} | producer total {us(a[8]):6.1f} us, waits: free stage {us(a[0]):6.1f}, A slab {us(a[1]):5.1f} | "
-          f"MMA total {us(a[4]):6.1f} (max {us(mx[4]):6.1f}), waits: operands {us(a[2]):6.1f}, accumulator {us(a[3]):6.1f} | "
-          f"epilogue total {us(a[7]):6.1f}, waits: accumulator {us(a[5]):6.1f}, store reads {us(a[6]):6.1f}", flush=True)
-
-
-print("wait-time breakdown (cycles / 1.9 GHz):")
-for H in (150, 200):
-    X = torch.randn(M, H, generator=g).cuda()
-    W = (torch.randn(V, H, generator=g) * 0.2).cuda()
-    b = torch.randn(V, generator=g).cuda()
-    xs, ws = ops.split_bf16(X), ops.split_bf16(W)
-    for mode in ("0", "1"):
-        os.environ["CAPHN_TC_ASTAT"] = mode
-        prof(xs, ws, f"logits H={H} astat={mode}", b)
-    os.environ.pop("CAPHN_TC_ASTAT", None)
-    tgt = torch.randint(0, V, (M,), generator=g).cuda()
-    logits = ops.gemm_tc(xs, ws, bias=b)
-    lb1, lse1, hi, lo = ops.ce_fwd_split(logits, tgt, 0)
-    d = ops.SplitOperand(hi, lo, M, V, hi.shape[1])
-    dT = ops.SplitOperand(hi, lo, V, M, hi.shape[1], True)
-    prof(d, ops.split_bf16_t(W), f"dH H={H}")
-    prof(dT, ops.split_bf16_t(X, ones_row=True), f"dW H={H}")
