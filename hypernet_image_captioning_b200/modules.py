@@ -193,6 +193,58 @@ def _run_grouped(fn, groups: torch.Tensor, tensors, n_groups: int):
     return tuple(torch.cat(o, 0).index_select(0, inv) for o in outs)
 
 
+def _beam_search(setup, beam_size, V, max_steps, end_sentence, sync_every):
+    """Device-resident beam search of HyperNet.test_step (hypernet_attention.py:247-326) for B images at once, around a
+    captioner's decoder step; returns a list of B results, each the best complete token sequence (leading 0, trailing
+    ``end_sentence``) or ``None`` where a beam is still open after ``max_steps`` + 1 steps.
+
+    ``setup(rep)`` runs after the argument checks and returns ``(h0 [B, H], step_fn)``; ``rep`` repeats a [B, ...] tensor
+    for the beams (rows b*k + j: beam j of image b).  ``step_fn(step, h, prev_tok, words)`` runs decoder step ``step``
+    (1-based) from the state ``h`` [B*k, H] -- ``rep(h0)`` at step 1 -- and the tokens the previous step chose
+    (``prev_tok`` int32, or ``words``: the embedding rows to feed, -1 = zero vector) and returns ``(logits [B*k, V],
+    h_out [B*k, H])``; it must not write ``h``.  Between steps ONE kernel per step (csrc/beam.cu, a CTA per image) does
+    the reference's host bookkeeping on the device; the host reads the results in one copy at the end and only peeks at
+    an 'all images finished' flag every ``sync_every`` steps to stop early."""
+    k = int(beam_size)
+    if not 1 <= k <= 8:
+        raise ValueError(f"beam_size {k} outside [1, 8]")
+    if k > V:
+        raise ValueError(f"beam_size {k} exceeds the vocabulary size {V}")
+    rep = lambda x: x.unsqueeze(1).expand(-1, k, *x.shape[1:]).reshape(x.shape[0] * k, *x.shape[1:]).contiguous()
+    h0, step_fn = setup(rep)
+    (B, H), dev = h0.shape, h0.device
+    R, L = B * k, int(max_steps) + 3
+    h = rep(h0)
+    i32 = lambda *s: torch.zeros(*s, device=dev, dtype=torch.int32)
+    h_next = torch.zeros(R, H, device=dev, dtype=torch.float32)     # rows of finished beams stay finite
+    scores = torch.zeros(R, device=dev, dtype=torch.float32)
+    live = torch.full((B,), k, device=dev, dtype=torch.int32)
+    prev_tok, ncomp, failed = i32(R), i32(B), i32(B)
+    words = torch.full((R,), -1, device=dev, dtype=torch.int64)  # every beam starts from word 0 -> zero embeddings (:265-266)
+    seq = [i32(R, L), i32(R, L)]                                  # histories start with the token 0
+    comp_score = torch.zeros(R, device=dev, dtype=torch.float32)
+    comp_seq, comp_len = i32(R, L), i32(R)
+    n_steps = int(max_steps) + 1
+    for step in range(1, n_steps + 1):
+        logits, h_out = step_fn(step, h, prev_tok, words)
+        ops.beam_step(logits, h_out, h_next, scores, live, prev_tok, words, seq[(step - 1) & 1], seq[step & 1],
+                      comp_score, comp_seq, comp_len, ncomp, failed, k, step, int(end_sentence), step == n_steps)
+        h = h_next
+        if sync_every and step % sync_every == 0 and step < n_steps and int(live.max()) == 0:
+            break
+    nc, fl = ncomp.cpu().tolist(), failed.cpu().tolist()           # the one read-back of the search
+    cs, cq, cl = comp_score.cpu().view(B, k), comp_seq.cpu().view(B, k, L), comp_len.cpu().view(B, k)
+    out = []
+    for b in range(B):
+        if fl[b] or nc[b] == 0:
+            out.append(None)
+            continue
+        sc = cs[b, :nc[b]].tolist()
+        j = sc.index(max(sc))                                     # first maximum, as list.index does (:319-321)
+        out.append(cq[b, j, :int(cl[b, j])].tolist())
+    return out
+
+
 class PooledFeatureEncoder(nn.Module):
     """Stands in for the frozen ResNet-101 + trainable fc of hypernet.py:40-48: the CNN trunk is out of scope
     (BASELINE.json), so ``forward`` takes the precomputed pooled 2048-d feature and applies ``fc``."""
@@ -389,77 +441,47 @@ class DecoderGRU(nn.Module):
         W_ih, W_hh, b_ih, b_hh = [t.detach().contiguous() for t in self._cells()[0]]
         if features.dim() != 2 or features.shape[1] != W_ih.shape[1]:
             raise ValueError(f"beam_search_batched expects features [B, {W_ih.shape[1]}], got {list(features.shape)}")
-        H, V, k = self.hidden_size, self.vocab_size, int(beam_size)
-        if not 1 <= k <= 8:
-            raise ValueError(f"beam_size {k} outside [1, 8]")
-        if k > V:
-            raise ValueError(f"beam_size {k} exceeds the vocabulary size {V}")
-        feats = features.contiguous().float()
-        if h0 is None:
-            h0 = self._h0(feats)
-        B, dev = feats.shape[0], feats.device
-        R, L = B * k, int(max_steps) + 3
-        rep = lambda x: x.unsqueeze(1).expand(B, k, *x.shape[1:]).reshape(R, *x.shape[1:]).contiguous()
-        emb, fc_w, fc_b = self.embed.weight.detach(), self.fc_out.weight.detach(), self.fc_out.bias.detach()
-        xproj, vocab = ops.LinearPlan(W_ih, b_ih), ops.LinearPlan(fc_w, fc_b)
-        table = ops.linear(emb, W_ih, b_ih)                           # [V, 3H]: the input projection of every word
-        GI0 = rep(xproj(feats))                                       # rows b*k + j: beam j of image b
-        h = rep(h0.contiguous().float())
-        fused = ops.gru_decode_step_tok_ok(H)                         # else: table gather + GRU step as two launches
-        tc = ops._tc_ok(R, V, H)
-        hop = hhi = hlo = None                                        # hop: the new state's operand rows for the GEMM
-        if fused:
-            hout = torch.empty(R, H, device=dev, dtype=torch.float32)
-            if tc:
-                Kp = ops.round64(H)
-                hhi = torch.empty(R, Kp, device=dev, dtype=torch.bfloat16)
-                hlo = torch.empty(R, Kp, device=dev, dtype=torch.bfloat16) if ops.TC_SPLIT else None
-                hop = ops.SplitOperand(hhi, hlo, R, H, Kp)
-        else:
-            WhhT = ops.transpose_pad(W_hh, ops.round4(3 * H))
-        i32 = lambda *s: torch.zeros(*s, device=dev, dtype=torch.int32)
-        h_next = torch.zeros(R, H, device=dev, dtype=torch.float32)     # rows of finished beams stay finite
-        scores = torch.zeros(R, device=dev, dtype=torch.float32)
-        live = torch.full((B,), k, device=dev, dtype=torch.int32)
-        prev_tok, ncomp, failed = i32(R), i32(B), i32(B)
-        words = torch.empty(R, device=dev, dtype=torch.int64)          # (the attention search's input; unused here)
-        seq = [i32(R, L), i32(R, L)]                                  # histories start with the token 0
-        comp_score = torch.zeros(R, device=dev, dtype=torch.float32)
-        comp_seq, comp_len = i32(R, L), i32(R)
-        logits = torch.empty(R, V, device=dev, dtype=torch.float32)
-        n_steps = int(max_steps) + 1
-        for step in range(1, n_steps + 1):
+        H, V = self.hidden_size, self.vocab_size
+
+        def setup(rep):
+            feats = features.contiguous().float()
+            h_init = self._h0(feats) if h0 is None else h0
+            dev = feats.device
+            emb, fc_w, fc_b = self.embed.weight.detach(), self.fc_out.weight.detach(), self.fc_out.bias.detach()
+            xproj, vocab = ops.LinearPlan(W_ih, b_ih), ops.LinearPlan(fc_w, fc_b)
+            table = ops.linear(emb, W_ih, b_ih)                       # [V, 3H]: the input projection of every word
+            GI0 = rep(xproj(feats))
+            R = GI0.shape[0]
+            fused = ops.gru_decode_step_tok_ok(H)                     # else: table gather + GRU step as two launches
+            hop = hhi = hlo = None                                    # hop: the new state's operand rows for the GEMM
             if fused:
-                if step == 1:
-                    ops.gru_decode_step(GI0, None, None, 0, None, W_hh, b_hh, h, hout, hhi, hlo)
+                hout = torch.empty(R, H, device=dev, dtype=torch.float32)
+                if ops._tc_ok(R, V, H):
+                    Kp = ops.round64(H)
+                    hhi = torch.empty(R, Kp, device=dev, dtype=torch.bfloat16)
+                    hlo = torch.empty(R, Kp, device=dev, dtype=torch.bfloat16) if ops.TC_SPLIT else None
+                    hop = ops.SplitOperand(hhi, hlo, R, H, Kp)
+            else:
+                WhhT = ops.transpose_pad(W_hh, ops.round4(3 * H))
+            logits = torch.empty(R, V, device=dev, dtype=torch.float32)
+
+            def step_fn(step, h, prev_tok, words):                    # (``words`` is the attention search's input)
+                if fused:
+                    if step == 1:
+                        ops.gru_decode_step(GI0, None, None, 0, None, W_hh, b_hh, h, hout, hhi, hlo)
+                    else:
+                        ops.gru_decode_step_tok(prev_tok, table, W_hh, b_hh, h, hout, hhi, hlo)
+                    h_out = hout
                 else:
-                    ops.gru_decode_step_tok(prev_tok, table, W_hh, b_hh, h, hout, hhi, hlo)
-            else:
-                GI = GI0 if step == 1 else ops.gather_rows(table, prev_tok.long())
-                hout = ops.gru_seq_fwd(GI, WhhT, b_hh, h, 1, save=False, want_bm=False)[0][1]
-            if hop is not None:
-                ops.gemm_tc(hop, vocab.operand(), bias=fc_b, out=logits)
-            else:
-                vocab(hout, out=logits)
-            ops._cabi.call("caphn_beam_step", logits.data_ptr(), hout.data_ptr(), h_next.data_ptr(), scores.data_ptr(),
-                           live.data_ptr(), prev_tok.data_ptr(), words.data_ptr(), seq[(step - 1) & 1].data_ptr(),
-                           seq[step & 1].data_ptr(), comp_score.data_ptr(), comp_seq.data_ptr(), comp_len.data_ptr(),
-                           ncomp.data_ptr(), failed.data_ptr(), B, k, V, H, L, step, int(end_sentence),
-                           int(step == n_steps), ops._stream())
-            h = h_next                                                # the decode step never writes the state it reads
-            if sync_every and step % sync_every == 0 and step < n_steps and int(live.max()) == 0:
-                break
-        nc, fl = ncomp.cpu().tolist(), failed.cpu().tolist()           # the one read-back of the search
-        cs, cq, cl = comp_score.cpu().view(B, k), comp_seq.cpu().view(B, k, L), comp_len.cpu().view(B, k)
-        out = []
-        for b in range(B):
-            if fl[b] or nc[b] == 0:
-                out.append(None)
-                continue
-            sc = cs[b, :nc[b]].tolist()
-            j = sc.index(max(sc))                                     # first maximum, as list.index does (:319-321)
-            out.append(cq[b, j, :int(cl[b, j])].tolist())
-        return out
+                    GI = GI0 if step == 1 else ops.gather_rows(table, prev_tok.long())
+                    h_out = ops.gru_seq_fwd(GI, WhhT, b_hh, h, 1, save=False, want_bm=False)[0][1]
+                if hop is not None:
+                    ops.gemm_tc(hop, vocab.operand(), bias=fc_b, out=logits)
+                else:
+                    vocab(h_out, out=logits)
+                return logits, h_out
+            return h_init.contiguous().float(), step_fn
+        return _beam_search(setup, beam_size, V, max_steps, end_sentence, sync_every)
 
 
 class DecoderRNN(DecoderGRU):

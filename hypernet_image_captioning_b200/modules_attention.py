@@ -11,7 +11,7 @@ from torch.autograd import Function
 
 from . import functional as Fn
 from . import ops, streams
-from .modules import RowsLinear, _Base, _HyperNetMixin, _run_grouped
+from .modules import RowsLinear, _Base, _HyperNetMixin, _beam_search, _run_grouped
 
 
 class FeatureFn(Function):
@@ -423,84 +423,17 @@ class AttentionGru(nn.Module):
         Reference quirks kept: every row starts from word 0 and ALL rows get a zero word embedding whenever the first
         row's previous word is 0 (:265-266); step 1 ranks ``scores[0]`` only (:274-275); scores are summed
         log-probabilities without length normalisation; finished beams leave the batch (:296-303).
-        Each step runs the recurrence kernels on the k live rows; the top-k bookkeeping is host logic as in the reference."""
-        streams.wait_pending()
-        feats = features.contiguous().float()
-        if feats.dim() != 3 or feats.shape[0] != 1:
+        Runs ``beam_search_batched`` on the one image, so ``beam_size`` must lie in [1, 8] and not exceed V."""
+        if features.dim() != 3 or features.shape[0] != 1:
             raise ValueError("beam_search expects the features of one image: [1, P, D]")
-        _, P, D = feats.shape
-        W_ih, W_hh, b_ih, b_hh = [w.detach().contiguous() for w in self._gru_weights()]
-        E, H, V = self.embedding_dim, self.hidden_dim, self.vocab_size
-        dev = feats.device
-        a = self.attention
-        emb_w = self.embed.weight.detach()
-        fc0, fc2 = self.feature_fc[0], self.feature_fc[2]
-        f1 = ops.linear(feats.view(P, D), fc0.weight.detach(), fc0.bias.detach(), relu=True)
-        f = ops.linear(f1, fc2.weight.detach(), fc2.bias.detach())                       # [P, F]
-        Fd = f.shape[1]
-        K1 = ops.linear(f, a.W_a.weight.detach(), a.W_a.bias.detach())                     # [P, H]
-        k = int(beam_size)
-        f3 = f.view(1, P, Fd).expand(k, P, Fd).contiguous()
-        Kp = K1.view(1, P, H).expand(k, P, H).contiguous()
-        h0 = ops.linear(ops.mean_pos(f3[:1].contiguous()), self.init_h.weight.detach(), self.init_h.bias.detach())
-        h = h0.expand(k, H).contiguous()
-        lw = ops.AttGruWeights(W_ih, W_hh, a.U_a.weight.detach().contiguous(), E, P)
-        va, bv = a.v_a.weight.detach().reshape(-1).contiguous(), a.v_a.bias.detach().reshape(1).contiguous()
-        bu = a.U_a.bias.detach().contiguous()
-        fc_w, fc_b = self.fc.weight.detach(), self.fc.bias.detach()
-        W_ih_w = W_ih[:, :E]
-        prev = [0] * k
-        seqs = [[0] for _ in range(k)]
-        top_scores = torch.zeros(k, device=dev)
-        complete, complete_scores = [], []
-        step = 1
-        while True:
-            kc = len(prev)
-            prev_t = torch.tensor(prev, device=dev, dtype=torch.int64)
-            xw = ops.gather_rows(emb_w, prev_t)
-            if prev[0] == 0:
-                xw.zero_()
-            GIw = ops.linear(xw, W_ih_w, b_ih)
-            Hall = torch.empty(2, kc, H, device=dev, dtype=torch.float32)
-            Hall[0].copy_(h)
-            attn = torch.empty(kc, 1, P, device=dev, dtype=torch.float32)
-            XC = torch.empty(kc, E + Fd, device=dev, dtype=torch.float32)
-            ops.attgru_fwd(Kp[:kc], f3[:kc], GIw, lw, bu, va, bv, b_hh, Hall, None, attn, XC, E, None, 0, 1)
-            h = Hall[1]
-            logits = ops.linear(h, fc_w, fc_b)                                            # [kc, V]
-            _, lse = ops.ce_fwd(logits, torch.zeros(kc, device=dev, dtype=torch.int64), None)
-            scores = top_scores[:kc, None] + (logits - lse[:, None])                      # log_softmax + running score
-            flat = scores[0] if step == 1 else scores.reshape(-1)
-            top_scores, top_words = flat.topk(k, 0, True, True)
-            words = top_words.tolist()
-            prev_inds = [w // V for w in words]
-            next_inds = [w % V for w in words]
-            seqs = [seqs[pi] + [ni] for pi, ni in zip(prev_inds, next_inds)]
-            incomplete = [i for i, w in enumerate(next_inds) if w != end_sentence]
-            done = [i for i in range(len(next_inds)) if i not in incomplete]
-            if done:
-                sc = top_scores.tolist()
-                complete.extend(seqs[i] for i in done)
-                complete_scores.extend(sc[i] for i in done)
-            k -= len(done)
-            if k == 0:
-                break
-            seqs = [seqs[i] for i in incomplete]
-            sel = torch.tensor([prev_inds[i] for i in incomplete], device=dev, dtype=torch.int64)
-            h = h.index_select(0, sel)
-            top_scores = top_scores[torch.tensor(incomplete, device=dev, dtype=torch.int64)]
-            prev = [next_inds[i] for i in incomplete]
-            if step > max_steps:
-                return None
-            step += 1
-        return complete[complete_scores.index(max(complete_scores))]
+        return self.beam_search_batched(features, beam_size, end_sentence, max_steps)[0]
 
     @torch.no_grad()
     def beam_search_batched(self, features, beam_size=3, end_sentence=2, max_steps=50, sync_every=8):
         """Beam search of HyperNet.test_step (hypernet_attention.py:247-326) for a whole batch at once, device-resident:
         ``features`` [B, P, D] -> list of B results, each the best complete token sequence (leading 0, trailing
         ``end_sentence``) or ``None`` where the reference computes no beam caption (a beam still open after
-        ``max_steps`` + 1 steps).  Same per-image semantics -- and the same results -- as ``beam_search``.
+        ``max_steps`` + 1 steps).  ``beam_size`` in [1, 8], at most V.
 
         All B*k beams go through the decoder step kernels together; between steps ONE kernel per step
         (csrc/beam.cu, a CTA per image) does the reference's host bookkeeping on the device: log-softmax + running scores,
@@ -508,69 +441,36 @@ class AttentionGru(nn.Module):
         state gathered from the parent beam), next input words.  The host reads the results in one copy at the end; it
         only peeks at an 'all images finished' flag every ``sync_every`` steps to stop early."""
         streams.wait_pending()
-        feats = features.contiguous().float()
-        if feats.dim() != 3:
+        if features.dim() != 3:
             raise ValueError("beam_search_batched expects features [B, P, D]")
-        B, P, D = feats.shape
-        k = int(beam_size)
         E, H, V = self.embedding_dim, self.hidden_dim, self.vocab_size
-        if k > V:
-            raise ValueError(f"beam_size {k} exceeds the vocabulary size {V}")
-        W_ih, W_hh, b_ih, b_hh = [w.detach().contiguous() for w in self._gru_weights()]
-        dev = feats.device
-        a = self.attention
-        emb_w = self.embed.weight.detach()
-        f3, K3, h0 = FeatureFn.apply(feats, *[p.detach() for p in self._feature_params()])
-        Fd = f3.shape[2]
-        rep = lambda x: x.unsqueeze(1).expand(B, k, *x.shape[1:]).reshape(B * k, *x.shape[1:]).contiguous()
-        f3k, K3k = rep(f3), rep(K3)                                   # rows b*k + j: beam j of image b
-        R, L = B * k, int(max_steps) + 3
-        lw = ops.AttGruWeights(W_ih, W_hh, a.U_a.weight.detach().contiguous(), E, P)
-        va, bv = a.v_a.weight.detach().reshape(-1).contiguous(), a.v_a.bias.detach().reshape(1).contiguous()
-        bu = a.U_a.bias.detach().contiguous()
-        xproj, vocab = ops.LinearPlan(W_ih[:, :E], b_ih), ops.LinearPlan(self.fc.weight.detach(), self.fc.bias.detach())
-        i32 = lambda *s: torch.zeros(*s, device=dev, dtype=torch.int32)
-        Hall = torch.empty(2, R, H, device=dev, dtype=torch.float32)
-        Hall[0].copy_(rep(h0))
-        h_next = torch.zeros(R, H, device=dev, dtype=torch.float32)     # rows of finished beams stay finite
-        scores = torch.zeros(R, device=dev, dtype=torch.float32)
-        live = torch.full((B,), k, device=dev, dtype=torch.int32)
-        prev_tok, ncomp, failed = i32(R), i32(B), i32(B)
-        words = torch.full((R,), -1, device=dev, dtype=torch.int64)  # every beam starts from word 0 -> zero embeddings (:265-266)
-        seq = [i32(R, L), i32(R, L)]                                  # histories start with the token 0
-        comp_score = torch.zeros(R, device=dev, dtype=torch.float32)
-        comp_seq, comp_len = i32(R, L), i32(R)
-        attn = torch.empty(R, 1, P, device=dev, dtype=torch.float32)
-        XC = torch.empty(R, E + Fd, device=dev, dtype=torch.float32)
-        GIw = torch.empty(R, 3 * H, device=dev, dtype=torch.float32)
-        logits = torch.empty(R, V, device=dev, dtype=torch.float32)
-        n_steps = int(max_steps) + 1
-        for step in range(1, n_steps + 1):
-            xw = ops.gather_rows(emb_w, words)                        # zeros where words == -1
-            xproj(xw, out=GIw)
-            ops.attgru_fwd(K3k, f3k, GIw, lw, bu, va, bv, b_hh, Hall, None, attn, XC, E, None, 0, 1)
-            lw._resume = None                                         # Hall[0] is rewritten below: re-convert next step
-            vocab(Hall[1], out=logits)
-            _cabi_call = ops._cabi.call
-            _cabi_call("caphn_beam_step", logits.data_ptr(), Hall[1].data_ptr(), h_next.data_ptr(), scores.data_ptr(),
-                       live.data_ptr(), prev_tok.data_ptr(), words.data_ptr(), seq[(step - 1) & 1].data_ptr(),
-                       seq[step & 1].data_ptr(), comp_score.data_ptr(), comp_seq.data_ptr(), comp_len.data_ptr(),
-                       ncomp.data_ptr(), failed.data_ptr(), B, k, V, H, L, step, int(end_sentence),
-                       int(step == n_steps), ops._stream())
-            Hall[0].copy_(h_next)
-            if sync_every and step % sync_every == 0 and step < n_steps and int(live.max()) == 0:
-                break
-        nc, fl = ncomp.cpu().tolist(), failed.cpu().tolist()           # the one read-back of the search
-        cs, cq, cl = comp_score.cpu().view(B, k), comp_seq.cpu().view(B, k, L), comp_len.cpu().view(B, k)
-        out = []
-        for b in range(B):
-            if fl[b] or nc[b] == 0:
-                out.append(None)
-                continue
-            sc = cs[b, :nc[b]].tolist()
-            j = sc.index(max(sc))                                     # first maximum, as list.index does (:319-321)
-            out.append(cq[b, j, :int(cl[b, j])].tolist())
-        return out
+
+        def setup(rep):
+            feats = features.contiguous().float()
+            P, dev = feats.shape[1], feats.device
+            W_ih, W_hh, b_ih, b_hh = [w.detach().contiguous() for w in self._gru_weights()]
+            a = self.attention
+            emb_w = self.embed.weight.detach()
+            f3, K3, h0 = FeatureFn.apply(feats, *[p.detach() for p in self._feature_params()])
+            f3k, K3k = rep(f3), rep(K3)
+            R, Fd = f3k.shape[0], f3.shape[2]
+            lw = ops.AttGruWeights(W_ih, W_hh, a.U_a.weight.detach().contiguous(), E, P)
+            va, bv = a.v_a.weight.detach().reshape(-1).contiguous(), a.v_a.bias.detach().reshape(1).contiguous()
+            bu = a.U_a.bias.detach().contiguous()
+            xproj, vocab = ops.LinearPlan(W_ih[:, :E], b_ih), ops.LinearPlan(self.fc.weight.detach(), self.fc.bias.detach())
+            Hall = torch.empty(2, R, H, device=dev, dtype=torch.float32)
+            attn = torch.empty(R, 1, P, device=dev, dtype=torch.float32)
+            XC = torch.empty(R, E + Fd, device=dev, dtype=torch.float32)
+            GIw = torch.empty(R, 3 * H, device=dev, dtype=torch.float32)
+            logits = torch.empty(R, V, device=dev, dtype=torch.float32)
+
+            def step_fn(step, h, prev_tok, words):
+                xproj(ops.gather_rows(emb_w, words), out=GIw)          # zeros where words == -1
+                Hall[0].copy_(h)
+                ops.attgru_fwd(K3k, f3k, GIw, lw, bu, va, bv, b_hh, Hall, None, attn, XC, E, None, 0, 1)
+                return vocab(Hall[1], out=logits), Hall[1]
+            return h0, step_fn
+        return _beam_search(setup, beam_size, V, max_steps, end_sentence, sync_every)
 
     @torch.no_grad()
     def greedy_search(self, features, end_sentence=2, max_sentence=20):

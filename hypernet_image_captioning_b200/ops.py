@@ -791,6 +791,25 @@ def gru_decode_step_tok(tok, table, W_hh, b_hh, hprev, hnew, hi=None, lo=None):
     return hnew
 
 
+def beam_step(logits, h_out, h_next, scores, live, prev_tok, words, seq_in, seq_out, comp_score, comp_seq, comp_len, ncomp,
+              failed, k, step, end_tok, last):
+    """One bookkeeping step of the batched beam search (csrc/beam.cu, caphn_beam_step) for B = live.numel() images x k
+    beams: log-softmax + running scores, top-k of the live rows' candidates, completed beams to the complete list,
+    survivors compacted (history, score, hidden state h_out -> h_next), next input words.  logits [B*k, V], h_out /
+    h_next [B*k, H], token histories seq_in / seq_out / comp_seq [B*k, L]; step is 1-based, ``last`` marks the final one."""
+    for t in (logits, h_out, h_next, scores, comp_score):
+        _chk(t)
+    for t in (live, prev_tok, seq_in, seq_out, comp_seq, comp_len, ncomp, failed):
+        _chk(t, torch.int32)
+    _chk(words, torch.int64)
+    assert all(t.is_contiguous() for t in (logits, h_out, h_next, scores, live, prev_tok, words, seq_in, seq_out,
+                                           comp_score, comp_seq, comp_len, ncomp, failed))
+    _cabi.call("caphn_beam_step", logits.data_ptr(), h_out.data_ptr(), h_next.data_ptr(), scores.data_ptr(),
+               live.data_ptr(), prev_tok.data_ptr(), words.data_ptr(), seq_in.data_ptr(), seq_out.data_ptr(),
+               comp_score.data_ptr(), comp_seq.data_ptr(), comp_len.data_ptr(), ncomp.data_ptr(), failed.data_ptr(),
+               live.numel(), k, logits.shape[1], h_out.shape[1], seq_in.shape[1], step, end_tok, int(last), _stream())
+
+
 def attstep_h_operand(lw, B, H, Fd, t_done):
     """The hidden state h_{t_done} as the bf16 hi/lo operand rows the step-split gates kernel has just written into its
     workspace for the next step's U kernel (attgru_step.cu: hsp buffers) -- the A operand of the vocabulary projection,

@@ -309,10 +309,9 @@ def beam_step_ref(t, k, V, L, step, end_tok, last):
 def beam_step_gpu(t, k, V, L, step, end_tok, last):
     ops = _ops()
     d = {name: x.cuda() for name, x in t.items()}
-    H = t["h_out"].shape[1]
-    ops._cabi.call("caphn_beam_step", *[d[n].data_ptr() for n in (
+    ops.beam_step(*[d[n] for n in (
         "logits", "h_out", "h_next", "scores", "live", "prev_tok", "words", "seq_in", "seq_out", "comp_score", "comp_seq",
-        "comp_len", "ncomp", "failed")], t["live"].numel(), k, V, H, L, step, end_tok, last, ops._stream())
+        "comp_len", "ncomp", "failed")], k, step, end_tok, last)
     torch.cuda.synchronize()
     return {name: d[name].cpu() for name in BEAM_OUT}
 

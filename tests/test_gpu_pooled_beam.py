@@ -127,6 +127,13 @@ def test_argument_errors():
         dec.beam_search_batched(torch.zeros(2, 7))
     with pytest.raises(NotImplementedError):
         C.DecoderRNN(8, 6, 5).beam_search_batched(f)
+    att = C.AttentionGru(2048, 8, 6, 6, 5)          # the same checks, before the feature branch runs
+    fa = torch.zeros(2, 49, 2048)
+    for k in (0, 9, 6):
+        with pytest.raises(ValueError):
+            att.beam_search_batched(fa, beam_size=k)
+    with pytest.raises(ValueError):
+        att.beam_search(fa)
 
 
 # ----------------------------------------------------------------------------------------------------------------------
