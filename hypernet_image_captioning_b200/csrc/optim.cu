@@ -175,12 +175,14 @@ __global__ void __launch_bounds__(OPT_THREADS) adam_lowrank_kernel(const AdamLrA
         }
 #pragma unroll
         for (int u = 0; u < LR_UNR; ++u) {
-            float g[4];
-            long n = nn[u]; int k = kk[u];
-#pragma unroll
-            for (int c = 0; c < 4; ++c) { g[c] = lowrank_g<G>(a, n, k); if (++k == a.K) { k = 0; ++n; } }
+            const long n0 = nn[u]; const int k0 = kk[u];
             nn[u] += dq; kk[u] += dr; if (kk[u] >= a.K) { kk[u] -= a.K; ++nn[u]; }
+            // a slot past the end has (n0, k0) beyond row N - 1: dP must not be read there
             if (u == 0 || i + u * stride < n4) {
+                float g[4];
+                long n = n0; int k = k0;
+#pragma unroll
+                for (int c = 0; c < 4; ++c) { g[c] = lowrank_g<G>(a, n, k); if (++k == a.K) { k = 0; ++n; } }
                 adam_one(pv[u].x, g[0], mv[u].x, vv[u].x, h, gs); adam_one(pv[u].y, g[1], mv[u].y, vv[u].y, h, gs);
                 adam_one(pv[u].z, g[2], mv[u].z, vv[u].z, h, gs); adam_one(pv[u].w, g[3], mv[u].w, vv[u].w, h, gs);
                 stg_stream4(reinterpret_cast<float*>(p4 + idx[u]), pv[u]);
