@@ -31,6 +31,8 @@ SIGNATURES = {
     "caphn_gemm_tc_ex": [P, P, L, I, P, P, L, I, L, P, L, P, I, I, I, I, P],
     "caphn_transpose_pad": [P, L, P, L, I, I, P],
     "caphn_copy_pad": [P, L, P, L, L, I, P],
+    "caphn_transpose_pad_batched": [P, L, L, P, L, L, I, I, I, P],
+    "caphn_copy_pad_batched": [P, L, L, P, L, L, I, L, I, P],
     "caphn_gru_seq_fwd": [P, P, I, P, P, P, P, P, P, I, I, I, I, P],
     "caphn_gru_seq_bwd": [P, P, P, P, P, I, P, P, P, P, P, P, I, I, I, I, P],
     "caphn_gru_cluster_plan": [I, P],
@@ -49,6 +51,8 @@ SIGNATURES = {
     "caphn_colsum": [P, L, L, I, P, P],
     "caphn_lstm_seq_fwd": [P, P, I, P, P, P, P, P, P, P, P, I, I, I, I, P],
     "caphn_lstm_seq_bwd": [P, P, P, I, P, P, P, I, I, I, I, P],
+    "caphn_lstm_seq_fwd_grouped": [P, P, I, P, L, P, P, P, P, I, I, I, P, I, P],
+    "caphn_lstm_seq_bwd_grouped": [P, P, P, I, P, P, I, I, I, P, I, P],
     "caphn_attgru_seq_fwd": [P] * 14 + [L] + [P] * 5 + [I] * 9 + [P],
     "caphn_attgru_seq_bwd": [P] * 23 + [I] * 7 + [P],
     "caphn_attstep_pack_size": [I, I, I, I, P, P],

@@ -196,10 +196,13 @@ __global__ void __launch_bounds__(AT_THREADS) gru_seq_bwd_kernel(const GruBwdArg
     }
 }
 
-// dst[c*ldd + r] = src[r*lds + c]  (r < R, c < C); pad columns [R, ldd) of dst are zeroed.
+// dst[c*ldd + r] = src[r*lds + c]  (r < R, c < C); pad columns [R, ldd) of dst are zeroed.  blockIdx.z = matrix z of a
+// batch: src + z * sstride -> dst + z * dstride.
 __global__ void transpose_pad_kernel(const float* __restrict__ src, long lds, float* __restrict__ dst, long ldd, int R,
-                                     int C) {
+                                     int C, long sstride, long dstride) {
     __shared__ float tile[32][33];
+    src += blockIdx.z * sstride;
+    dst += blockIdx.z * dstride;
     const int r0 = blockIdx.y * 32, c0 = blockIdx.x * 32;
     for (int i = threadIdx.y; i < 32; i += blockDim.y) {
         const int r = r0 + i, c = c0 + threadIdx.x;
@@ -212,11 +215,13 @@ __global__ void transpose_pad_kernel(const float* __restrict__ src, long lds, fl
     }
 }
 
-// dst[r*ldd + c] = c < C ? src[r*lds + c] : 0
+// dst[r*ldd + c] = c < C ? src[r*lds + c] : 0;  blockIdx.y = matrix y of a batch (src + y * sstride -> dst + y * dstride)
 __global__ void copy_pad_kernel(const float* __restrict__ src, long lds, float* __restrict__ dst, long ldd, long R,
-                                int C) {
+                                int C, long sstride, long dstride) {
     const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= R * ldd) return;
+    src += blockIdx.y * sstride;
+    dst += blockIdx.y * dstride;
     const long r = i / ldd;
     const int c = (int)(i - r * ldd);
     dst[i] = c < C ? src[r * lds + c] : 0.f;
@@ -231,13 +236,30 @@ extern "C" {
 int caphn_transpose_pad(const float* src, long lds, float* dst, long ldd, int R, int C, void* stream) {
     if (R <= 0 || C <= 0 || ldd < R) return CAPHN_EINVAL;
     dim3 grid(ceil_div(C, 32), ceil_div(ldd, 32));
-    transpose_pad_kernel<<<grid, dim3(32, 8), 0, (cudaStream_t)stream>>>(src, lds, dst, ldd, R, C);
+    transpose_pad_kernel<<<grid, dim3(32, 8), 0, (cudaStream_t)stream>>>(src, lds, dst, ldd, R, C, 0, 0);
     CAPHN_RETURN_LAST();
 }
 
 int caphn_copy_pad(const float* src, long lds, float* dst, long ldd, long R, int C, void* stream) {
     if (R <= 0 || C <= 0 || ldd < C) return CAPHN_EINVAL;
-    copy_pad_kernel<<<ceil_div(R * ldd, 256), 256, 0, (cudaStream_t)stream>>>(src, lds, dst, ldd, R, C);
+    copy_pad_kernel<<<ceil_div(R * ldd, 256), 256, 0, (cudaStream_t)stream>>>(src, lds, dst, ldd, R, C, 0, 0);
+    CAPHN_RETURN_LAST();
+}
+
+// nb matrices in one launch: matrix z at src + z * sstride -> dst + z * dstride (floats); dst pitch ldd as above.
+int caphn_transpose_pad_batched(const float* src, long sstride, long lds, float* dst, long dstride, long ldd, int nb,
+                                int R, int C, void* stream) {
+    if (nb <= 0 || nb > 65535 || R <= 0 || C <= 0 || ldd < R || dstride < (long)C * ldd) return CAPHN_EINVAL;
+    dim3 grid(ceil_div(C, 32), ceil_div(ldd, 32), nb);
+    transpose_pad_kernel<<<grid, dim3(32, 8), 0, (cudaStream_t)stream>>>(src, lds, dst, ldd, R, C, sstride, dstride);
+    CAPHN_RETURN_LAST();
+}
+
+int caphn_copy_pad_batched(const float* src, long sstride, long lds, float* dst, long dstride, long ldd, int nb, long R,
+                           int C, void* stream) {
+    if (nb <= 0 || nb > 65535 || R <= 0 || C <= 0 || ldd < C || dstride < R * ldd) return CAPHN_EINVAL;
+    copy_pad_kernel<<<dim3(ceil_div(R * ldd, 256), nb), 256, 0, (cudaStream_t)stream>>>(src, lds, dst, ldd, R, C, sstride,
+                                                                                       dstride);
     CAPHN_RETURN_LAST();
 }
 

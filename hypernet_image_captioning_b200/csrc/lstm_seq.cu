@@ -9,7 +9,8 @@
 // The pre-activation is a plain sum gi + gh, so one gate-gradient array dG serves both weight-gradient products.
 //
 // Same decomposition as gru_seq.cu: a CTA owns 4 batch rows and keeps (h, c) in shared memory; the generated weights
-// (k-major, 16-byte rows) stream from L2 every step.
+// (k-major, 16-byte rows) stream from L2 every step.  The grouped kernels run the same rows code for a many-style batch:
+// each CTA takes a tile of <= 4 rows of one style group and that group's slice of a per-group weight pack.
 #include "seq_common.cuh"
 
 namespace caphn {
@@ -33,7 +34,10 @@ struct LstmFwdArgs {
     int NL, B, T, H, ld4;
 };
 
-__global__ void __launch_bounds__(AT_THREADS) lstm_seq_fwd_kernel(const LstmFwdArgs a) {
+// Batch rows [b0, b0 + nb) (nb <= AT_BT) of the whole recurrence; cell 0 uses WhhT / bhh.  The single-style kernel passes
+// the CTA's 4 rows and the call's weights, the grouped kernel a tile of one style group and that group's weights.
+__device__ __forceinline__ void lstm_fwd_rows(const LstmFwdArgs& a, const float* __restrict__ WhhT,
+                                              const float* __restrict__ bhh0, int b0, int nb) {
     constexpr int BT = AT_BT;
     extern __shared__ __align__(16) float smem[];
     const int H = a.H, B = a.B, T = a.T, ld4 = a.ld4, H4 = 4 * a.H;
@@ -43,16 +47,15 @@ __global__ void __launch_bounds__(AT_THREADS) lstm_seq_fwd_kernel(const LstmFwdA
     float* part_gh = cs + ((BT * H + 3) & ~3);  // [KG][BT][ld4]
     float* part_gi = part_gh + KG * BT * ld4;   // [KG][BT][ld4]   (extra layers only)
     const int tid = threadIdx.x;
-    const int b0 = blockIdx.x * BT;
     const long TBH = (long)T * B * H;
 
     for (int i = tid; i < H * BT; i += AT_THREADS) {
         const int k = i / BT, b = i - k * BT;
-        hs[i] = (b0 + b < B) ? a.Hall[(long)(b0 + b) * H + k] : 0.f;
+        hs[i] = (b < nb) ? a.Hall[(long)(b0 + b) * H + k] : 0.f;
     }
     for (int i = tid; i < BT * H; i += AT_THREADS) {
         const int b = i / H, j = i - b * H;
-        cs[i] = (a.c0 && b0 + b < B) ? a.c0[(long)(b0 + b) * H + j] : 0.f;
+        cs[i] = (a.c0 && b < nb) ? a.c0[(long)(b0 + b) * H + j] : 0.f;
     }
     __syncthreads();
 
@@ -60,17 +63,17 @@ __global__ void __launch_bounds__(AT_THREADS) lstm_seq_fwd_kernel(const LstmFwdA
         for (int l = 0; l < a.NL; ++l) {
             const bool last = (l == a.NL - 1);
             if (l == 0) {
-                block_matvec<BT, false>(a.WhhT, ld4, H, hs, part_gh, CQT, tid);
+                block_matvec<BT, false>(WhhT, ld4, H, hs, part_gh, CQT, tid);
             } else {
                 block_matvec<BT, false>(a.xWihT[l - 1], ld4, H, hs, part_gi, CQT, tid);
                 block_matvec<BT, false>(a.xWhhT[l - 1], ld4, H, hs, part_gh, CQT, tid);
             }
             __syncthreads();
-            const float* bhh = (l == 0) ? a.bhh : a.xbhh[l - 1];
+            const float* bhh = (l == 0) ? bhh0 : a.xbhh[l - 1];
             for (int i = tid; i < BT * H; i += AT_THREADS) {
                 const int b = i / H, j = i - b * H;
                 const int gb = b0 + b;
-                if (gb < B) {
+                if (b < nb) {
                     float g4[4];
 #pragma unroll
                     for (int q = 0; q < 4; ++q) {
@@ -105,8 +108,21 @@ __global__ void __launch_bounds__(AT_THREADS) lstm_seq_fwd_kernel(const LstmFwdA
     if (a.cT)
         for (int i = tid; i < BT * H; i += AT_THREADS) {
             const int b = i / H, j = i - b * H;
-            if (b0 + b < B) a.cT[(long)(b0 + b) * H + j] = cs[i];
+            if (b < nb) a.cT[(long)(b0 + b) * H + j] = cs[i];
         }
+}
+
+__global__ void __launch_bounds__(AT_THREADS) lstm_seq_fwd_kernel(const LstmFwdArgs a) {
+    const int b0 = blockIdx.x * AT_BT;
+    lstm_fwd_rows(a, a.WhhT, a.bhh, b0, min(AT_BT, a.B - b0));
+}
+
+// Many-style batch (rows sorted by group, one layer): CTA i runs tile i = {first row, rows <= AT_BT, group, 0} with its
+// group's slice [H][ld4] of the W_hh^T pack and b_hh at bhh + group * bstride.
+__global__ void __launch_bounds__(AT_THREADS) lstm_seq_fwd_grouped_kernel(const LstmFwdArgs a, const int4* __restrict__ tiles,
+                                                                          long bstride) {
+    const int4 tl = tiles[blockIdx.x];
+    lstm_fwd_rows(a, a.WhhT + (long)tl.z * a.H * a.ld4, a.bhh + (long)tl.z * bstride, tl.x, tl.y);
 }
 
 struct LstmBwdArgs {
@@ -120,7 +136,8 @@ struct LstmBwdArgs {
     int NL, B, T, H, ldh;
 };
 
-__global__ void __launch_bounds__(AT_THREADS) lstm_seq_bwd_kernel(const LstmBwdArgs a) {
+// Batch rows [b0, b0 + nb) (nb <= AT_BT) of the BPTT; cell 0 uses Whh.
+__device__ __forceinline__ void lstm_bwd_rows(const LstmBwdArgs& a, const float* __restrict__ Whh, int b0, int nb) {
     constexpr int BT = AT_BT;
     extern __shared__ __align__(16) float smem[];
     const int H = a.H, B = a.B, T = a.T, ldh = a.ldh, H4 = 4 * a.H;
@@ -131,7 +148,6 @@ __global__ void __launch_bounds__(AT_THREADS) lstm_seq_bwd_kernel(const LstmBwdA
     float* part_dh = dhin + ((BT * H + 3) & ~3);     // [KGh][BT][ldh]  dG . W_hh of layer 0 (for the previous step)
     float* part_di = part_dh + KGh * BT * ldh;       // [KGh][BT][ldh]  dG . (W_hh + W_ih) of an extra layer
     const int tid = threadIdx.x;
-    const int b0 = blockIdx.x * BT;
     const long TBH = (long)T * B * H, TB4 = (long)T * B * H4;
 
     for (int i = tid; i < BT * H; i += AT_THREADS) dcs[i] = 0.f;
@@ -146,7 +162,7 @@ __global__ void __launch_bounds__(AT_THREADS) lstm_seq_bwd_kernel(const LstmBwdA
                 const int gb = b0 + b;
                 float da[4] = {0.f, 0.f, 0.f, 0.f};
                 float dcp = 0.f;
-                if (gb < B) {
+                if (b < nb) {
                     float dh;
                     if (top) dh = a.dHbm[((long)gb * T + t) * H + j] + part_sum(part_dh, KGh, BT, ldh, b, j);
                     else dh = dhin[i];
@@ -168,7 +184,7 @@ __global__ void __launch_bounds__(AT_THREADS) lstm_seq_bwd_kernel(const LstmBwdA
             }
             __syncthreads();
             if (l == 0) {
-                block_matvec<BT, false>(a.Whh, ldh, H4, dg, part_dh, CQTh, tid);
+                block_matvec<BT, false>(Whh, ldh, H4, dg, part_dh, CQTh, tid);
                 __syncthreads();
             } else {
                 // input and state of an extra cell are the same vector: both products flow into the cell below
@@ -185,8 +201,19 @@ __global__ void __launch_bounds__(AT_THREADS) lstm_seq_bwd_kernel(const LstmBwdA
     }
     for (int i = tid; i < BT * H; i += AT_THREADS) {
         const int b = i / H, j = i - b * H;
-        if (b0 + b < B) a.dh0[(long)(b0 + b) * H + j] = part_sum(part_dh, KGh, BT, ldh, b, j);
+        if (b < nb) a.dh0[(long)(b0 + b) * H + j] = part_sum(part_dh, KGh, BT, ldh, b, j);
     }
+}
+
+__global__ void __launch_bounds__(AT_THREADS) lstm_seq_bwd_kernel(const LstmBwdArgs a) {
+    const int b0 = blockIdx.x * AT_BT;
+    lstm_bwd_rows(a, a.Whh, b0, min(AT_BT, a.B - b0));
+}
+
+// BPTT of lstm_seq_fwd_grouped_kernel: tile i with its group's slice [4H][ldh] of the W_hh pack.
+__global__ void __launch_bounds__(AT_THREADS) lstm_seq_bwd_grouped_kernel(const LstmBwdArgs a, const int4* __restrict__ tiles) {
+    const int4 tl = tiles[blockIdx.x];
+    lstm_bwd_rows(a, a.Whh + (long)tl.z * 4 * a.H * a.ldh, tl.x, tl.y);
 }
 
 }  // namespace caphn
@@ -239,6 +266,42 @@ int caphn_lstm_seq_bwd(const float* dHbm, const float* saved, const float* Whh, 
     if (smem > 227 * 1024) return CAPHN_EINVAL;
     CAPHN_CHECK(cudaFuncSetAttribute(lstm_seq_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     lstm_seq_bwd_kernel<<<ceil_div(B, AT_BT), AT_THREADS, smem, (cudaStream_t)stream>>>(a);
+    CAPHN_RETURN_LAST();
+}
+
+// Single-layer LSTM recurrence of a many-style batch (rows sorted by style group; h0 = Hall[0], c0 = zeros).  CTA i runs
+// tiles[i] = {first row, rows (1..4), group, 0} (16-byte aligned int4 table, no tile straddles two groups) with the group's
+// W_hh^T from the pack WhhT [G][H][ld4] and b_hh = bhh + group * bstride (floats).  GI, Hall, Hbm, saved [6][T,B,H] and
+// cT (or NULL) as in caphn_lstm_seq_fwd; every row computes exactly what the single-style kernel computes for it.
+int caphn_lstm_seq_fwd_grouped(const float* GI, const float* WhhT, int ld4, const float* bhh, long bstride, float* Hall,
+                               float* Hbm, float* saved, float* cT, int B, int T, int H, const int* tiles, int ntiles,
+                               void* stream) {
+    if (B <= 0 || T <= 0 || H <= 0 || (ld4 & 3) || ld4 < 4 * H || ((uintptr_t)WhhT & 15)) return CAPHN_EINVAL;
+    if (!tiles || ntiles < 1 || ((uintptr_t)tiles & 15) || bstride < 0) return CAPHN_EINVAL;
+    LstmFwdArgs a{};
+    a.GI = GI; a.WhhT = WhhT; a.bhh = bhh; a.Hall = Hall; a.Hbm = Hbm; a.saved = saved; a.cT = cT;
+    a.NL = 1; a.B = B; a.T = T; a.H = H; a.ld4 = ld4;
+    const int KG = AT_THREADS / at_cqt(ld4);
+    const size_t smem = ((size_t)H * AT_BT + (size_t)((AT_BT * H + 3) & ~3) + 2 * (size_t)KG * AT_BT * ld4) * sizeof(float);
+    if (smem > 227 * 1024) return CAPHN_EINVAL;
+    CAPHN_CHECK(cudaFuncSetAttribute(lstm_seq_fwd_grouped_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    lstm_seq_fwd_grouped_kernel<<<ntiles, AT_THREADS, smem, (cudaStream_t)stream>>>(a, (const int4*)tiles, bstride);
+    CAPHN_RETURN_LAST();
+}
+
+// BPTT of caphn_lstm_seq_fwd_grouped: the group's W_hh from the pack Whh [G][4H][ldh]; dG [T,B,4H], dh0 [B,H].
+int caphn_lstm_seq_bwd_grouped(const float* dHbm, const float* saved, const float* Whh, int ldh, float* dG, float* dh0,
+                               int B, int T, int H, const int* tiles, int ntiles, void* stream) {
+    if (B <= 0 || T <= 0 || H <= 0 || (ldh & 3) || ldh < H || ((uintptr_t)Whh & 15)) return CAPHN_EINVAL;
+    if (!tiles || ntiles < 1 || ((uintptr_t)tiles & 15)) return CAPHN_EINVAL;
+    LstmBwdArgs a{};
+    a.dHbm = dHbm; a.saved = saved; a.Whh = Whh; a.dG = dG; a.dh0 = dh0; a.NL = 1; a.B = B; a.T = T; a.H = H; a.ldh = ldh;
+    const int KGh = AT_THREADS / at_cqt(ldh);
+    const size_t smem = ((size_t)4 * H * AT_BT + 2 * (size_t)((AT_BT * H + 3) & ~3) + 2 * (size_t)KGh * AT_BT * ldh) *
+                        sizeof(float);
+    if (smem > 227 * 1024) return CAPHN_EINVAL;
+    CAPHN_CHECK(cudaFuncSetAttribute(lstm_seq_bwd_grouped_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    lstm_seq_bwd_grouped_kernel<<<ntiles, AT_THREADS, smem, (cudaStream_t)stream>>>(a, (const int4*)tiles);
     CAPHN_RETURN_LAST();
 }
 

@@ -86,6 +86,7 @@ class GroupPlan:
         self.tiles_fwd = i32(self._tiles(self.tile_rows_fwd))
         self.tiles_bwd = i32(self._tiles(self.tile_rows_bwd))
         self.tiles8 = i32(self._tiles(8))                           # 8-row tiles: the weights-resident cluster GRU (pooled variant)
+        self.tiles4 = i32(self._tiles(4))                           # 4-row tiles: the streaming LSTM recurrence (pooled variant)
         absent = [g for g in range(G) if cnt[g] == 0]
         self.absent_dev = i64(absent) if absent else None         # groups without rows: their d(theta) rows are zero
         self._units: Dict[Tuple, torch.Tensor] = {}
@@ -316,65 +317,77 @@ class AttentionGruGroupedLossFn(Function):
 
 
 # ----------------------------------------------------------------------------------------------------------------------
-# pooled variant (hypernet.HyperNet + DecoderGRU, single layer): grouped x-projection + weights-resident cluster GRU whose
-# clusters each keep THEIR group's W_hh in shared memory for all T steps
+# pooled variant (hypernet.HyperNet + DecoderGRU / DecoderRNN, single layer): grouped x-projection, then either the
+# weights-resident cluster GRU whose clusters each keep THEIR group's W_hh in shared memory for all T steps, or the
+# streaming LSTM recurrence whose CTAs each run a <= 4-row tile of one group against that group's slice of a W_hh pack
 # ----------------------------------------------------------------------------------------------------------------------
-def _layout_pooled(E, H):
-    """Offsets of (W_ih [3H, E], W_hh [3H, H], b_ih, b_hh) inside one row of Theta (hypernet.py:62-68 parameter order)."""
-    H3 = 3 * H
-    o_hh = H3 * E
-    o_bi = o_hh + H3 * H
-    o_bh = o_bi + H3
-    return H3, o_hh, o_bi, o_bh, o_bh + H3
+def _layout_pooled(E, H, gates=3):
+    """Offsets of (W_ih [gH, E], W_hh [gH, H], b_ih, b_hh) inside one row of Theta (hypernet.py:62-68 parameter order);
+    g = 3 gates for the GRU cell, 4 for the LSTM cell."""
+    NG = gates * H
+    o_hh = NG * E
+    o_bi = o_hh + NG * H
+    o_bh = o_bi + NG
+    return NG, o_hh, o_bi, o_bh, o_bh + NG
 
 
-def _pooled_grouped_forward(plan: GroupPlan, feats, caps, h0, Theta, emb_w, fc_w, fc_b):
-    """Teacher-forced DecoderGRU.forward (later.py:389-457, num_layers = 1) for a batch SORTED by style group.  Returns logits
-    in the ORIGINAL batch order."""
+def _pooled_grouped_forward(plan: GroupPlan, lstm, feats, caps, h0, Theta, emb_w, fc_w, fc_b):
+    """Teacher-forced DecoderGRU.forward (later.py:389-457) or, with ``lstm``, DecoderRNN.forward (later.py:254-324), one
+    layer, for a batch SORTED by style group.  Returns logits in the ORIGINAL batch order."""
     B, T = caps.shape
     E, H, V = emb_w.shape[1], fc_w.shape[1], fc_w.shape[0]
     G, theta = Theta.shape
-    H3, o_hh, o_bi, o_bh, total = _layout_pooled(E, H)
+    NG, o_hh, o_bi, o_bh, total = _layout_pooled(E, H, 4 if lstm else 3)
     assert theta == total and plan.B == B and plan.T == T and plan.G == G
     dev = feats.device
     Theta = Theta.contiguous()
     emb_w = emb_w.contiguous()
     X = ops.build_inputs(feats.contiguous(), emb_w, caps, 0)                # [T*B, E] time-major: x_0 = feature, x_t = Emb[caps[:, t-1]]
     b_ih_g = Theta[:, o_bi:o_bh].contiguous()
-    Wsp = ops.split_bf16_batched(Theta, theta, E, G, H3, E)                  # W_ih of every group: [G*3H, Kp]
+    Wsp = ops.split_bf16_batched(Theta, theta, E, G, NG, E)                  # W_ih of every group: [G*gH, Kp]
     Xgm = ops.split_bf16_gather(X, plan.gm2tm, plan.R_gm)
-    GI = torch.empty(T * B, H3, device=dev, dtype=torch.float32)
-    ops.gemm_tc_grouped(Xgm, False, Wsp, False, GI, H3, plan.units_xproj(H3, E, 128), 128, bias=b_ih_g, rowmap=plan.gm2tm)
-    Hall = torch.empty(T + 1, B, H, device=dev, dtype=torch.float32)
-    Hall[0].copy_(h0)
-    Hbm = torch.empty(B, T, H, device=dev, dtype=torch.float32)
-    saved = torch.empty(1, 4, T, B, H, device=dev, dtype=torch.float32)
-    ops._cabi.call("caphn_gru_cluster_fwd_grouped", GI.data_ptr(), Theta.data_ptr() + 4 * o_hh, Theta.data_ptr() + 4 * o_bh,
-                   Hall.data_ptr(), Hbm.data_ptr(), saved.data_ptr(), B, T, H, plan.tiles8.data_ptr(), plan.tiles8.shape[0],
-                   theta, theta, ops._stream())
+    GI = torch.empty(T * B, NG, device=dev, dtype=torch.float32)
+    ops.gemm_tc_grouped(Xgm, False, Wsp, False, GI, NG, plan.units_xproj(NG, E, 128), 128, bias=b_ih_g, rowmap=plan.gm2tm)
+    if lstm:
+        WhhT = ops.transpose_pad_batched(Theta[:, o_hh:o_bi], NG, H, ops.round4(NG))     # [G, H, ld4]
+        Hall, Hbm, saved = ops.lstm_seq_fwd_grouped(GI, WhhT, Theta[:, o_bh:], h0, T, plan.tiles4)
+    else:
+        Hall = torch.empty(T + 1, B, H, device=dev, dtype=torch.float32)
+        Hall[0].copy_(h0)
+        Hbm = torch.empty(B, T, H, device=dev, dtype=torch.float32)
+        saved = torch.empty(1, 4, T, B, H, device=dev, dtype=torch.float32)
+        ops._cabi.call("caphn_gru_cluster_fwd_grouped", GI.data_ptr(), Theta.data_ptr() + 4 * o_hh,
+                       Theta.data_ptr() + 4 * o_bh, Hall.data_ptr(), Hbm.data_ptr(), saved.data_ptr(), B, T, H,
+                       plan.tiles8.data_ptr(), plan.tiles8.shape[0], theta, theta, ops._stream())
     Hbm_o = ops.gather_rows(Hbm.view(B, T * H), plan.inv).view(B, T, H)
     logits = ops.linear(Hbm_o.view(B * T, H), fc_w.contiguous(), fc_b).view(B, T, V)
     sv = (caps, X, Hall, Hbm_o, saved, emb_w, Theta, fc_w, Wsp.hi, Wsp.lo)
     return logits, sv, (B, T, E, H, V, G)
 
 
-def _pooled_grouped_backward(plan: GroupPlan, sv, dims, vocab, need_feats):
+def _pooled_grouped_backward(plan: GroupPlan, lstm, sv, dims, vocab, need_feats):
     caps, X, Hall, Hbm_o, saved, emb_w, Theta, fc_w, Wsp_hi, Wsp_lo = sv
     B, T, E, H, V, G = dims
-    H3, o_hh, o_bi, o_bh, theta = _layout_pooled(E, H)
+    NG, o_hh, o_bi, o_bh, theta = _layout_pooled(E, H, 4 if lstm else 3)
     dfc_w, dfc_b, dHbm_o = vocab
     dev = X.device
     dHbm = ops.gather_rows(dHbm_o.reshape(B, T * H).contiguous(), plan.order).view(B, T, H)
-    dGI = torch.empty(T * B, H3, device=dev, dtype=torch.float32)
-    dGH = torch.empty(T * B, H3, device=dev, dtype=torch.float32)
-    dh0 = torch.empty(B, H, device=dev, dtype=torch.float32)
-    ops._cabi.call("caphn_gru_cluster_bwd_grouped", dHbm.data_ptr(), saved.data_ptr(), Hall.data_ptr(),
-                   Theta.data_ptr() + 4 * o_hh, dGI.data_ptr(), dGH.data_ptr(), dh0.data_ptr(), B, T, H,
-                   plan.tiles8.data_ptr(), plan.tiles8.shape[0], theta, ops._stream())
+    if lstm:
+        # the LSTM pre-activation is the plain sum gi + gh: one gate gradient dG serves both weight products and both biases
+        Whh_p = ops.copy_pad_batched(Theta[:, o_hh:o_bi], NG, H, ops.round4(H))          # [G, 4H, ldh]
+        dGI, dh0 = ops.lstm_seq_bwd_grouped(dHbm, saved, Hall, Whh_p, plan.tiles4)
+        dGH = dGI
+    else:
+        dGI = torch.empty(T * B, NG, device=dev, dtype=torch.float32)
+        dGH = torch.empty(T * B, NG, device=dev, dtype=torch.float32)
+        dh0 = torch.empty(B, H, device=dev, dtype=torch.float32)
+        ops._cabi.call("caphn_gru_cluster_bwd_grouped", dHbm.data_ptr(), saved.data_ptr(), Hall.data_ptr(),
+                       Theta.data_ptr() + 4 * o_hh, dGI.data_ptr(), dGH.data_ptr(), dh0.data_ptr(), B, T, H,
+                       plan.tiles8.data_ptr(), plan.tiles8.shape[0], theta, ops._stream())
     Hprev = Hall[:-1].reshape(T * B, H)
     R = plan.R_gm
     dGI_gm = ops.split_bf16_gather(dGI, plan.gm2tm, R)
-    dGH_gm = ops.split_bf16_gather(dGH, plan.gm2tm, R)
+    dGH_gm = dGI_gm if dGH is dGI else ops.split_bf16_gather(dGH, plan.gm2tm, R)
     X_gm = ops.split_bf16_gather(X, plan.gm2tm, R)
     Hp_gm = ops.split_bf16_gather(Hprev, plan.gm2tm, R)
     dTheta = torch.empty(G, theta, device=dev, dtype=torch.float32)
@@ -382,13 +395,13 @@ def _pooled_grouped_backward(plan: GroupPlan, sv, dims, vocab, need_feats):
     if plan.absent_dev is not None:
         dTheta.index_fill_(0, plan.absent_dev, 0.0)
     mn = lambda op: ops.SplitOperand(op.hi, op.lo, op.K, op.rows, op.ld, True)
-    ops.gemm_tc_grouped(mn(dGI_gm), True, mn(X_gm), True, dTheta, E, plan.units_dw(H3, E, 128, theta, 0, E), 128)
-    ops.gemm_tc_grouped(mn(dGH_gm), True, mn(Hp_gm), True, dTheta, H, plan.units_dw(H3, H, 128, theta, o_hh, H), 128)
+    ops.gemm_tc_grouped(mn(dGI_gm), True, mn(X_gm), True, dTheta, E, plan.units_dw(NG, E, 128, theta, 0, E), 128)
+    ops.gemm_tc_grouped(mn(dGH_gm), True, mn(Hp_gm), True, dTheta, H, plan.units_dw(NG, H, 128, theta, o_hh, H), 128)
     ops.group_colsum(dGI, plan.goff_dev, G, B, T, dTheta[:, o_bi:o_bh])
     ops.group_colsum(dGH, plan.goff_dev, G, B, T, dTheta[:, o_bh:])
-    Wsp = ops.SplitOperand(Wsp_hi, Wsp_lo, E, G * H3, Wsp_hi.shape[1], True)
+    Wsp = ops.SplitOperand(Wsp_hi, Wsp_lo, E, G * NG, Wsp_hi.shape[1], True)
     dX = torch.empty(T * B, E, device=dev, dtype=torch.float32)
-    ops.gemm_tc_grouped(dGI_gm, False, Wsp, True, dX, E, plan.units_dx(H3, E, 128), 128, rowmap=plan.gm2tm)
+    ops.gemm_tc_grouped(dGI_gm, False, Wsp, True, dX, E, plan.units_dx(NG, E, 128), 128, rowmap=plan.gm2tm)
     dfeats = dX[:B].clone() if need_feats else None                       # rows of t = 0 (sorted order)
     demb = torch.zeros_like(emb_w)
     ops.embed_scatter_add(dX, caps, demb, 1)
@@ -401,10 +414,7 @@ class DecoderGRUGroupedFn(Function):
 
     @staticmethod
     def forward(ctx, plan, feats, caps, h0, Theta, emb_w, fc_w, fc_b):
-        logits, sv, dims = _pooled_grouped_forward(plan, feats, caps, h0, Theta, emb_w, fc_w, fc_b)
-        ctx.save_for_backward(*sv)
-        ctx.plan, ctx.dims = plan, dims
-        return logits
+        return _pooled_fn_forward(ctx, False, plan, feats, caps, h0, Theta, emb_w, fc_w, fc_b)
 
     @staticmethod
     def backward(ctx, dlogits):
@@ -412,9 +422,67 @@ class DecoderGRUGroupedFn(Function):
         B, T, E, H, V, G = ctx.dims
         dl = dlogits.reshape(B * T, V).contiguous()
         vocab = Fn.vocab_bwd_from_dlogits(dl, sv[3].view(B * T, H), sv[7])
-        dfeats, dh0, dTheta, demb, dfc_w, dfc_b = _pooled_grouped_backward(ctx.plan, sv, ctx.dims, vocab,
+        dfeats, dh0, dTheta, demb, dfc_w, dfc_b = _pooled_grouped_backward(ctx.plan, ctx.lstm, sv, ctx.dims, vocab,
                                                                          ctx.needs_input_grad[1])
         return None, dfeats, None, dh0 if ctx.needs_input_grad[3] else None, dTheta, demb, dfc_w, dfc_b
+
+
+class DecoderRNNGroupedFn(DecoderGRUGroupedFn):
+    """DecoderGRUGroupedFn for the LSTM captioner (DecoderRNN, single layer): same inputs and outputs."""
+
+    @staticmethod
+    def forward(ctx, plan, feats, caps, h0, Theta, emb_w, fc_w, fc_b):
+        return _pooled_fn_forward(ctx, True, plan, feats, caps, h0, Theta, emb_w, fc_w, fc_b)
+
+
+def _pooled_fn_forward(ctx, lstm, plan, *args):
+    logits, sv, dims = _pooled_grouped_forward(plan, lstm, *args)
+    ctx.save_for_backward(*sv)
+    ctx.plan, ctx.dims, ctx.lstm = plan, dims, lstm
+    return logits
+
+
+class DecoderGRUGroupedLossFn(Function):
+    """DecoderGRUGroupedFn + mean cross-entropy (hypernet.py:139-145 for a many-style batch; ``ignore_index`` None = no
+    masking) as one node: returns (loss, logits).  The captions of the loss are in the ORIGINAL order (``caps_o``); the
+    one-pass CE kernel writes the softmax gradient as tensor-core operands, so fp32 dlogits never exist."""
+
+    @staticmethod
+    def forward(ctx, ignore_index, plan, caps_o, feats, caps, h0, Theta, emb_w, fc_w, fc_b):
+        return _pooled_loss_forward(ctx, False, ignore_index, plan, caps_o, feats, caps, h0, Theta, emb_w, fc_w, fc_b)
+
+    @staticmethod
+    def backward(ctx, g, _dl):
+        allsv = ctx.saved_tensors
+        sv, (logits, targets, lse, lossbuf, dhi, dlo) = allsv[:-6], allsv[-6:]
+        B, T, E, H, V, G = ctx.dims
+        g = g.reshape(1).to(torch.float32).contiguous()
+        vocab = Fn.vocab_bwd_fused(logits.view(B * T, V), targets, ctx.ignore_index, lse, lossbuf, g,
+                                   sv[3].view(B * T, H), sv[7], dhi, dlo)
+        dfeats, dh0, dTheta, demb, dfc_w, dfc_b = _pooled_grouped_backward(ctx.plan, ctx.lstm, sv, ctx.dims, vocab,
+                                                                         ctx.needs_input_grad[3])
+        return (None, None, None, dfeats, None, dh0 if ctx.needs_input_grad[5] else None, dTheta, demb, dfc_w, dfc_b)
+
+
+class DecoderRNNGroupedLossFn(DecoderGRUGroupedLossFn):
+    """DecoderGRUGroupedLossFn for the LSTM captioner (DecoderRNN, single layer): same inputs and outputs."""
+
+    @staticmethod
+    def forward(ctx, ignore_index, plan, caps_o, feats, caps, h0, Theta, emb_w, fc_w, fc_b):
+        return _pooled_loss_forward(ctx, True, ignore_index, plan, caps_o, feats, caps, h0, Theta, emb_w, fc_w, fc_b)
+
+
+def _pooled_loss_forward(ctx, lstm, ignore_index, plan, caps_o, *args):
+    logits, sv, dims = _pooled_grouped_forward(plan, lstm, *args)
+    B, T, V = logits.shape
+    targets = caps_o.reshape(-1).contiguous()
+    lossbuf, lse, dhi, dlo = Fn.ce_fwd_for_loss(logits.view(B * T, V), targets, ignore_index, dims[3],
+                                                any(ctx.needs_input_grad))
+    ctx.save_for_backward(*sv, logits, targets, lse, lossbuf, dhi, dlo)
+    ctx.plan, ctx.dims, ctx.lstm, ctx.ignore_index = plan, dims, lstm, ignore_index
+    ctx.mark_non_differentiable(logits)
+    ctx.set_materialize_grads(False)
+    return lossbuf[0].clone(), logits
 
 
 # ----------------------------------------------------------------------------------------------------------------------

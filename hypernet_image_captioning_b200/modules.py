@@ -300,13 +300,13 @@ class DecoderGRU(nn.Module):
                 h0 = self._h0(features)
             if self._grouped_kernels_ok(features):
                 # many-style batch on the grouped kernels (grouped.py): batch sorted by group, one grouped tensor-core launch
-                # per time-batched product, clusters that keep THEIR group's W_hh in shared memory for all T steps
+                # per time-batched product, a recurrence that runs every row tile with THEIR group's W_hh
                 from . import grouped as Gp
                 Theta = self._theta_groups
                 plan = Gp.GroupPlan.get(groups, Theta.shape[0], captions.shape[1], features.device)
                 fs = Gp.RowPermuteFn.apply(features, plan.order, plan.inv)
                 hs = Gp.RowPermuteFn.apply(h0, plan.order, plan.inv)
-                return Gp.DecoderGRUGroupedFn.apply(plan, fs, captions.index_select(0, plan.order), hs, Theta,
+                return self._grouped_fns()[0].apply(plan, fs, captions.index_select(0, plan.order), hs, Theta,
                                                     self.embed.weight, self.fc_out.weight, self.fc_out.bias)
             return _run_grouped(lambda g, f, c, h: self._forward_one(f, c, h, self._cells(g)), groups,
                                 [features, captions, h0], len(self._generated_groups))[0]
@@ -316,13 +316,46 @@ class DecoderGRU(nn.Module):
 
     def _grouped_kernels_ok(self, features):
         """Grouped kernels: single-layer GRU captioner whose W_hh fits the weights-resident cluster kernel, fp32 mode."""
-        return (type(self) is DecoderGRU and self.num_layers == 1 and getattr(self, "_theta_groups", None) is not None
-                and features.is_cuda and ops.gru_cluster_size(self.hidden_size) > 0 and ops.TC_SPLIT)
+        return (self.num_layers == 1 and getattr(self, "_theta_groups", None) is not None and features.is_cuda
+                and ops.TC_SPLIT and ops.gru_cluster_size(self.hidden_size) > 0)
 
-    def forward_loss(self, features, captions, h0=None, ignore_index=None):
+    def _grouped_fns(self):
+        """(forward node, forward + loss node) of the grouped kernels for this cell type."""
+        from . import grouped as Gp
+        return Gp.DecoderGRUGroupedFn, Gp.DecoderGRUGroupedLossFn
+
+    def _forward_loss_grouped(self, features, captions, h0, ignore_index, groups):
+        """forward_loss for a many-style batch: one autograd node (grouped.py) whose loss and logits are the numbers of
+        ``cross_entropy(self(features, captions, h0=h0, groups=groups), captions, ignore_index)``."""
+        fallback = "use forward(..., groups=...) + cross_entropy instead"
+        if self.num_layers > 1:
+            raise NotImplementedError(f"forward_loss(groups=...) covers single-layer captioners; {fallback}")
+        Theta = getattr(self, "_theta_groups", None)
+        if Theta is None:
+            raise ValueError("forward_loss(groups=...) needs the weights of every group: call the hypernet's "
+                             "forward_grouped(X) after its last forward(x)")
+        from . import grouped as Gp
+        plan = Gp.GroupPlan.get(groups, Theta.shape[0], captions.shape[1], features.device)     # checks the group ids
+        if not self._grouped_kernels_ok(features):
+            raise NotImplementedError("forward_loss(groups=...) runs on the grouped CUDA kernels: CUDA tensors, fp32 "
+                                      f"precision and a hidden size their recurrence covers; {fallback}")
+        if h0 is None:
+            h0 = self._h0(features)
+        streams.wait_pending()
+        fs = Gp.RowPermuteFn.apply(features, plan.order, plan.inv)
+        hs = Gp.RowPermuteFn.apply(h0, plan.order, plan.inv)
+        return self._grouped_fns()[1].apply(ignore_index, plan, captions.contiguous(), fs,
+                                            captions.index_select(0, plan.order), hs, Theta, self.embed.weight,
+                                            self.fc_out.weight, self.fc_out.bias)
+
+    def forward_loss(self, features, captions, h0=None, ignore_index=None, groups=None):
         """Teacher-forced forward fused with the mean cross-entropy of hypernet.py:145 (``ignore_index=None``: no
         masking): returns ``(loss, logits)``.  Same numbers as ``cross_entropy(self(features, captions), captions)``
-        but one autograd node whose backward writes the softmax gradient straight into tensor-core operands."""
+        but one autograd node whose backward writes the softmax gradient straight into tensor-core operands.
+        ``groups`` ([B] group id per row, after the hypernet's ``forward_grouped``): many-style batch, single layer, fp32
+        mode, CUDA tensors; elsewhere ``NotImplementedError`` (use ``forward(..., groups=...)`` + ``cross_entropy``)."""
+        if groups is not None:
+            return self._forward_loss_grouped(features, captions, h0, ignore_index, groups)
         if h0 is None:
             h0 = self._h0(features)
         # (no wait_pending here: the fused node waits for the generated weights slice by slice, Fn._gru_decoder_forward)
@@ -506,7 +539,18 @@ class DecoderRNN(DecoderGRU):
         raise NotImplementedError("beam search is implemented for the GRU captioner (DecoderGRU) only: the LSTM cell state "
                                   "would have to follow the beams, and there is no LSTM decode-step kernel")
 
-    def forward_loss(self, features, captions, h0=None, ignore_index=None):
+    def _grouped_kernels_ok(self, features):
+        """Grouped kernels: single-layer LSTM captioner whose recurrence fits one CTA's shared memory, fp32 mode."""
+        return (self.num_layers == 1 and getattr(self, "_theta_groups", None) is not None and features.is_cuda
+                and ops.TC_SPLIT and ops.lstm_seq_fits(self.hidden_size))
+
+    def _grouped_fns(self):
+        from . import grouped as Gp
+        return Gp.DecoderRNNGroupedFn, Gp.DecoderRNNGroupedLossFn
+
+    def forward_loss(self, features, captions, h0=None, ignore_index=None, groups=None):
+        if groups is not None:
+            return self._forward_loss_grouped(features, captions, h0, ignore_index, groups)
         if h0 is None:
             h0 = self._h0(features)
         streams.wait_pending()

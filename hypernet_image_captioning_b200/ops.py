@@ -196,6 +196,29 @@ def copy_pad(src, ldd):
     return dst
 
 
+def transpose_pad_batched(src, R, C, ldd):
+    """src [nb, R*C]: row z holds a matrix [R, C] (e.g. the W_hh block of every row of Theta, a column slice).  Returns
+    dst [nb, C, ldd] with dst[z, c, r] = src_z[r, c], zero padded; one launch for all nb."""
+    _chk(src)
+    nb = src.shape[0]
+    assert src.dim() == 2 and src.stride(1) == 1 and src.shape[1] == R * C
+    dst = torch.empty(nb, C, ldd, device=src.device, dtype=torch.float32)
+    _cabi.call("caphn_transpose_pad_batched", src.data_ptr(), src.stride(0), C, dst.data_ptr(), C * ldd, ldd, nb, R, C,
+               _stream())
+    return dst
+
+
+def copy_pad_batched(src, R, C, ldd):
+    """src [nb, R*C] as in transpose_pad_batched -> dst [nb, R, ldd] with dst[z, r, c] = src_z[r, c], zero padded."""
+    _chk(src)
+    nb = src.shape[0]
+    assert src.dim() == 2 and src.stride(1) == 1 and src.shape[1] == R * C
+    dst = torch.empty(nb, R, ldd, device=src.device, dtype=torch.float32)
+    _cabi.call("caphn_copy_pad_batched", src.data_ptr(), src.stride(0), C, dst.data_ptr(), R * ldd, ldd, nb, R, C,
+               _stream())
+    return dst
+
+
 def round4(n):
     return (n + 3) // 4 * 4
 
@@ -258,6 +281,54 @@ def lstm_seq_bwd(dHbm, saved, Hall, Whh_p, extra=()):
     arr = _ptr_array([t for cell in extra for t in cell])
     _cabi.call("caphn_lstm_seq_bwd", dHbm.data_ptr(), saved.data_ptr(), Whh_p.data_ptr(), Whh_p.stride(0),
                arr if NL > 1 else None, dG.data_ptr(), dh0.data_ptr(), NL, B, T, H, _stream())
+    return dG, dh0
+
+
+def _at_cqt(ld):
+    return min(512, max(32, 1 << max(0, (ld // 4 - 1).bit_length())))
+
+
+def lstm_seq_fits(H):
+    """Whether the single-layer LSTM recurrence (forward and BPTT) fits the 227 KB of shared memory of one CTA at hidden
+    size H: the same sizes the entry points of csrc/lstm_seq.cu check."""
+    ld4, ldh = round4(4 * H), round4(H)
+    fwd = H * 4 + round4(4 * H) + 2 * (512 // _at_cqt(ld4)) * 4 * ld4
+    bwd = 16 * H + 2 * round4(4 * H) + 2 * (512 // _at_cqt(ldh)) * 4 * ldh
+    return 4 * max(fwd, bwd) <= 227 * 1024
+
+
+def lstm_seq_fwd_grouped(GI, WhhT, bhh, h0, T, tiles, want_c=False):
+    """Single-layer LSTM recurrence of a batch sorted by style group.  GI [T*B, 4H]; WhhT [G, H, ld4] (one W_hh^T per
+    group); bhh [G, 4H] (row stride free, e.g. a column slice of Theta); tiles int32 [n, 4] = (first row, rows <= 4,
+    group, 0).  Returns Hall [T+1,B,H], Hbm [B,T,H], saved [6,T,B,H] (+ cT [B,H] with ``want_c``)."""
+    B, H = h0.shape
+    dev = GI.device
+    _chk(GI), _chk(WhhT), _chk(bhh), _chk(tiles, torch.int32)
+    assert WhhT.is_contiguous() and WhhT.shape[1] == H and bhh.stride(1) == 1 and tiles.is_contiguous()
+    Hall = torch.empty(T + 1, B, H, device=dev, dtype=torch.float32)
+    Hall[0].copy_(h0)
+    Hbm = torch.empty(B, T, H, device=dev, dtype=torch.float32)
+    saved = torch.empty(6, T, B, H, device=dev, dtype=torch.float32)
+    cT = torch.empty(B, H, device=dev, dtype=torch.float32) if want_c else None
+    _cabi.call("caphn_lstm_seq_fwd_grouped", GI.data_ptr(), WhhT.data_ptr(), WhhT.shape[2], bhh.data_ptr(), bhh.stride(0),
+               Hall.data_ptr(), Hbm.data_ptr(), saved.data_ptr(), _p(cT), B, T, H, tiles.data_ptr(), tiles.shape[0],
+               _stream())
+    if want_c:
+        return Hall, Hbm, saved, cT
+    return Hall, Hbm, saved
+
+
+def lstm_seq_bwd_grouped(dHbm, saved, Hall, Whh_p, tiles):
+    """BPTT of lstm_seq_fwd_grouped; Whh_p [G, 4H, ldh] (one padded W_hh per group).  Returns dG [T*B, 4H], dh0 [B, H]."""
+    Tp1, B, H = Hall.shape
+    T = Tp1 - 1
+    dev = Hall.device
+    _chk(dHbm), _chk(saved), _chk(Whh_p), _chk(tiles, torch.int32)
+    assert dHbm.is_contiguous() and saved.is_contiguous() and Whh_p.is_contiguous() and tiles.is_contiguous()
+    dG = torch.empty(T * B, 4 * H, device=dev, dtype=torch.float32)
+    dh0 = torch.empty(B, H, device=dev, dtype=torch.float32)
+    _cabi.call("caphn_lstm_seq_bwd_grouped", dHbm.data_ptr(), saved.data_ptr(), Whh_p.data_ptr(), Whh_p.shape[2],
+               dG.data_ptr(), dh0.data_ptr(), B, T, H, tiles.data_ptr(), tiles.shape[0], _stream())
     return dG, dh0
 
 

@@ -71,6 +71,12 @@ int caphn_gemm_tc_ex(const void* Ahi, const void* Alo, long a_ld, int a_mn, cons
  * weights out with 16-byte rows for the recurrence kernels. */
 int caphn_transpose_pad(const float* src, long lds, float* dst, long ldd, int R, int C, void* stream);
 int caphn_copy_pad(const float* src, long lds, float* dst, long ldd, long R, int C, void* stream);
+/* The same for nb matrices in one launch: matrix z is read at src + z*sstride and written at dst + z*dstride (floats) --
+ * e.g. the per-group W_hh packs of a many-style batch, read straight out of Theta [G, theta] (sstride = theta). */
+int caphn_transpose_pad_batched(const float* src, long sstride, long lds, float* dst, long dstride, long ldd, int nb,
+                                int R, int C, void* stream);
+int caphn_copy_pad_batched(const float* src, long sstride, long lds, float* dst, long dstride, long ldd, int nb, long R,
+                           int C, void* stream);
 
 /* ---- pooled-feature decoder recurrence (later.py:389-490 DecoderGRU; torch GRUCell gates r,z,n) -------------------- */
 
@@ -128,6 +134,16 @@ int caphn_lstm_seq_fwd(const float* GI, const float* WhhT, int ld4, const float*
                        int T, int H, void* stream);
 int caphn_lstm_seq_bwd(const float* dHbm, const float* saved, const float* Whh, int ldh, const void* const* extra,
                        float* dG, float* dh0, int NL, int B, int T, int H, void* stream);
+/* Single-layer LSTM recurrence of a many-style batch (pooled DecoderRNN with per-row style groups): rows sorted by group,
+ * CTA i runs tiles[i] = {first row, rows 1..4, group, 0} (int32, 16-byte aligned; a tile never straddles two groups) with
+ * that group's weights: forward WhhT pack [G][H][ld4] and b_hh at bhh + group*bstride, backward Whh pack [G][4H][ldh].
+ * h0 = Hall[0], c0 = zeros; saved [6][T,B,H], dG [T,B,4H], cT / dh0 [B,H] as in the single-style calls.  Each row
+ * computes exactly what caphn_lstm_seq_fwd / _bwd compute for it. */
+int caphn_lstm_seq_fwd_grouped(const float* GI, const float* WhhT, int ld4, const float* bhh, long bstride, float* Hall,
+                               float* Hbm, float* saved, float* cT, int B, int T, int H, const int* tiles, int ntiles,
+                               void* stream);
+int caphn_lstm_seq_bwd_grouped(const float* dHbm, const float* saved, const float* Whh, int ldh, float* dG, float* dh0,
+                               int B, int T, int H, const int* tiles, int ntiles, void* stream);
 /* Step-split forward (default for H, F <= 208): three batch-wide launches per time step instead of one persistent
  * kernel, chained with programmatic dependent launch -- U: u = U_a h + b_u on the warp tensor cores (bf16 hi/lo split,
  * fp32 accumulate); A: one CTA per batch row, K_b / f_b fetched into shared memory by bulk TMA copies, scores, softmax,
