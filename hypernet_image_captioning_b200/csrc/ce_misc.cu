@@ -37,6 +37,11 @@ __device__ __forceinline__ float block_reduce_max(float v, float* sh) {
     return sh[0];
 }
 
+// Target contract of every kernel below (DESIGN.md §6): a row whose target equals the ignore index is ignored (loss 0, not
+// counted, zero gradient); any other target outside [0, V) still counts as a row, its loss is NaN (so the mean is NaN and
+// the error shows without a host sync) and its gradient row is zero.  x[t] is read only for t in [0, V).
+__device__ __forceinline__ bool ce_in_range(long long t, int V) { return (unsigned long long)t < (unsigned long long)V; }
+
 // One CTA per row: lse[m], row_loss[m] = valid ? lse - x[target] : 0, row_valid[m].
 __global__ void __launch_bounds__(CE_THREADS) ce_fwd_kernel(const float* __restrict__ X, long ld,
                                                             const long long* __restrict__ tgt, int V, int has_ignore,
@@ -72,7 +77,7 @@ __global__ void __launch_bounds__(CE_THREADS) ce_fwd_kernel(const float* __restr
         const long long t = tgt[m];
         const bool valid = !(has_ignore && t == ignore);
         row_valid[m] = valid ? 1.f : 0.f;
-        row_loss[m] = valid ? (l - x[t]) : 0.f;
+        row_loss[m] = valid ? (ce_in_range(t, V) ? l - x[t] : __int_as_float(0x7fc00000)) : 0.f;
     }
 }
 
@@ -99,7 +104,7 @@ __global__ void __launch_bounds__(CE_THREADS) ce_bwd_kernel(const float* __restr
     const float* x = X + m * ld;
     float* dx = dX + m * lddx;
     const long long t = tgt[m];
-    const bool valid = !(has_ignore && t == ignore);
+    const bool valid = !(has_ignore && t == ignore) && ce_in_range(t, V);     // a zero row for an out-of-range target
     const float sc = valid ? gscale[0] / fmaxf(lossbuf[1], 1.f) : 0.f;
     const float l = lse[m];
     const bool vec = ((ld & 3) == 0) && ((lddx & 3) == 0) && ((V & 3) == 0) && (((uintptr_t)X & 15) == 0) &&
@@ -128,7 +133,8 @@ __global__ void __launch_bounds__(CE_THREADS) ce_bwd_kernel(const float* __restr
 //   hiT/loT [V, Mp] bf16 split of d^T      (operand of dW  = d^T . H,     K = M)
 //   dbias[v] += sum_m d[m,v]
 // One CTA per 64 x 64 tile: coalesced row-major writes, shared-memory transpose for the [V, Mp] copy.
-__global__ void __launch_bounds__(256) ce_bwd_split_kernel(
+// (256, 8): 32 registers, 8 CTAs per SM -- without the bound ptxas takes 36 once the m-tiles are on blockIdx.x
+__global__ void __launch_bounds__(256, 8) ce_bwd_split_kernel(
     const float* __restrict__ X, long ld, const long long* __restrict__ tgt, int M, int V, int has_ignore,
     long long ignore, const float* __restrict__ lse, const float* __restrict__ gscale,
     const float* __restrict__ lossbuf, __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo, long Vp,
@@ -136,7 +142,7 @@ __global__ void __launch_bounds__(256) ce_bwd_split_kernel(
     __shared__ float tile[64][65];
     __shared__ float csum[16][64];
     const int tid = threadIdx.x;
-    const int m0 = blockIdx.y * 64, v0 = blockIdx.x * 64;
+    const int m0 = blockIdx.x * 64, v0 = blockIdx.y * 64;      // m-tiles on x: up to 2^24 of them
     const float sc0 = gscale[0] / fmaxf(lossbuf[1], 1.f);
     const int c4 = (tid & 15) * 4;
     const bool vecx = ((ld & 3) == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0) && (v0 + c4 + 3 < V);
@@ -148,7 +154,7 @@ __global__ void __launch_bounds__(256) ce_bwd_split_kernel(
         float d[4] = {0.f, 0.f, 0.f, 0.f};
         if (m < M) {
             const long long t = tgt[m];
-            const bool valid = !(has_ignore && t == ignore);
+            const bool valid = !(has_ignore && t == ignore) && ce_in_range(t, V);
             if (valid) {
                 const float l = lse[m];
                 const float* xp = X + (long)m * ld + v0 + c4;
@@ -292,16 +298,17 @@ __global__ void __launch_bounds__(CE_THREADS) ce_fwd_split_kernel(const float* _
     s = block_reduce_sum(s, sh);          // its barriers also publish the exponentials to the whole CTA
     const long long t = tgt[m];
     const bool valid = !(has_ignore && t == ignore);
+    const bool live = valid && ce_in_range(t, V);       // counted, but an out-of-range target gets NaN and a zero row
     if (threadIdx.x == 0) {
         const float l = mx + logf(s);
         lse[m] = l;
         row_valid[m] = valid ? 1.f : 0.f;
-        row_loss[m] = valid ? (l - x[t]) : 0.f;
+        row_loss[m] = valid ? (live ? l - x[t] : __int_as_float(0x7fc00000)) : 0.f;
     }
-    const float inv = valid ? 1.f / s : 0.f;
+    const float inv = live ? 1.f / s : 0.f;
     __nv_bfloat16* hrow = hi + m * Vp;
     __nv_bfloat16* lrow = lo ? lo + m * Vp : nullptr;
-    const int tcol = valid ? (int)t : -1;
+    const int tcol = live ? (int)t : -1;
     for (int i = threadIdx.x * 4; i < Vp; i += CE_THREADS * 4) {      // Vp % 64 == 0; shared row holds round4(V) floats
         float u[4] = {0.f, 0.f, 0.f, 0.f};
         if (i < V) {
@@ -644,7 +651,8 @@ int caphn_ce_bwd_split(const float* X, long ld, const long long* tgt, long M, in
                        const float* lse, const float* gscale, const float* lossbuf, void* hi, void* lo, long Vp,
                        void* hiT, void* loT, long Mp, float* dbias, void* stream) {
     if (M <= 0 || V <= 0 || Vp < V || (Vp & 63) || Mp < M || (Mp & 63) || M > (1L << 30)) return CAPHN_EINVAL;
-    dim3 grid((unsigned)(Vp / 64), (unsigned)(Mp / 64));
+    if (Vp / 64 > 65535) return CAPHN_EINVAL;               // v-tiles on gridDim.y
+    dim3 grid((unsigned)(Mp / 64), (unsigned)(Vp / 64));
     ce_bwd_split_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(
         X, ld, tgt, (int)M, V, has_ignore, ignore, lse, gscale, lossbuf, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo, Vp,
         (__nv_bfloat16*)hiT, (__nv_bfloat16*)loT, Mp, dbias);
@@ -704,6 +712,7 @@ int caphn_colsum(const float* X, long ld, long M, int N, float* out, void* strea
     const long xb = ceil_div(N, 128);
     long rpb = 256;
     while (rpb > 16 && xb * ceil_div(M, rpb) < 8L * kNumSMs) rpb >>= 1;
+    if (ceil_div(M, rpb) > 65535) rpb = (M + 65534) / 65535;     // the row blocks are on gridDim.y, which stops at 65535
     dim3 grid(xb, ceil_div(M, rpb));
     colsum_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(X, ld, M, N, rpb, out);
     CAPHN_RETURN_LAST();

@@ -184,30 +184,37 @@ int caphn_attn_df(const float* attn, const float* dCTX, float* df, int B, int T,
 /* ---- loss / sampling / embedding (cc_train_hypernet.py:153, hypernet.py:145; decoderlstm.py:62,91-96; later.py:472-479) */
 
 /* Mean softmax cross-entropy over rows of X[M,V] whose target != ignore (when has_ignore).  lse [M]; scratch [2M];
- * lossbuf[0] = mean loss, lossbuf[1] = number of counted rows. */
+ * lossbuf[0] = mean loss, lossbuf[1] = number of counted rows.  Targets (every caphn_ce_* entry point): the ignore index
+ * may be any value; any other target outside [0, V) is a counted row with a NaN loss (so the mean is NaN) and a zero
+ * gradient row, and nothing outside the row is read for it. */
 int caphn_ce_fwd(const float* X, long ld, const long long* tgt, long M, int V, int has_ignore, long long ignore,
                  float* lse, float* scratch, float* lossbuf, void* stream);
 /* dX = gscale[0] * d(mean loss)/dX, using lse / lossbuf from caphn_ce_fwd (no host sync). */
 int caphn_ce_bwd(const float* X, long ld, const long long* tgt, long M, int V, int has_ignore, long long ignore,
                  const float* lse, const float* gscale, const float* lossbuf, float* dX, long lddx, void* stream);
 /* Same gradient, written directly as tensor-core operands (no fp32 dlogits): hi/lo [M,Vp] = split(d), hiT/loT [V,Mp] =
- * split(d^T) (Vp, Mp multiples of 64), dbias[v] += sum_m d[m,v] (zero-initialised by the caller). */
+ * split(d^T) (Vp, Mp multiples of 64), dbias[v] += sum_m d[m,v] (zero-initialised by the caller).  M <= 2^30,
+ * Vp <= 64 * 65535. */
 int caphn_ce_bwd_split(const float* X, long ld, const long long* tgt, long M, int V, int has_ignore, long long ignore,
                        const float* lse, const float* gscale, const float* lossbuf, void* hi, void* lo, long Vp,
                        void* hiT, void* loT, long Mp, float* dbias, void* stream);
 /* Y (optional) = row softmax of X[M,V]; amax (optional, int64) = row argmax, lowest index on ties, NaN counted as -inf
  * (an all-NaN / all -inf row gives 0). */
 int caphn_softmax_argmax(const float* X, long ld, long M, int V, float* Y, long ldy, long long* amax, void* stream);
-/* out[i,:] = table[idx[i],:]  (idx int64; negative idx -> zero row). */
+/* out[i,:] = table[idx[i],:]  (idx int64; negative idx -> zero row; idx must be below the table's row count, which the
+ * call does not know). */
 int caphn_gather_rows(const float* table, const long long* idx, long n, int E, float* out, long ldo, void* stream);
 /* Time-major decoder inputs X[T,B,E].  mode 0 (later.py:411,418): X[0]=feat, X[t]=Emb[caps[:,t-1]];
- * mode 1 (models/decoderlstm.py:82-88): X[0]=X[1]=0, X[t]=Emb[caps[:,t-1]]. */
+ * mode 1 (models/decoderlstm.py:82-88): X[0]=X[1]=0, X[t]=Emb[caps[:,t-1]].  The tokens read must lie in
+ * [0, rows of Emb): they are addresses, not checked. */
 int caphn_build_inputs(const float* feat, const float* emb, const long long* caps, int B, int T, int E, int mode,
                        float* X, void* stream);
-/* dEmb[caps[b,t-1],:] += dX[t,b,:] for t >= t0  (embedding_dense_backward). */
+/* dEmb[caps[b,t-1],:] += dX[t,b,:] for t >= t0  (embedding_dense_backward); nothing when T <= t0.  The tokens read must
+ * lie in [0, rows of dEmb): they are addresses, not checked. */
 int caphn_embed_scatter_add(const float* dX, const long long* caps, int B, int T, int E, int t0, float* dEmb,
                             void* stream);
-/* table[idx[i],:] += dX[i*ldx + :]  for idx[i] >= 0  (embedding backward for arbitrary fed-back tokens). */
+/* table[idx[i],:] += dX[i*ldx + :]  for idx[i] >= 0  (embedding backward for arbitrary fed-back tokens); idx must be
+ * below the table's row count, which the call does not know. */
 int caphn_scatter_add_rows(const float* dX, long ldx, const long long* idx, long n, int E, float* table, void* stream);
 /* out[n] += sum_m X[m*ld+n]  (bias gradients). */
 int caphn_colsum(const float* X, long ld, long M, int N, float* out, void* stream);
